@@ -6,6 +6,7 @@ batch 1 per GPU, data-parallel over N B200s.
     python bench.py --gpus 1 --steps 10 --warmup 3                    # our CUDA path (one JSON line)
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...                               # the reference algorithm on the host CPU cores
+    python bench.py --gpus 1 --steps 10 --warmup 3 --dump-outputs DIR  # + the last timed step's results as DIR/*.npy
 
 `value`      : whole-job samples/s with inputs already resident in HBM (CUDA events, max over ranks).
 `e2e`        : same metric through the public model API from pinned HOST buffers: per step the H2D copy of that
@@ -215,6 +216,33 @@ def make_loss(device, config4=False):
     return LossHandler(p).to(device).train()
 
 
+DUMP_GRAD_ELEMS = 1 << 17     # per gradient; larger ones are sampled (51 of the 162 tensors of the headline model)
+DUMP_PRED_ELEMS = 1 << 21     # of the (B, 73, 720, 1440) prediction
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, loss, pred, model):
+    """What one training step hands its caller -- the loss, the prediction and every parameter gradient -- as float32
+    DIR/loss.npy, DIR/pred.npy and DIR/grad.<parameter name>.npy.  An array above its element cap is replaced by the
+    elements at a fixed set of flat positions (seeded by the array's size, sorted), the same in every run, so the files of
+    two builds compare element for element."""
+    import numpy as np
+    arrays = {"loss": (loss, 1), "pred": (pred, DUMP_PRED_ELEMS)}
+    arrays.update({f"grad.{k}": (p.grad, DUMP_GRAD_ELEMS) for k, p in model.named_parameters() if p.grad is not None})
+    host = {}
+    for name, (t, cap) in arrays.items():
+        a = t.detach()
+        if a.numel() > cap:
+            idx = torch.randint(0, a.numel(), (cap,), generator=torch.Generator().manual_seed(a.numel())).sort().values
+            a = a.reshape(-1)[idx.to(a.device)]
+        host[name] = a.float().cpu().numpy()
+    total = sum(a.nbytes for a in host.values())
+    assert total <= DUMP_MAX_BYTES, f"output dump of {total} bytes exceeds {DUMP_MAX_BYTES}"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # ==============================================================================================================
 # our arm
 # ==============================================================================================================
@@ -248,6 +276,7 @@ def run_ours(args):
     t_res = host_t[:, :, :720].contiguous().to(dev)
 
     zen_res = (torch.rand(B, 1, 720, 1440, generator=gen) * 2 - 1).to(dev) if config4 else None
+    last = {}                   # --dump-outputs: the latest step's loss and prediction
 
     def step(x, t, t_ready=None):
         for p in params:
@@ -257,6 +286,8 @@ def run_ours(args):
             torch.cuda.current_stream().wait_event(t_ready)
         loss = lossf(pred, t, x)
         loss.backward()
+        if args.dump_outputs:
+            last.update(loss=loss, pred=pred)
         return loss
 
     def barrier():
@@ -299,6 +330,8 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     fam = timer.summary()
     peak_mem = torch.cuda.max_memory_allocated(dev) / 2 ** 30
+    if args.dump_outputs and rank == 0:     # the gradients are all-reduced; the prediction is rank 0's sample
+        dump_outputs(args.dump_outputs, last["loss"], last["pred"], model)
 
     # ---- leg 2: end to end from pinned host buffers (prefetch on a copy stream, double-buffered) ---------------
     from swin_v2_weather_b200.utils.host_io import copy_cropped_async
@@ -682,7 +715,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--profile-step", action="store_true", help="run one profiled step (for ncu) and exit")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps with resident inputs, write the last one's loss, prediction and parameter "
+                         "gradients to DIR/*.npy (float32, large arrays as a fixed sample, <= 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.sweep or args.profile_step):
+        ap.error("--dump-outputs applies to the timed steps of the default CUDA path")
     if args.sweep == "attn":
         run_attn_sweep(args)
     elif args.impl == "reference":

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- generates tests/golden/*.pt by running the UNMODIFIED reference
-(/root/reference, imported through oracle/shim.py) on CPU in fp32.
+(a checkout named by SWIN_REFERENCE_ROOT, imported through oracle/shim.py) on CPU in fp32.
 
-Run in the build container:   python -m oracle.make_golden
+Run:   SWIN_REFERENCE_ROOT=<reference checkout> python -m oracle.make_golden
 The fixtures are small: inputs and weights are *not* stored -- they are regenerated from seeds with
 `oracle.swinv2_oracle.init_state_dict` / CPU generators, which is deterministic for a given torch build.
 Stored per case: prediction, loss, per-parameter gradient norms and 64 sampled gradient entries.

@@ -1,14 +1,15 @@
 """TEST INFRASTRUCTURE ONLY -- import shim for the *unmodified* reference.
 
-The reference hot-path file (`/root/reference/networks/swinv2_global.py:5,12`) hard-imports
-`ruamel.yaml` and `timm.layers`, neither of which is installed in this image (and there is no
-network).  This module registers minimal stand-ins in `sys.modules` so the reference file can be
-imported *unmodified* in the build container, where it is used for exactly two things:
+The reference is not part of this repository: point `SWIN_REFERENCE_ROOT` at a checkout of it
+(the directory holding `networks/` and `utils/`) to use it.  Its hot-path file
+(`networks/swinv2_global.py:5,12`) hard-imports `ruamel.yaml` and `timm.layers`, which need not
+be installed.  This module registers minimal stand-ins in `sys.modules` so the reference file can be
+imported *unmodified*, where it is used for exactly two things:
 
   * validating `oracle/swinv2_oracle.py` (our CPU restatement) against the real reference, and
   * generating the golden fixtures under `tests/golden/` (`oracle/make_golden.py`).
 
-`/root/reference` does not exist on the GPU box, so nothing in `-m gpu` tests, `smoke()` or
+Without `SWIN_REFERENCE_ROOT` the reference is absent, so nothing in `-m gpu` tests, `smoke()` or
 `bench.py` may call `import_reference()`.  The product package never imports this file.
 
 Third-party semantics restated here (timm is un-pinned by the reference; header says "Adapted from
@@ -27,7 +28,7 @@ import types
 import torch
 import torch.nn as nn
 
-REFERENCE_ROOT = os.environ.get("SWIN_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("SWIN_REFERENCE_ROOT", "")
 
 
 def _to_2tuple(x):
@@ -121,13 +122,13 @@ def install():
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "networks", "swinv2_global.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "networks", "swinv2_global.py"))
 
 
 def import_reference():
     """Returns (swinv2_global module, losses module) of the unmodified reference."""
     if not reference_available():
-        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference tree not found: set SWIN_REFERENCE_ROOT (now {REFERENCE_ROOT!r})")
     install()
     # the reference uses top-level package names `networks` / `utils`; load them under private
     # names so they can never shadow (or be shadowed by) anything of ours

@@ -1,5 +1,5 @@
 """CPU: the oracle (our restatement) against fixtures produced by the unmodified reference
-(`oracle/make_golden.py`, run in the build container where /root/reference exists)."""
+(`oracle/make_golden.py`, run with SWIN_REFERENCE_ROOT naming a checkout of the reference)."""
 import os
 
 import numpy as np

@@ -1,12 +1,13 @@
-"""CPU, build container only: the oracle against the live, unmodified reference (skipped where
-/root/reference is absent, e.g. on the GPU box -- there the committed fixtures stand in)."""
+"""CPU: the oracle against the live, unmodified reference.  The reference is not part of this repository: these tests
+run when SWIN_REFERENCE_ROOT names a checkout of it and are skipped otherwise -- then the committed fixtures of
+tests/test_oracle_golden.py stand in for it."""
 import pytest
 import torch
 
 from oracle import shim
 from oracle import swinv2_oracle as O
 
-pytestmark = pytest.mark.skipif(not shim.reference_available(), reason="reference tree not present")
+pytestmark = pytest.mark.skipif(not shim.reference_available(), reason="reference tree not present (set SWIN_REFERENCE_ROOT)")
 
 
 @pytest.mark.parametrize("rel_pos", [False, True])
