@@ -25,6 +25,11 @@ __device__ __forceinline__ void window_slot(const WinGeom& g, int b, int w, int 
 }
 
 constexpr int kAttnWarps = 8;
+constexpr int kMaxHeadDim = 256;
+
+// GLOBAL_KV: the per-window operand tiles (2 x L rows of d + 1 fp32 / d + 2 bf16 values) do not fit in shared memory -- fp32 at
+// head_dim 256 needs 333 KB for 9x18 windows -- so the dot products read their rows in place from global memory (L2).
+// This back end is the validation / bring-up path; the layout of the loops is the same either way.
 
 template <typename T>
 __device__ __forceinline__ int pad_d(int d) { return sizeof(T) == 4 ? d + 1 : d + 2; }
@@ -32,7 +37,7 @@ __device__ __forceinline__ int pad_d(int d) { return sizeof(T) == 4 ? d + 1 : d 
 // ------------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------------
-template <typename T>
+template <typename T, bool GLOBAL_KV>
 __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_fwd_kernel(const T* __restrict__ qkv, const float* __restrict__ scale_p,
                                                                         const float* __restrict__ bias, T* __restrict__ o,
                                                                         float* __restrict__ lse, WinGeom g) {
@@ -43,8 +48,8 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_fwd_kernel(const T*
   const int b = blockIdx.x / (g.heads * g.nW());
   const bool masked = (g.s0 > 0 || g.s1 > 0);
   T* Ks = reinterpret_cast<T*>(smem_raw);
-  T* Vs = Ks + (size_t)L * dp;
-  float* fbase = reinterpret_cast<float*>(Vs + (size_t)L * dp);  // 2*L*dp*sizeof(T) is a multiple of 4
+  T* Vs = Ks + (GLOBAL_KV ? 0 : (size_t)L * dp);
+  float* fbase = reinterpret_cast<float*>(Vs + (GLOBAL_KV ? 0 : (size_t)L * dp));  // 2*L*dp*sizeof(T) is a multiple of 4
   float* qs = fbase;                          // [warps][d]
   float* ps = qs + kAttnWarps * d;            // [warps][L]
   int* tok = reinterpret_cast<int*>(ps + kAttnWarps * L);  // [L]
@@ -59,13 +64,17 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_fwd_kernel(const T*
     lab[n] = l;
   }
   __syncthreads();
-  for (int it = threadIdx.x; it < L * d; it += blockDim.x) {
-    const int n = it / d, c = it % d;
-    const T* row = qkv + (size_t)tok[n] * C3 + head * d + c;
-    Ks[n * dp + c] = row[g.C];
-    Vs[n * dp + c] = row[2 * g.C];
+  if (!GLOBAL_KV) {
+    for (int it = threadIdx.x; it < L * d; it += blockDim.x) {
+      const int n = it / d, c = it % d;
+      const T* row = qkv + (size_t)tok[n] * C3 + head * d + c;
+      Ks[n * dp + c] = row[g.C];
+      Vs[n * dp + c] = row[2 * g.C];
+    }
+    __syncthreads();
   }
-  __syncthreads();
+  auto k_row = [&](int j) -> const T* { return GLOBAL_KV ? qkv + (size_t)tok[j] * C3 + g.C + head * d : Ks + j * dp; };
+  auto v_row = [&](int j) -> const T* { return GLOBAL_KV ? qkv + (size_t)tok[j] * C3 + 2 * g.C + head * d : Vs + j * dp; };
 
   const float scale = scale_p[head];
   float* myq = qs + wid * d;
@@ -77,7 +86,7 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_fwd_kernel(const T*
     float mx = -INFINITY;
     for (int j = lane; j < L; j += 32) {
       float acc = 0.f;
-      const T* kr = Ks + j * dp;
+      const T* kr = k_row(j);
       for (int c = 0; c < d; ++c) acc = fmaf(myq[c], Act<T>::ld(kr + c), acc);
       float s = acc * scale;
       if (bias) s += bias[((size_t)head * L + i) * L + j];
@@ -98,7 +107,7 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_fwd_kernel(const T*
     T* orow = o + (size_t)tok[i] * g.C + head * d;
     for (int c = lane; c < d; c += 32) {
       float acc = 0.f;
-      for (int j = 0; j < L; ++j) acc = fmaf(myp[j], Act<T>::ld(Vs + j * dp + c), acc);
+      for (int j = 0; j < L; ++j) acc = fmaf(myp[j], Act<T>::ld(v_row(j) + c), acc);
       Act<T>::st(orow + c, acc * inv);
     }
     if (lane == 0) lse[(((size_t)b * g.nW() + w) * g.heads + head) * L + i] = mx + logf(sum);
@@ -109,7 +118,7 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_fwd_kernel(const T*
 // ------------------------------------------------------------------------------------------------
 // backward
 // ------------------------------------------------------------------------------------------------
-template <typename T>
+template <typename T, bool GLOBAL_KV>
 __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T* __restrict__ qkv, const float* __restrict__ inv_norm,
                                                                         const float* __restrict__ scale_p, const float* __restrict__ bias,
                                                                         const T* __restrict__ o, const T* __restrict__ d_o,
@@ -123,8 +132,8 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T*
   const int b = blockIdx.x / (g.heads * g.nW());
   const bool masked = (g.s0 > 0 || g.s1 > 0);
   T* M0 = reinterpret_cast<T*>(smem_raw);   // phase 1: Khat ; phase 2: Qhat
-  T* M1 = M0 + (size_t)L * dp;              // phase 1: V    ; phase 2: dO
-  float* fbase = reinterpret_cast<float*>(M1 + (size_t)L * dp);
+  T* M1 = M0 + (GLOBAL_KV ? 0 : (size_t)L * dp);              // phase 1: V    ; phase 2: dO
+  float* fbase = reinterpret_cast<float*>(M1 + (GLOBAL_KV ? 0 : (size_t)L * dp));
   float* va = fbase;                         // [warps][d]  phase 1: qhat_i ; phase 2: khat_j
   float* vb = va + kAttnWarps * d;           // [warps][d]  phase 1: dO_i   ; phase 2: v_j
   float* ps = vb + kAttnWarps * d;           // [warps][L]  dS
@@ -146,13 +155,24 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T*
     lses[n] = lse[(((size_t)b * g.nW() + w) * g.heads + head) * L + n];
   }
   __syncthreads();
-  for (int it = threadIdx.x; it < L * d; it += blockDim.x) {
-    const int n = it / d, c = it % d;
-    const T* row = qkv + (size_t)tok[n] * C3 + head * d + c;
-    M0[n * dp + c] = row[g.C];
-    M1[n * dp + c] = row[2 * g.C];
+  if (!GLOBAL_KV) {
+    for (int it = threadIdx.x; it < L * d; it += blockDim.x) {
+      const int n = it / d, c = it % d;
+      const T* row = qkv + (size_t)tok[n] * C3 + head * d + c;
+      M0[n * dp + c] = row[g.C];
+      M1[n * dp + c] = row[2 * g.C];
+    }
+    __syncthreads();
   }
-  __syncthreads();
+  int phase = 1;
+  auto m0_row = [&](int n) -> const T* {
+    if (!GLOBAL_KV) return M0 + n * dp;
+    return qkv + (size_t)tok[n] * C3 + (phase == 1 ? g.C : 0) + head * d;
+  };
+  auto m1_row = [&](int n) -> const T* {
+    if (!GLOBAL_KV) return M1 + n * dp;
+    return phase == 1 ? qkv + (size_t)tok[n] * C3 + 2 * g.C + head * d : d_o + (size_t)tok[n] * g.C + head * d;
+  };
 
   const float scale = scale_p[head];
   float dsc_acc = 0.f;
@@ -177,8 +197,8 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T*
     const float lse_i = lses[i];
     for (int j = lane; j < L; j += 32) {
       float cs = 0.f, dpv = 0.f;
-      const T* kr = M0 + j * dp;
-      const T* vr = M1 + j * dp;
+      const T* kr = m0_row(j);
+      const T* vr = m1_row(j);
       for (int c = 0; c < d; ++c) {
         cs = fmaf(mya[c], Act<T>::ld(kr + c), cs);
         dpv = fmaf(myb[c], Act<T>::ld(vr + c), dpv);
@@ -194,12 +214,12 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T*
     }
     __syncwarp();
     // dqhat, then back through the normalisation: dq = inv_norm * (dqhat - qhat * <qhat, dqhat>)
-    float dq[6];
+    float dq[kMaxHeadDim / 32];
     float dot = 0.f;
     int cc = 0;
     for (int c = lane; c < d; c += 32, ++cc) {
       float acc = 0.f;
-      for (int j = 0; j < L; ++j) acc = fmaf(myds[j], Act<T>::ld(M0 + j * dp + c), acc);
+      for (int j = 0; j < L; ++j) acc = fmaf(myds[j], Act<T>::ld(m0_row(j) + c), acc);
       dq[cc] = acc * scale;
       dot += dq[cc] * mya[c];
     }
@@ -213,12 +233,15 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T*
   __syncthreads();
 
   // ---- phase 2: reload with Qhat / dO; one key row per warp-iteration -> dk, dv ------------------
-  for (int it = threadIdx.x; it < L * d; it += blockDim.x) {
-    const int n = it / d, c = it % d;
-    M0[n * dp + c] = qkv[(size_t)tok[n] * C3 + head * d + c];
-    M1[n * dp + c] = d_o[(size_t)tok[n] * g.C + head * d + c];
+  phase = 2;
+  if (!GLOBAL_KV) {
+    for (int it = threadIdx.x; it < L * d; it += blockDim.x) {
+      const int n = it / d, c = it % d;
+      M0[n * dp + c] = qkv[(size_t)tok[n] * C3 + head * d + c];
+      M1[n * dp + c] = d_o[(size_t)tok[n] * g.C + head * d + c];
+    }
+    __syncthreads();
   }
-  __syncthreads();
   for (int j = wid; j < L; j += kAttnWarps) {
     const size_t t = tok[j];
     for (int c = lane; c < d; c += 32) {
@@ -228,8 +251,8 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T*
     __syncwarp();
     for (int i = lane; i < L; i += 32) {
       float cs = 0.f, dpv = 0.f;
-      const T* qr = M0 + i * dp;
-      const T* gr = M1 + i * dp;
+      const T* qr = m0_row(i);
+      const T* gr = m1_row(i);
       for (int c = 0; c < d; ++c) {
         cs = fmaf(mya[c], Act<T>::ld(qr + c), cs);
         dpv = fmaf(myb[c], Act<T>::ld(gr + c), dpv);
@@ -242,14 +265,14 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T*
       myds[i] = p * (dpv - Ds[i]);
     }
     __syncwarp();
-    float dk[6];
+    float dk[kMaxHeadDim / 32];
     float dot = 0.f;
     int cc = 0;
     for (int c = lane; c < d; c += 32, ++cc) {
       float ak = 0.f, av = 0.f;
       for (int i = 0; i < L; ++i) {
-        ak = fmaf(myds[i], Act<T>::ld(M0 + i * dp + c), ak);
-        av = fmaf(myp[i], Act<T>::ld(M1 + i * dp + c), av);
+        ak = fmaf(myds[i], Act<T>::ld(m0_row(i) + c), ak);
+        av = fmaf(myp[i], Act<T>::ld(m1_row(i) + c), av);
       }
       dk[cc] = ak * scale;
       dot += dk[cc] * mya[c];
@@ -274,10 +297,10 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T*
 }
 
 template <typename T>
-static size_t attn_smem_bytes(const WinGeom& g, bool bwd) {
+static size_t attn_smem_bytes(const WinGeom& g, bool bwd, bool global_kv) {
   const int L = g.L(), d = g.d();
   const int dp = sizeof(T) == 4 ? d + 1 : d + 2;
-  size_t b = 2 * (size_t)L * dp * sizeof(T);
+  size_t b = global_kv ? 0 : 2 * (size_t)L * dp * sizeof(T);
   b = (b + 3) / 4 * 4;
   if (!bwd)
     b += (size_t)(kAttnWarps * d + kAttnWarps * L) * 4 + 2 * (size_t)L * 4;
@@ -288,13 +311,15 @@ static size_t attn_smem_bytes(const WinGeom& g, bool bwd) {
 
 template <typename T>
 static int launch_fwd(const T* qkv, const float* scale, const float* bias, T* o, float* lse, const WinGeom& g, cudaStream_t s) {
-  const size_t smem = attn_smem_bytes<T>(g, false);
+  const bool global_kv = attn_smem_bytes<T>(g, false, false) > 227 * 1024;
+  const size_t smem = attn_smem_bytes<T>(g, false, global_kv);
   if (smem > 227 * 1024) {
     set_error("window_attn_fwd (CUDA-core back end): window %dx%d, head_dim %d needs %zu B of shared memory", g.Wh, g.Ww, g.d(), smem);
     return SWINB200_ERR_UNSUPPORTED;
   }
-  SWB_CUDA(cudaFuncSetAttribute(attn_simt_fwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  attn_simt_fwd_kernel<T><<<g.B * g.nW() * g.heads, kAttnWarps * 32, smem, s>>>(qkv, scale, bias, o, lse, g);
+  auto kernel = global_kv ? attn_simt_fwd_kernel<T, true> : attn_simt_fwd_kernel<T, false>;
+  SWB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<g.B * g.nW() * g.heads, kAttnWarps * 32, smem, s>>>(qkv, scale, bias, o, lse, g);
   SWB_LAUNCH_CHECK();
   return SWINB200_OK;
 }
@@ -302,13 +327,15 @@ static int launch_fwd(const T* qkv, const float* scale, const float* bias, T* o,
 template <typename T>
 static int launch_bwd(const T* qkv, const float* inv_norm, const float* scale, const float* bias, const T* o, const T* d_o,
                       const float* lse, T* dqkv, float* dscale, float* dbias, const WinGeom& g, cudaStream_t s) {
-  const size_t smem = attn_smem_bytes<T>(g, true);
+  const bool global_kv = attn_smem_bytes<T>(g, true, false) > 227 * 1024;
+  const size_t smem = attn_smem_bytes<T>(g, true, global_kv);
   if (smem > 227 * 1024) {
     set_error("window_attn_bwd (CUDA-core back end): window %dx%d, head_dim %d needs %zu B of shared memory", g.Wh, g.Ww, g.d(), smem);
     return SWINB200_ERR_UNSUPPORTED;
   }
-  SWB_CUDA(cudaFuncSetAttribute(attn_simt_bwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  attn_simt_bwd_kernel<T><<<g.B * g.nW() * g.heads, kAttnWarps * 32, smem, s>>>(qkv, inv_norm, scale, bias, o, d_o, lse, dqkv, dscale, dbias, g);
+  auto kernel = global_kv ? attn_simt_bwd_kernel<T, true> : attn_simt_bwd_kernel<T, false>;
+  SWB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<g.B * g.nW() * g.heads, kAttnWarps * 32, smem, s>>>(qkv, inv_norm, scale, bias, o, d_o, lse, dqkv, dscale, dbias, g);
   SWB_LAUNCH_CHECK();
   return SWINB200_OK;
 }
@@ -322,7 +349,7 @@ int attn_tcgen05_bwd(const void* qkv, const float* inv_norm, const float* scale,
 static int check_geom(const char* who, int B, int H, int W, int C, int heads, int Wh, int Ww, int s0, int s1) {
   SWB_CHECK_ARG(B > 0 && H > 0 && W > 0 && C > 0 && heads > 0, "%s: bad shape", who);
   SWB_CHECK_ARG(Wh > 0 && Ww > 0 && H % Wh == 0 && W % Ww == 0, "%s: window (%d,%d) does not tile the (%d,%d) grid", who, Wh, Ww, H, W);
-  SWB_CHECK_ARG(C % heads == 0 && (C / heads) % 8 == 0 && C / heads <= 192, "%s: head_dim %d unsupported", who, C / heads);
+  SWB_CHECK_ARG(C % heads == 0 && (C / heads) % 8 == 0 && C / heads <= kMaxHeadDim, "%s: head_dim %d unsupported", who, C / heads);
   SWB_CHECK_ARG(s0 >= 0 && s0 < Wh && s1 >= 0 && s1 < Ww, "%s: shift (%d,%d) must be smaller than the window", who, s0, s1);
   return SWINB200_OK;
 }

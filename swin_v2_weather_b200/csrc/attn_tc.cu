@@ -547,7 +547,7 @@ int attn_make_geom(AttnGeom& g, int B, int H, int W, int C, int heads, int Wh, i
   g.nWw = W / Ww;
   g.nW = (H / Wh) * g.nWw;
   if (!attn_gen_supports(C / heads)) {
-    set_error("window_attn (tcgen05): head_dim %d is not instantiated (48, 64, 96, 128, 192)", C / heads);
+    set_error("window_attn (tcgen05): head_dim %d is not instantiated (48, 64, 96, 128, 192, 256)", C / heads);
     return SWINB200_ERR_UNSUPPORTED;
   }
   return SWINB200_OK;

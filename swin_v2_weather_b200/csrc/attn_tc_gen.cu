@@ -1,13 +1,20 @@
 // tcgen05 window attention for every geometry the specialised 9x18 / head_dim-96 kernels (attn_tc_fwd3.cu,
-// attn_tc_bwd3.cu) are not instantiated for: head_dim 48 / 64 / 96 / 128 / 192 and windows of any size (BASELINE config 5:
-// 6x12, 12x24, 18x36 ...).  Restates WindowMultiHeadAttention.forward (reference networks/swinv2_global.py:300-319) and its
-// backward as three flash-style kernels of one shape:
+// attn_tc_bwd3.cu) are not instantiated for: head_dim 48 / 64 / 96 / 128 / 192 / 256 and windows of any size (BASELINE
+// config 5: 6x12, 12x24, 18x36 ...).  Restates WindowMultiHeadAttention.forward (reference networks/swinv2_global.py:300-319)
+// and its backward as three flash-style kernels of one shape:
 //
 //   a CTA owns one 128-row "stationary" tile X of a (sample, window, head) item and streams 64-row tiles Y past it
 //
 //   forward      X = Q^ rows          Y = (K^, V) rows     S = X Y0^T -> P -> O += P Y1                  (thread = query)
 //   backward A   X = (Q^, dO) rows    Y = (K^, V) rows     S, dP = X1 Y1^T -> dS -> dQ^ += dS Y0         (thread = query)
 //   backward B   X = (K^, V) rows     Y = (Q^, dO) rows    S^T, dP^T -> P^T, dS^T -> dV += P^T Y1, dK^ += dS^T Y0   (thread = key)
+//
+// head_dim 256 (the e2048 / 8-head config) does not fit that shape everywhere: backward A streams 32-row tiles (two 128 x 256
+// stationary operands leave no room for 64-row double buffers), and backward B -- two 256-column fp32 accumulators plus the
+// S^T / dP^T tiles exceed the 512 tensor-memory columns at any tile height -- runs as two passes over the same items:
+//   backward V   X = K^ rows          Y = (Q^, dO) rows    S^T -> P^T -> dV += P^T Y1                                  (thread = key)
+//   backward K   X = (K^, V) rows     Y = (Q^, dO) rows    S^T, dP^T -> dS^T -> dK^ += dS^T Y0, d(bias)              (thread = key)
+// d(scale) is summed by backward A only and d(bias) by backward B / K only, so the split counts neither twice.
 //
 // S-type products take both operands from shared memory (un-swizzled core-matrix layout [16-byte chunk][row][8 elements]: the
 // same bytes serve K-major and MN-major descriptors, so no transposed copy exists anywhere); P / dS are packed to bf16 in place
@@ -23,14 +30,15 @@
 namespace swinb200 {
 namespace {
 
-constexpr int kModeFwd = 0, kModeBwdQ = 1, kModeBwdKV = 2;
+constexpr int kModeFwd = 0, kModeBwdQ = 1, kModeBwdKV = 2, kModeBwdV = 3, kModeBwdK = 4;
+__host__ __device__ constexpr bool key_mode(int mode) { return mode >= kModeBwdKV; }     // thread = key, Y = (Q^, dO)
 
 __host__ __device__ constexpr int pow2_cols(int n) { return n <= 32 ? 32 : n <= 64 ? 64 : n <= 128 ? 128 : n <= 256 ? 256 : 512; }
 
 template <int D, int KT, int MODE, bool HAS_BIAS>
 struct GenCfg {
   static constexpr int kChunks = D / 8;
-  static constexpr int kNX = (MODE == kModeFwd) ? 1 : 2;
+  static constexpr int kNX = (MODE == kModeFwd || MODE == kModeBwdV) ? 1 : 2;
   static constexpr int kCSX = 128 * 16 + 16;                 // chunk stride of the stationary tile (+16: spreads the gather over banks)
   static constexpr int kTileX = kChunks * kCSX;
   static constexpr int kCSY = KT * 16 + 16;
@@ -41,11 +49,11 @@ struct GenCfg {
   static constexpr int kOffColA = kOffTokX + 128 * 4;         // [2][KT]  log2-domain LSE of the streamed query rows (backward B)
   static constexpr int kOffColB = kOffColA + 2 * KT * 4;      // [2][KT]  D = <dO, O> of the streamed query rows
   static constexpr int kOffBias = kOffColB + 2 * KT * 4;      // [4 warps][32 rows][20] bias pieces on their way to their rows (fwd / A)
-  static constexpr int kOffBar = kOffBias + ((MODE == kModeBwdKV || !HAS_BIAS) ? 0 : 4 * 32 * 20 * 4);
+  static constexpr int kOffBar = kOffBias + ((key_mode(MODE) || !HAS_BIAS) ? 0 : 4 * 32 * 20 * 4);
   static constexpr int kBytes = kOffBar + 64;
   static constexpr int kStagePitch = D * 2 + 16;              // output rows parked in the (dead) Y buffers
   static constexpr int kColS = 0, kColDP = KT;
-  static constexpr int kColAcc0 = (MODE == kModeFwd) ? KT : 2 * KT;
+  static constexpr int kColAcc0 = (kNX == 1) ? KT : 2 * KT;     // one stationary operand: no dP tile
   static constexpr int kColAcc1 = kColAcc0 + D;
   static constexpr int kColAdd = kColAcc0 + D;               // forward: log2-domain addend (bias + mask) of the current tile
   static constexpr int kColsUsed = kColAcc0 + ((MODE == kModeBwdKV) ? 2 : 1) * D + ((MODE == kModeFwd && HAS_BIAS) ? KT : 0);
@@ -163,7 +171,7 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
       const int r = i / CF::kChunks, c = i - r * CF::kChunks;
       int rr;
       const size_t tk = (size_t)win_token(g, b, w, t * KT + r, rr);
-      if (MODE == kModeBwdKV) {
+      if (key_mode(MODE)) {
         if (op_mask & 1) cp_async16(base + c * CF::kCSY + r * 16, a.qkv + tk * C3 + head * D + c * 8);
         if (op_mask & 2) cp_async16(base + CF::kTileY + c * CF::kCSY + r * 16, a.d_o + tk * C + head * D + c * 8);
       } else {
@@ -171,7 +179,7 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
         if (op_mask & 2) cp_async16(base + CF::kTileY + c * CF::kCSY + r * 16, a.qkv + tk * C3 + 2 * C + head * D + c * 8);
       }
     }
-    if (MODE == kModeBwdKV && tid < KT) {        // per-column (= streamed query) terms
+    if (key_mode(MODE) && tid < KT) {            // per-column (= streamed query) terms
       if (tid < rows) {
         int rr;
         const size_t tk = (size_t)win_token(g, b, w, t * KT + tid, rr);
@@ -212,7 +220,7 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
   auto bias_fetch = [&](int y0_) {               // y0_ = first streamed slot of the chunk; out-of-range chunks fetch nothing
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
-      if (MODE == kModeBwdKV) {
+      if (key_mode(MODE)) {
         const int qi = y0_ + i;
         nb[i] = (row_ok && qi < L) ? __ldg(a.bias + ((size_t)head * L + qi) * L + nx) : 0.f;
       } else {
@@ -223,7 +231,7 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
     }
   };
   auto bias_take = [&](float (&bv)[16]) {        // the chunk fetched last, as log2-domain addends of this thread's 16 columns
-    if (MODE == kModeBwdKV) {
+    if (key_mode(MODE)) {
 #pragma unroll
       for (int j = 0; j < 16; ++j) bv[j] = nb[j] * kLog2e;
     } else {
@@ -271,7 +279,7 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
       for (int k = 0; k < D / 16; ++k)
         umma_bf16_ss(tmem_base + CF::kColS, umma_desc_nosw(x0 + 2 * k * CF::kCSX, CF::kCSX, 128),
                      umma_desc_nosw(yb + 2 * k * CF::kCSY, CF::kCSY, 128), idesc_s, k > 0);
-      if (MODE != kModeFwd) {
+      if (CF::kNX == 2) {
 #pragma unroll
         for (int k = 0; k < D / 16; ++k)
           umma_bf16_ss(tmem_base + CF::kColDP, umma_desc_nosw(x0 + CF::kTileX + 2 * k * CF::kCSX, CF::kCSX, 128),
@@ -392,7 +400,7 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
       for (int c0 = 0; c0 < KT; c0 += 16) {
         uint32_t v[16], dp[16];
         tmem_ld_32x16(t_lane + CF::kColS + c0, v);
-        tmem_ld_32x16(t_lane + CF::kColDP + c0, dp);
+        if (MODE != kModeBwdV) tmem_ld_32x16(t_lane + CF::kColDP + c0, dp);
         float ls[16], dd[16];
 #pragma unroll
         for (int j = 0; j < 16; j += 4) {
@@ -415,13 +423,15 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
             if (use_mask && ((qi >= label_split) ? 1 : 0) != x_label) s += kMaskL2;
           }
           const float p = row_ok ? ex2_approx(fmaf(-ls[j], kLog2e, s)) : 0.f;     // pad queries: lse = +inf -> 0
-          const float d = (qi < L) ? p * (as_f(dp[j]) - dd[j]) : 0.f;
           pp[j] = p;
-          ds[j] = d;
-          if (a.dbias != nullptr && row_ok && qi < L) atomicAdd(a.dbias + ((size_t)head * L + qi) * L + nx, d);
+          if (MODE != kModeBwdV) {
+            const float d = (qi < L) ? p * (as_f(dp[j]) - dd[j]) : 0.f;
+            ds[j] = d;
+            if (a.dbias != nullptr && row_ok && qi < L) atomicAdd(a.dbias + ((size_t)head * L + qi) * L + nx, d);
+          }
         }
-        tmem_st_32x8(t_lane + CF::kColS + c0 / 2, pack8(pp, 0), pack8(pp, 8));
-        tmem_st_32x8(t_lane + CF::kColDP + c0 / 2, pack8(ds, 0), pack8(ds, 8));
+        if (MODE != kModeBwdK) tmem_st_32x8(t_lane + CF::kColS + c0 / 2, pack8(pp, 0), pack8(pp, 8));
+        if (MODE != kModeBwdV) tmem_st_32x8(t_lane + CF::kColDP + c0 / 2, pack8(ds, 0), pack8(ds, 8));
       }
     }
     tmem_st_wait();
@@ -441,14 +451,19 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
           umma_bf16_ts(tmem_base + CF::kColAcc0, tmem_base + CF::kColDP + k * 8, umma_desc_nosw(yb + k * 256, 128, CF::kCSY), idesc_o,
                        acc | (uint32_t)(k > 0));
       } else {
+        if (MODE != kModeBwdK) {
 #pragma unroll
-        for (int k = 0; k < KT / 16; ++k)        // dV += P^T dO
-          umma_bf16_ts(tmem_base + CF::kColAcc0, tmem_base + CF::kColS + k * 8, umma_desc_nosw(yb + CF::kTileY + k * 256, 128, CF::kCSY),
-                       idesc_o, acc | (uint32_t)(k > 0));
+          for (int k = 0; k < KT / 16; ++k)      // dV += P^T dO
+            umma_bf16_ts(tmem_base + CF::kColAcc0, tmem_base + CF::kColS + k * 8, umma_desc_nosw(yb + CF::kTileY + k * 256, 128, CF::kCSY),
+                         idesc_o, acc | (uint32_t)(k > 0));
+        }
+        if (MODE != kModeBwdV) {
+          const uint32_t col_dk = (MODE == kModeBwdKV) ? CF::kColAcc1 : CF::kColAcc0;
 #pragma unroll
-        for (int k = 0; k < KT / 16; ++k)        // dK^ += dS^T Q^
-          umma_bf16_ts(tmem_base + CF::kColAcc1, tmem_base + CF::kColDP + k * 8, umma_desc_nosw(yb + k * 256, 128, CF::kCSY), idesc_o,
-                       acc | (uint32_t)(k > 0));
+          for (int k = 0; k < KT / 16; ++k)      // dK^ += dS^T Q^
+            umma_bf16_ts(tmem_base + col_dk, tmem_base + CF::kColDP + k * 8, umma_desc_nosw(yb + k * 256, 128, CF::kCSY), idesc_o,
+                         acc | (uint32_t)(k > 0));
+        }
       }
       umma_commit(bar);
     }
@@ -533,15 +548,20 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
     dsc_acc = warp_sum(dsc_acc);
     if (lane == 0 && dsc_acc != 0.f) atomicAdd(a.dscale + head, dsc_acc);
   } else {
-    park(CF::kColAcc0, 1.f, false, 0.f, 1.f);    // dv
-    __syncthreads();
-    scatter(C3, 2 * C + head * D);
-    __syncthreads();
-    const float dot = row_dot(CF::kColAcc1, scale);
-    const float ink = row_ok ? a.inv_norm[(size_t)tokX[tid] * 2 * g.heads + g.heads + head] : 0.f;
-    park(CF::kColAcc1, scale, true, dot, ink);
-    __syncthreads();
-    scatter(C3, C + head * D);
+    if (MODE != kModeBwdK) {
+      park(CF::kColAcc0, 1.f, false, 0.f, 1.f);  // dv
+      __syncthreads();
+      scatter(C3, 2 * C + head * D);
+      __syncthreads();
+    }
+    if (MODE != kModeBwdV) {
+      const uint32_t col_dk = (MODE == kModeBwdKV) ? CF::kColAcc1 : CF::kColAcc0;
+      const float dot = row_dot(col_dk, scale);
+      const float ink = row_ok ? a.inv_norm[(size_t)tokX[tid] * 2 * g.heads + g.heads + head] : 0.f;
+      park(col_dk, scale, true, dot, ink);
+      __syncthreads();
+      scatter(C3, C + head * D);
+    }
   }
   tc_fence_before();
   __syncthreads();
@@ -573,6 +593,18 @@ int launch_gen(const GenArgs& a, const AttnGeom& g, cudaStream_t stream) {
   return a.bias != nullptr ? launch_gen_b<D, KT, MODE, true>(a, g, stream) : launch_gen_b<D, KT, MODE, false>(a, g, stream);
 }
 
+// head_dim 256: 206 KB of shared memory for the forward at KT = 64 and for backward A at KT = 32; backward B as the V pass
+// (KT = 64) followed by the K pass (KT = 32), 196 KB each; every one of them allocates 512 tensor-memory columns
+template <int MODE>
+int launch_gen_256(const GenArgs& a, const AttnGeom& g, cudaStream_t stream) {
+  if constexpr (MODE == kModeFwd) return launch_gen<256, 64, kModeFwd>(a, g, stream);
+  if constexpr (MODE == kModeBwdQ) return launch_gen<256, 32, kModeBwdQ>(a, g, stream);
+  if constexpr (MODE == kModeBwdKV) {
+    if (int e = launch_gen<256, 64, kModeBwdV>(a, g, stream)) return e;
+    return launch_gen<256, 32, kModeBwdK>(a, g, stream);
+  }
+}
+
 template <int MODE>
 int dispatch_gen(const GenArgs& a, const AttnGeom& g, cudaStream_t stream) {
   switch (g.C / g.heads) {
@@ -581,15 +613,18 @@ int dispatch_gen(const GenArgs& a, const AttnGeom& g, cudaStream_t stream) {
     case 96: return launch_gen<96, 64, MODE>(a, g, stream);
     case 128: return launch_gen<128, 64, MODE>(a, g, stream);
     case 192: return launch_gen<192, 64, MODE>(a, g, stream);
+    case 256: return launch_gen_256<MODE>(a, g, stream);
     default:
-      set_error("window_attn (tcgen05): head_dim %d is not instantiated (48, 64, 96, 128, 192)", g.C / g.heads);
+      set_error("window_attn (tcgen05): head_dim %d is not instantiated (48, 64, 96, 128, 192, 256)", g.C / g.heads);
       return SWINB200_ERR_UNSUPPORTED;
   }
 }
 
 }  // namespace
 
-bool attn_gen_supports(int head_dim) { return head_dim == 48 || head_dim == 64 || head_dim == 96 || head_dim == 128 || head_dim == 192; }
+bool attn_gen_supports(int head_dim) {
+  return head_dim == 48 || head_dim == 64 || head_dim == 96 || head_dim == 128 || head_dim == 192 || head_dim == 256;
+}
 
 int attn_tcgen05_gen_fwd(const void* qkv, const float* scale, const float* bias, void* o, float* lse, const AttnGeom& g, cudaStream_t stream) {
   GenArgs a{};

@@ -370,7 +370,9 @@ __device__ __forceinline__ void lnb_mbar_wait(uint64_t* bar, uint32_t parity) {
   }
 }
 
-template <typename T>
+// NJ: 256-channel chunks per row in pass 1 (4: C <= 1024, gamma held in registers; 8: C <= 2048, gamma re-read through L1 --
+// 64 more registers would spill at two CTAs per SM)
+template <typename T, int NJ>
 __global__ void __launch_bounds__(256, 2) ln_residual_bwd_kernel(const float* __restrict__ dx, const T* __restrict__ z,
                                                                  const float* __restrict__ stats, const float* __restrict__ gamma,
                                                                  const float* __restrict__ sample_scale, T* __restrict__ dz,
@@ -414,13 +416,16 @@ __global__ void __launch_bounds__(256, 2) ln_residual_bwd_kernel(const float* __
 #pragma unroll
   for (int e = 0; e < 8; ++e) { gm2[e] = 0.f; a_g[e] = 0.f; a_b[e] = 0.f; a_z[e] = 0.f; }
   if (p2_active) ld8(gamma + c2, gm2);
-  // pass-1 ownership: lane holds channels lane*8 + 256*j (j < 4) of every row its warp visits
-  float gm1[4][8];
+  // pass-1 ownership: lane holds channels lane*8 + 256*j (j < NJ) of every row its warp visits
+  constexpr bool kGammaRegs = NJ <= 4;
+  float gm1[kGammaRegs ? NJ : 1][8];
+  if constexpr (kGammaRegs) {
 #pragma unroll
-  for (int j = 0; j < 4; ++j) {
+    for (int j = 0; j < NJ; ++j) {
 #pragma unroll
-    for (int e = 0; e < 8; ++e) gm1[j][e] = 0.f;
-    if (lane * 8 + j * 256 < C) ld8(gamma + lane * 8 + j * 256, gm1[j]);
+      for (int e = 0; e < 8; ++e) gm1[j][e] = 0.f;
+      if (lane * 8 + j * 256 < C) ld8(gamma + lane * 8 + j * 256, gm1[j]);
+    }
   }
 
   int it = 0;
@@ -442,15 +447,22 @@ __global__ void __launch_bounds__(256, 2) ln_residual_bwd_kernel(const float* __
       const int row = r0 + rr;
       float A = 0.f, Bq = 0.f;
 #pragma unroll
-      for (int j = 0; j < 4; ++j) {
+      for (int j = 0; j < NJ; ++j) {
         const int c = lane * 8 + j * 256;
         if (c < C) {
           float d8[8], z8[8];
           ld8(dxt + (size_t)rr * C + c, d8);
           ld8(zt + (size_t)rr * C + c, z8);
+          float gj[8];
+          if constexpr (kGammaRegs) {
+#pragma unroll
+            for (int e = 0; e < 8; ++e) gj[e] = gm1[j][e];
+          } else {
+            ld8(gamma + c, gj);
+          }
 #pragma unroll
           for (int e = 0; e < 8; ++e) {
-            const float g = d8[e] * gm1[j][e];
+            const float g = d8[e] * gj[e];
             A += g;
             Bq = fmaf(g, z8[e], Bq);
           }
@@ -868,7 +880,11 @@ static int launch_ln_fwd(const T* z, const float* x_in, const float* gamma, cons
     case 2: SWB_LN_FWD(2); break;
     case 3: SWB_LN_FWD(3); break;
     case 4: SWB_LN_FWD(4); break;
-    default: set_error("ln_residual_fwd: C=%d > 1024 unsupported", C); return SWINB200_ERR_UNSUPPORTED;
+    case 5: SWB_LN_FWD(5); break;          // 5..8: embed_dim up to 2048 (the e2048 config), 128 row values per lane
+    case 6: SWB_LN_FWD(6); break;
+    case 7: SWB_LN_FWD(7); break;
+    case 8: SWB_LN_FWD(8); break;
+    default: set_error("ln_residual_fwd: C=%d > 2048 unsupported", C); return SWINB200_ERR_UNSUPPORTED;
   }
 #undef SWB_LN_FWD
   SWB_LAUNCH_CHECK();
@@ -1100,14 +1116,19 @@ static int launch_ln_bwd(const float* dx, const T* z, const float* stats, const 
     return SWINB200_ERR_UNSUPPORTED;
   }
   const size_t smem = (size_t)TR * per_row + (size_t)TR * 16 + 64;
-  static bool configured = false;
-  if (!configured) {
-    SWB_CUDA(cudaFuncSetAttribute(ln_residual_bwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-    configured = true;
+  const bool wide = C > 1024;
+  static bool configured[2] = {false, false};
+  if (!configured[wide]) {
+    SWB_CUDA(cudaFuncSetAttribute(wide ? ln_residual_bwd_kernel<T, 8> : ln_residual_bwd_kernel<T, 4>,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+    configured[wide] = true;
   }
   const int ntiles = (rows + TR - 1) / TR;
   const int blocks = max(1, min(ntiles, 2 * sm_count()));
-  ln_residual_bwd_kernel<T><<<blocks, 256, smem, s>>>(dx, z, stats, gamma, ss, dz, dgamma, dbeta, dbias_prev, rows, C, rps, TR);
+  if (wide)
+    ln_residual_bwd_kernel<T, 8><<<blocks, 256, smem, s>>>(dx, z, stats, gamma, ss, dz, dgamma, dbeta, dbias_prev, rows, C, rps, TR);
+  else
+    ln_residual_bwd_kernel<T, 4><<<blocks, 256, smem, s>>>(dx, z, stats, gamma, ss, dz, dgamma, dbeta, dbias_prev, rows, C, rps, TR);
   SWB_LAUNCH_CHECK();
   return SWINB200_OK;
 }

@@ -392,13 +392,13 @@ class SwinTransformerV2Cr(nn.Module):
         window_size = tuple([s // img_window_ratio for s in img_size]) if window_size is None else to_2tuple(window_size)
         if patch_size != 4:
             raise NotImplementedError("the kernels are specialised for patch_size 4 (every reference config)")
-        # kernel limits, checked here rather than at the first forward: the LayerNorm kernels hold a row in registers
-        # (C <= 1024) and the attention kernels are instantiated for head_dim <= 192.  The one shipped config beyond them is
-        # swin_73var_geo_depth24_e2048_mlp2_chweight_invar (embed_dim 2048, head_dim 256) -- see DESIGN.md section 7.
-        if embed_dim > 1024 or embed_dim % 8 != 0:
-            raise NotImplementedError(f"embed_dim {embed_dim}: the B200 kernels support multiples of 8 up to 1024")
-        if embed_dim % num_heads[0] != 0 or (embed_dim // num_heads[0]) % 8 != 0 or embed_dim // num_heads[0] > 192:
-            raise NotImplementedError(f"head_dim {embed_dim / num_heads[0]:g}: the attention kernels support multiples of 8 up to 192")
+        # kernel limits, checked here rather than at the first forward: the LayerNorm forward holds a row in registers
+        # (C <= 2048) and the attention kernels are instantiated for head_dim <= 256.  The largest shipped config,
+        # swin_73var_geo_depth24_e2048_mlp2_chweight_invar (embed_dim 2048, 8 heads of 256), sits on both limits.
+        if embed_dim > 2048 or embed_dim % 8 != 0:
+            raise NotImplementedError(f"embed_dim {embed_dim}: the B200 kernels support multiples of 8 up to 2048")
+        if embed_dim % num_heads[0] != 0 or (embed_dim // num_heads[0]) % 8 != 0 or embed_dim // num_heads[0] > 256:
+            raise NotImplementedError(f"head_dim {embed_dim / num_heads[0]:g}: the attention kernels support multiples of 8 up to 256")
         self.patch_size = patch_size
         self.img_size = img_size
         self.window_size = window_size

@@ -318,15 +318,15 @@ def shift_mask(H, W, Wh, Ww, s0, s1, device) -> torch.Tensor:
     return mask
 
 
-TCGEN05_HEAD_DIMS = (48, 64, 96, 128, 192)
+TCGEN05_HEAD_DIMS = (48, 64, 96, 128, 192, 256)
 
 
 def attn_backend_for(mode: ComputeMode, C: int, heads: int, Wh: int, Ww: int) -> int:
-    """bf16 mode runs window attention on the tcgen05 kernels for head_dim 48 / 64 / 96 / 128 / 192 and any window size:
-    the tuned persistent kernels for head_dim 96 with up to 176 (padded) tokens per window -- every shipped config, 9x18 =
-    162 -- and the tiled flash-style kernels (csrc/attn_tc_gen.cu) for everything else (BASELINE config 5).  Other head
-    dims and the fp32 validation mode run on the CUDA-core kernels; this is a dispatch on the problem shape decided up
-    front, not an error fallback."""
+    """bf16 mode runs window attention on the tcgen05 kernels for head_dim 48 / 64 / 96 / 128 / 192 / 256 and any window
+    size: the tuned persistent kernels for head_dim 96 with up to 176 (padded) tokens per window -- the 9x18 = 162 headline
+    config -- and the tiled flash-style kernels (csrc/attn_tc_gen.cu) for everything else (BASELINE config 5, the e2048 /
+    head_dim-256 config).  Other head dims and the fp32 validation mode run on the CUDA-core kernels; this is a dispatch on
+    the problem shape decided up front, not an error fallback."""
     if mode.attn_backend == BACKEND_TCGEN05 and C // heads in TCGEN05_HEAD_DIMS:
         return BACKEND_TCGEN05
     return BACKEND_SIMT
