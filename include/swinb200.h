@@ -218,6 +218,54 @@ int swinb200_adam_step(int n_tensors, void* const* params, const void* const* gr
                        double beta1, double beta2, double eps, double weight_decay, long long step,
                        const float* grad_scale, const float* found_inf, void* stream);
 
+/* ---- deterministic mode ---------------------------------------------------------------------------------
+ * Bitwise-reproducible versions of every entry point above whose float sums would otherwise depend on the order in which
+ * CTAs or warps finish (atomics).  Each writes its partial sums with plain stores into caller-owned scratch `part`
+ * (part_floats floats, fp32, 16-byte aligned), one slot per split / statically assigned CTA / row block / (sample,
+ * window, head) item, and then adds the slots in slot order with swinb200_ordered_reduce.  Outputs are defined exactly as
+ * by the plain entry points (accumulating outputs are still added to, once).  Same build, same GPU model, same inputs ->
+ * the same bits.  NULL or short scratch: SWINB200_ERR_INVALID_ARG.  The library still allocates nothing.
+ *
+ * swinb200_ordered_reduce: out[i] = (accumulate ? out[i] : 0) + sum_{p < n_part} sum_{j < inner} part[p*stride + i*inner + j],
+ *   i < n, summed in exactly that order (the fixed-order second stage of every entry below; stride >= n * inner).
+ * swinb200_gemm_wgrad_det: D[M,N] += sum_k A(k,m) B(k,n), A stored (K, M), B stored (K, N), D dense (ldd = N) fp32 -- the
+ *   split-K weight gradient of swinb200_gemm(a_major 1, b_major 1, EPI_F32, accumulate).  tcgen05: every split TMA-stores
+ *   its tile into its own slice of a [S, M, N] scratch; scratch >= split_k*M*N floats.  SIMT: the CUDA-core GEMM does not
+ *   split K (one thread adds each element once), scratch unused and may be NULL.
+ * swinb200_linear_wgrad_det: swinb200_linear_wgrad with dW dense (lddw = n_in); scratch >= split_k*(n_out*n_in + n_out).
+ * swinb200_ln_residual_bwd_det: swinb200_ln_residual_bwd; scratch >= 3*C*256*max(1, 2048/C) floats (integer division):
+ *   at most 256 CTAs, each leaving one [3, C] row per group of threads that covers all channels.
+ * swinb200_colsum_det: swinb200_colsum; scratch >= cols*min(ceil(rows/64), 256).
+ * swinb200_latw_l2_fwd_det / _l1_fwd_det / _acc_det: the loss / metric entry points; scratch >= 2*B*C*H (L2, L1) and
+ *   3*B*C*H (ACC) floats (at most one row block per image row).
+ * swinb200_window_attn_bwd_det: swinb200_window_attn_bwd; with nW = (H/Wh)*(W/Ww), L = Wh*Ww and items = B*nW*heads,
+ *   scratch >= items*(4*ceil(L/128) + (dbias ? L*L : 0)) floats: d(scale) slots per item, then one (L, L) d(bias) slice
+ *   per item (336 MB at 9x18 windows / 8 heads / B = 1 on the 180x360 token grid with a bias table).  The tcgen05 kernels
+ *   selected by SWINB200_ATTN_BWD=1/2, a NULL ws or operands that are not 16-byte aligned have no deterministic version:
+ *   SWINB200_ERR_UNSUPPORTED, nothing launched. */
+int swinb200_ordered_reduce(const float* part, int n_part, long long stride, long long n, int inner, float* out, int accumulate,
+                            void* stream);
+int swinb200_gemm_wgrad_det(int backend, int M, int N, int K, const void* A, int lda, const void* B, int ldb, int in_dtype,
+                            float* D, int split_k, float* part, long long part_floats, void* stream);
+int swinb200_linear_wgrad_det(int backend, int n_out, int n_in, int T, const void* dY, int ldy, const void* X, int ldx,
+                              float* dW, float* dbias, int split_k, float* part, long long part_floats, void* stream);
+int swinb200_ln_residual_bwd_det(const float* dx, const void* z, int act_dtype, const float* stats, const float* gamma,
+                                 const float* sample_scale, void* dz, float* dgamma, float* dbeta, float* dbias_prev, int rows,
+                                 int C, int rows_per_sample, float* part, long long part_floats, void* stream);
+int swinb200_colsum_det(const void* x, int act_dtype, float* out, int rows, int cols, int ld, float* part, long long part_floats,
+                        void* stream);
+int swinb200_latw_l2_fwd_det(const float* prd, const float* tar, const float* qw, const float* chw, int relative, int squared,
+                             float* num, float* den, float* loss, int B, int C, int H, int W, float* part, long long part_floats,
+                             void* stream);
+int swinb200_latw_l1_fwd_det(const float* prd, const float* tar, const float* qw, const float* chw, int relative, float* sums,
+                             float* loss, int B, int C, int H, int W, float* part, long long part_floats, void* stream);
+int swinb200_latw_acc_det(const float* prd, const float* tar, const float* qw, float* sums, float* acc, int B, int C, int H,
+                          int W, float* part, long long part_floats, void* stream);
+int swinb200_window_attn_bwd_det(int backend, const void* qkv, int act_dtype, const float* inv_norm, const float* scale,
+                                 const float* bias, const void* o, const void* d_o, const float* lse, void* dqkv, float* dscale,
+                                 float* dbias, float* ws, int B, int H, int W, int C, int heads, int Wh, int Ww, int s0, int s1,
+                                 float* part, long long part_floats, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -18,6 +18,7 @@ BACKEND_SIMT, BACKEND_TCGEN05 = 0, 1
 
 _P = c_void_p
 _I = c_int
+_LL = ctypes.c_longlong
 
 # name -> argtypes, exactly the prototypes of include/swinb200.h
 PROTOTYPES = {
@@ -48,13 +49,29 @@ PROTOTYPES = {
     "swinb200_latw_l2_bwd": [_P, _P, _P, _P, _P, _P, _P, _I, _I, _P, _I, _I, _I, _I, _P],
     "swinb200_adam_step": [_I, _P, _P, _P, _P, _P, _P, ctypes.c_double, ctypes.c_double, ctypes.c_double, ctypes.c_double,
                            ctypes.c_double, ctypes.c_longlong, _P, _P, _P],
+    # deterministic mode: caller-owned scratch (pointer, size in floats) before the stream
+    "swinb200_ordered_reduce": [_P, _I, _LL, _LL, _I, _P, _I, _P],
+    "swinb200_gemm_wgrad_det": [_I, _I, _I, _I, _P, _I, _P, _I, _I, _P, _I, _P, _LL, _P],
+    "swinb200_linear_wgrad_det": [_I, _I, _I, _I, _P, _I, _P, _I, _P, _P, _I, _P, _LL, _P],
+    "swinb200_ln_residual_bwd_det": [_P, _P, _I, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P, _LL, _P],
+    "swinb200_colsum_det": [_P, _I, _P, _I, _I, _I, _P, _LL, _P],
+    "swinb200_latw_l2_fwd_det": [_P, _P, _P, _P, _I, _I, _P, _P, _P, _I, _I, _I, _I, _P, _LL, _P],
+    "swinb200_latw_l1_fwd_det": [_P, _P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _P, _LL, _P],
+    "swinb200_latw_acc_det": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _P, _LL, _P],
+    "swinb200_window_attn_bwd_det": [_I, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _LL,
+                                     _P],
 }
 
 _lib = None
 
 
+ERR_INVALID_ARG, ERR_CUDA, ERR_UNSUPPORTED = 1, 2, 3
+
+
 class SwinB200Error(RuntimeError):
-    pass
+    def __init__(self, msg: str, code: int = 0):
+        super().__init__(msg)
+        self.code = code        # SWINB200_ERR_* of a failed call, 0 for errors raised on the Python side
 
 
 def load() -> ctypes.CDLL:
@@ -98,4 +115,4 @@ def call(name: str, *args) -> None:
         rc = getattr(lib, name)(*args)
     if rc != 0:
         msg = lib.swinb200_last_error().decode("utf-8", "replace")
-        raise SwinB200Error(f"{name} failed (code {rc}): {msg}")
+        raise SwinB200Error(f"{name} failed (code {rc}): {msg}", rc)

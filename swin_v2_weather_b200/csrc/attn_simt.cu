@@ -118,7 +118,9 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_fwd_kernel(const T*
 // ------------------------------------------------------------------------------------------------
 // backward
 // ------------------------------------------------------------------------------------------------
-template <typename T, bool GLOBAL_KV>
+// DET (deterministic mode): dscale is a (B*nW*heads) scratch receiving the CTA's d(scale) at its item index, dbias a
+// (B*nW*heads, L, L) scratch receiving the item's slice (each (i, j) is visited by exactly one lane of the CTA)
+template <typename T, bool GLOBAL_KV, bool DET = false>
 __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T* __restrict__ qkv, const float* __restrict__ inv_norm,
                                                                         const float* __restrict__ scale_p, const float* __restrict__ bias,
                                                                         const T* __restrict__ o, const T* __restrict__ d_o,
@@ -210,7 +212,11 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T*
       const float ds = p * (dpv - dsum);
       myds[j] = ds;
       dsc_acc += ds * cs;
-      if (dbias) atomicAdd(dbias + ((size_t)head * L + i) * L + j, ds);
+      if constexpr (DET) {
+        if (dbias) dbias[((size_t)blockIdx.x * L + i) * L + j] = ds;
+      } else {
+        if (dbias) atomicAdd(dbias + ((size_t)head * L + i) * L + j, ds);
+      }
     }
     __syncwarp();
     // dqhat, then back through the normalisation: dq = inv_norm * (dqhat - qhat * <qhat, dqhat>)
@@ -292,7 +298,8 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_bwd_kernel(const T*
   if (threadIdx.x == 0) {
     float s = 0.f;
     for (int i = 0; i < kAttnWarps; ++i) s += redsc[i];
-    atomicAdd(dscale + head, s);
+    if constexpr (DET) dscale[blockIdx.x] = s;
+    else atomicAdd(dscale + head, s);
   }
 }
 
@@ -326,12 +333,26 @@ static int launch_fwd(const T* qkv, const float* scale, const float* bias, T* o,
 
 template <typename T>
 static int launch_bwd(const T* qkv, const float* inv_norm, const float* scale, const float* bias, const T* o, const T* d_o,
-                      const float* lse, T* dqkv, float* dscale, float* dbias, const WinGeom& g, cudaStream_t s) {
+                      const float* lse, T* dqkv, float* dscale, float* dbias, const WinGeom& g, cudaStream_t s,
+                      float* det_part = nullptr) {
   const bool global_kv = attn_smem_bytes<T>(g, true, false) > 227 * 1024;
   const size_t smem = attn_smem_bytes<T>(g, true, global_kv);
   if (smem > 227 * 1024) {
     set_error("window_attn_bwd (CUDA-core back end): window %dx%d, head_dim %d needs %zu B of shared memory", g.Wh, g.Ww, g.d(), smem);
     return SWINB200_ERR_UNSUPPORTED;
+  }
+  if (det_part != nullptr) {
+    const int bw = g.B * g.nW(), L = g.L();
+    const long long dbias_n = (long long)g.heads * L * L;
+    // same slot layout as the tcgen05 back ends: the d(scale) slots first, then the per-item d(bias) slices
+    float* dbias_part = (dbias != nullptr) ? det_part + (long long)bw * g.heads * 4 * ((L + 127) / 128) : nullptr;
+    auto kernel = global_kv ? attn_simt_bwd_kernel<T, true, true> : attn_simt_bwd_kernel<T, false, true>;
+    SWB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<bw * g.heads, kAttnWarps * 32, smem, s>>>(qkv, inv_norm, scale, bias, o, d_o, lse, dqkv, det_part, dbias_part, g);
+    SWB_LAUNCH_CHECK();
+    if (int e = ordered_reduce(det_part, bw, g.heads, g.heads, 1, dscale, 1, s)) return e;
+    if (dbias != nullptr) return ordered_reduce(dbias_part, bw, dbias_n, dbias_n, 1, dbias, 1, s);
+    return SWINB200_OK;
   }
   auto kernel = global_kv ? attn_simt_bwd_kernel<T, true> : attn_simt_bwd_kernel<T, false>;
   SWB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -344,7 +365,7 @@ int attn_tcgen05_fwd(const void* qkv, const float* scale, const float* bias, voi
                      int heads, int Wh, int Ww, int s0, int s1, cudaStream_t stream);
 int attn_tcgen05_bwd(const void* qkv, const float* inv_norm, const float* scale, const float* bias, const void* o,
                      const void* d_o, const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, int B, int H, int W,
-                     int C, int heads, int Wh, int Ww, int s0, int s1, cudaStream_t stream);
+                     int C, int heads, int Wh, int Ww, int s0, int s1, cudaStream_t stream, float* det_part = nullptr);
 
 static int check_geom(const char* who, int B, int H, int W, int C, int heads, int Wh, int Ww, int s0, int s1) {
   SWB_CHECK_ARG(B > 0 && H > 0 && W > 0 && C > 0 && heads > 0, "%s: bad shape", who);
@@ -395,4 +416,30 @@ extern "C" int swinb200_window_attn_bwd(int backend, const void* qkv, int act_dt
   if (act_dtype == SWINB200_F32)
     return launch_bwd<float>((const float*)qkv, inv_norm, scale, bias, (const float*)o, (const float*)d_o, lse, (float*)dqkv, dscale, dbias, g, s);
   SWB_CHECK_ARG(false, "window_attn_bwd: bad act_dtype %d", act_dtype);
+}
+
+extern "C" int swinb200_window_attn_bwd_det(int backend, const void* qkv, int act_dtype, const float* inv_norm, const float* scale,
+                                            const float* bias, const void* o, const void* d_o, const float* lse, void* dqkv,
+                                            float* dscale, float* dbias, float* ws, int B, int H, int W, int C, int heads, int Wh,
+                                            int Ww, int s0, int s1, float* part, long long part_floats, void* stream) {
+  SWB_CHECK_ARG(qkv && inv_norm && scale && o && d_o && lse && dqkv && dscale, "window_attn_bwd_det: null pointer");
+  SWB_CHECK_ARG(dbias == nullptr || bias != nullptr, "window_attn_bwd_det: dbias needs the bias table");
+  if (int e = check_geom("window_attn_bwd_det", B, H, W, C, heads, Wh, Ww, s0, s1)) return e;
+  const WinGeom g{B, H, W, C, heads, Wh, Ww, s0, s1};
+  const long long items = (long long)B * g.nW() * heads, L = g.L();
+  const long long need = items * (4 * ((L + 127) / 128) + (dbias != nullptr ? L * L : 0));
+  SWB_CHECK_ARG(part != nullptr && part_floats >= need, "window_attn_bwd_det: scratch of %lld floats required, got %lld", need, part_floats);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (backend == SWINB200_GEMM_TCGEN05) {
+    SWB_CHECK_ARG(act_dtype == SWINB200_BF16, "window_attn_bwd_det: the tcgen05 back end needs bf16 activations");
+    return attn_tcgen05_bwd(qkv, inv_norm, scale, bias, o, d_o, lse, dqkv, dscale, dbias, ws, B, H, W, C, heads, Wh, Ww, s0, s1, s, part);
+  }
+  SWB_CHECK_ARG(backend == SWINB200_GEMM_SIMT, "window_attn_bwd_det: unknown backend %d", backend);
+  if (act_dtype == SWINB200_BF16)
+    return launch_bwd<__nv_bfloat16>((const __nv_bfloat16*)qkv, inv_norm, scale, bias, (const __nv_bfloat16*)o, (const __nv_bfloat16*)d_o,
+                                     lse, (__nv_bfloat16*)dqkv, dscale, dbias, g, s, part);
+  if (act_dtype == SWINB200_F32)
+    return launch_bwd<float>((const float*)qkv, inv_norm, scale, bias, (const float*)o, (const float*)d_o, lse, (float*)dqkv, dscale, dbias,
+                             g, s, part);
+  SWB_CHECK_ARG(false, "window_attn_bwd_det: bad act_dtype %d", act_dtype);
 }

@@ -1592,7 +1592,7 @@ int attn_make_window_tmap(CUtensorMap* m, const void* base, int B, int H, int W,
 // kernel does everything in place.
 int attn_tcgen05_bwd(const void* qkv, const float* inv_norm, const float* scale, const float* bias, const void* o,
                      const void* d_o, const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, int B, int H, int W,
-                     int C, int heads, int Wh, int Ww, int s0, int s1, cudaStream_t stream) {
+                     int C, int heads, int Wh, int Ww, int s0, int s1, cudaStream_t stream, float* det_part) {
   AttnGeom g;
   if (int e = attn_make_geom(g, B, H, W, C, heads, Wh, Ww, s0, s1)) return e;
   static int variant = -1;
@@ -1601,10 +1601,15 @@ int attn_tcgen05_bwd(const void* qkv, const float* inv_norm, const float* scale,
     variant = e ? atoi(e) : 3;   // 1 = one CTA per (window, head);  2 = persistent two-sweep kernel;  3 = single-pass warp-specialised;  4 = generic
   }
   if (!attn_is_specialised(g) || variant == 4)
-    return attn_tcgen05_gen_bwd(qkv, inv_norm, scale, bias, o, d_o, lse, dqkv, dscale, dbias, ws, g, stream);
+    return attn_tcgen05_gen_bwd(qkv, inv_norm, scale, bias, o, d_o, lse, dqkv, dscale, dbias, ws, g, stream, det_part);
   const bool aligned = ((uintptr_t)qkv % 16 == 0) && ((uintptr_t)d_o % 16 == 0);
   if (variant == 3 && ws != nullptr && aligned)
-    return attn_tcgen05_bwd3(qkv, inv_norm, scale, bias, o, d_o, lse, dqkv, dscale, dbias, ws, g, stream);
+    return attn_tcgen05_bwd3(qkv, inv_norm, scale, bias, o, d_o, lse, dqkv, dscale, dbias, ws, g, stream, det_part);
+  if (det_part != nullptr) {
+    set_error("window_attn_bwd: the one-CTA-per-window and two-sweep kernels (SWINB200_ATTN_BWD=1/2, no workspace or unaligned "
+              "operands) have no deterministic version");
+    return SWINB200_ERR_UNSUPPORTED;
+  }
   if (variant == 1 || ws == nullptr || !aligned) {
     using SM = BwdSmem<96>;
     static bool configured = false;

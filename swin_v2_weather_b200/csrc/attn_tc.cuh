@@ -131,13 +131,19 @@ __device__ __forceinline__ void scatter_rows(const unsigned char* stage, int nro
 
 bool attn_gen_supports(int head_dim);
 int attn_tcgen05_gen_fwd(const void* qkv, const float* scale, const float* bias, void* o, float* lse, const AttnGeom& g, cudaStream_t stream);
+// det_part (deterministic mode, see swinb200_window_attn_bwd_det): attn_det_dscale_slots(g) d(scale) slots, followed (with a
+// bias table) by the (B*nW*heads, L, L) per-item d(bias) slices
 int attn_tcgen05_gen_bwd(const void* qkv, const float* inv_norm, const float* scale, const float* bias, const void* o, const void* d_o,
-                         const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, const AttnGeom& g, cudaStream_t stream);
+                         const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, const AttnGeom& g, cudaStream_t stream,
+                         float* det_part = nullptr);
 int attn_make_geom(AttnGeom& g, int B, int H, int W, int C, int heads, int Wh, int Ww, int s0, int s1);
 int attn_make_window_tmap(CUtensorMap* m, const void* base, int B, int H, int W, int channels, int Wh, int Ww);
 int attn_tcgen05_fwd4(const void* qkv, const float* scale, const float* bias, void* o, float* lse, const AttnGeom& g, cudaStream_t stream);
 int attn_tcgen05_fwd3(const void* qkv, const float* scale, const float* bias, void* o, float* lse, const AttnGeom& g, cudaStream_t stream);
 int attn_tcgen05_bwd3(const void* qkv, const float* inv_norm, const float* scale, const float* bias, const void* o, const void* d_o,
-                      const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, const AttnGeom& g, cudaStream_t stream);
+                      const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, const AttnGeom& g, cudaStream_t stream,
+                      float* det_part = nullptr);
+// one slot per (item, 128-row tile, warp of attn_tc_gen.cu) -- enough for every back end
+inline long long attn_det_dscale_slots(const AttnGeom& g) { return (long long)g.B * g.nW * g.heads * 4 * ((g.L + 127) / 128); }
 
 }  // namespace swinb200

@@ -91,7 +91,10 @@ __device__ __forceinline__ unsigned char* slab_at(unsigned char* slab, int rr, i
   return slab + rr * 64 + ((p ^ ((rr >> 1) & 3)) << 4);
 }
 
-template <int D, bool kProf>
+// DET (deterministic mode): dscale is a (B*nW*heads) scratch that receives each item's d(scale), folded over the 12 compute
+// warps in warp order (two 16-slot buffers in the per-head area, alternating per item); dbias is a (B*nW*heads, L, L)
+// scratch in which each item writes its own slice with plain stores.  Items are statically assigned (item += gridDim.x).
+template <int D, bool kProf, bool DET = false>
 __global__ void __launch_bounds__(kB3Threads, 1)
 attn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constant__ CUtensorMap tm_do,
                     const float* __restrict__ Dpre, const __nv_bfloat16* __restrict__ qkv, const float* __restrict__ inv_norm,
@@ -428,6 +431,13 @@ attn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_con
       const float scale = scale_p[head];
       const float scale_l2 = scale * kLog2e;
       named_bar_sync(1, kB3Compute);      // this item's per-slot rows / tok (written during the previous item) are visible
+      if constexpr (DET) {
+        if (tid == 0 && it > 0) {           // the previous item's warp sums are complete
+          float v = 0.f;
+          for (int w8 = 0; w8 < kB3Compute / 32; ++w8) v += dsc_heads[((it - 1) & 1) * 16 + w8];
+          dscale[item - gridDim.x] = v;
+        }
+      }
       // reciprocal norms of this thread's rows, taken now: the per-slot arrays are refilled for the next item before the
       // last epilogues of this one run
       float my_ink[2], my_inq[2];
@@ -510,7 +520,11 @@ attn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_con
                 ds[j] = (key_ok && qi < L) ? p * (as_f(pv[j]) - Dv[qi]) : 0.f;
                 part = fmaf(ds[j], cosv, part);
                 partc = fmaf(ds[j], s_ec[qi], partc);
-                if (dbias != nullptr && key_ok && qi < L) atomicAdd(dbias + ((size_t)head * L + qi) * L + jk, ds[j]);
+                if constexpr (DET) {
+                  if (dbias != nullptr && key_ok && qi < L) dbias[((size_t)item * L + qi) * L + jk] = ds[j];
+                } else {
+                  if (dbias != nullptr && key_ok && qi < L) atomicAdd(dbias + ((size_t)head * L + qi) * L + jk, ds[j]);
+                }
               }
               tmem_st_32x4(t_lane + kColP + cb / 2, pack8f(pp));
               if (row_exists) *reinterpret_cast<uint4*>(sDS + (cb / 8) * SM::kDSCS + jk * 16) = pack8f(ds);
@@ -643,14 +657,26 @@ attn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_con
           for (int i = 0; i < 4; ++i) mbar_arrive(&full[i]);
       }
       dsc_acc = warp_sum(dsc_acc);
-      if (lane == 0) atomicAdd(&dsc_heads[head], dsc_acc);
+      if constexpr (DET) {
+        if (lane == 0) dsc_heads[(it & 1) * 16 + warp] = dsc_acc;
+      } else {
+        if (lane == 0) atomicAdd(&dsc_heads[head], dsc_acc);
+      }
       const int tmp = kb; kb = vb; vb = tmp;
       SWB_ACC(7);
     }
     named_bar_sync(1, kB3Compute);
-    if (tid < g.heads) {
-      const float v = dsc_heads[tid];
-      if (v != 0.f) atomicAdd(dscale + tid, v);
+    if constexpr (DET) {
+      if (tid == 0 && it > 0) {
+        float v = 0.f;
+        for (int w8 = 0; w8 < kB3Compute / 32; ++w8) v += dsc_heads[((it - 1) & 1) * 16 + w8];
+        dscale[first + (it - 1) * gridDim.x] = v;
+      }
+    } else {
+      if (tid < g.heads) {
+        const float v = dsc_heads[tid];
+        if (v != 0.f) atomicAdd(dscale + tid, v);
+      }
     }
     if (kProf && g_phase_buf3 != nullptr && tid == 0 && blockIdx.x < 4096)
       for (int i = 0; i < 16; ++i) g_phase_buf3[blockIdx.x * 16 + i] = ph_acc[i];
@@ -696,12 +722,14 @@ int attn_set_phase_buffer3(long long* buf) {
 }
 
 int attn_tcgen05_bwd3(const void* qkv, const float* inv_norm, const float* scale, const float* bias, const void* o, const void* d_o,
-                      const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, const AttnGeom& g, cudaStream_t stream) {
+                      const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, const AttnGeom& g, cudaStream_t stream,
+                      float* det_part) {
   using SM = Bwd3Smem<96>;
   static bool configured = false;
   if (!configured) {
     SWB_CUDA(cudaFuncSetAttribute(attn_tc_bwd3_kernel<96, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM::kBytes));
     SWB_CUDA(cudaFuncSetAttribute(attn_tc_bwd3_kernel<96, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM::kBytes));
+    SWB_CUDA(cudaFuncSetAttribute(attn_tc_bwd3_kernel<96, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM::kBytes));
     configured = true;
   }
   CUtensorMap tm_qkv, tm_do;
@@ -714,6 +742,17 @@ int attn_tcgen05_bwd3(const void* qkv, const float* inv_norm, const float* scale
   const int grid = min(g.B * g.nW * g.heads, sm_count());
   static int dbg_env = -1;   // bring-up timing experiments (wrong results): SWINB200_BWD3_DEBUG bit mask, see the kernel
   if (dbg_env < 0) { const char* e = getenv("SWINB200_BWD3_DEBUG"); dbg_env = e ? atoi(e) : 0; }
+  if (det_part != nullptr) {
+    const int bw = g.B * g.nW;
+    float* dbias_part = (dbias != nullptr) ? det_part + attn_det_dscale_slots(g) : nullptr;
+    attn_tc_bwd3_kernel<96, false, true><<<grid, kB3Threads, SM::kBytes, stream>>>(tm_qkv, tm_do, ws, (const __nv_bfloat16*)qkv, inv_norm,
+                                                                                   scale, bias, (const __nv_bfloat16*)d_o, lse,
+                                                                                   (__nv_bfloat16*)dqkv, det_part, dbias_part, g, dbg_env);
+    SWB_LAUNCH_CHECK();
+    if (int e = ordered_reduce(det_part, bw, g.heads, g.heads, 1, dscale, 1, stream)) return e;
+    if (dbias != nullptr) return ordered_reduce(dbias_part, bw, (long long)g.heads * g.L * g.L, (long long)g.heads * g.L * g.L, 1, dbias, 1, stream);
+    return SWINB200_OK;
+  }
   if (g_prof3)
     attn_tc_bwd3_kernel<96, true><<<grid, kB3Threads, SM::kBytes, stream>>>(tm_qkv, tm_do, ws, (const __nv_bfloat16*)qkv, inv_norm, scale,
                                                                             bias, (const __nv_bfloat16*)d_o, lse, (__nv_bfloat16*)dqkv,

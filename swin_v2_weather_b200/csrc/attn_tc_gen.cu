@@ -88,7 +88,9 @@ __device__ __forceinline__ void tmem_st_32x16(uint32_t taddr, const float (&v)[1
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_1() { asm volatile("cp.async.wait_group 1;" ::: "memory"); }
 
-template <int D, int KT, int MODE, bool HAS_BIAS>
+// DET (deterministic mode): a.dscale holds one slot per (item, X tile, warp) and a.dbias one (L, L) slice per item, all
+// written with plain stores (every (query, key) of an item is visited by exactly one thread of the K pass)
+template <int D, int KT, int MODE, bool HAS_BIAS, bool DET = false>
 __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const AttnGeom g) {
   using CF = GenCfg<D, KT, MODE, HAS_BIAS>;
   constexpr float kLog2e = 1.4426950408889634f;
@@ -427,7 +429,11 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
           if (MODE != kModeBwdV) {
             const float d = (qi < L) ? p * (as_f(dp[j]) - dd[j]) : 0.f;
             ds[j] = d;
-            if (a.dbias != nullptr && row_ok && qi < L) atomicAdd(a.dbias + ((size_t)head * L + qi) * L + nx, d);
+            if constexpr (DET) {
+              if (a.dbias != nullptr && row_ok && qi < L) a.dbias[((size_t)item * L + qi) * L + nx] = d;
+            } else {
+              if (a.dbias != nullptr && row_ok && qi < L) atomicAdd(a.dbias + ((size_t)head * L + qi) * L + nx, d);
+            }
           }
         }
         if (MODE != kModeBwdK) tmem_st_32x8(t_lane + CF::kColS + c0 / 2, pack8(pp, 0), pack8(pp, 8));
@@ -546,7 +552,11 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
     __syncthreads();
     scatter(C3, head * D);
     dsc_acc = warp_sum(dsc_acc);
-    if (lane == 0 && dsc_acc != 0.f) atomicAdd(a.dscale + head, dsc_acc);
+    if constexpr (DET) {
+      if (lane == 0) a.dscale[((size_t)item * nX + xt) * 4 + warp] = dsc_acc;
+    } else {
+      if (lane == 0 && dsc_acc != 0.f) atomicAdd(a.dscale + head, dsc_acc);
+    }
   } else {
     if (MODE != kModeBwdK) {
       park(CF::kColAcc0, 1.f, false, 0.f, 1.f);  // dv
@@ -571,12 +581,12 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
   }
 }
 
-template <int D, int KT, int MODE, bool HAS_BIAS>
+template <int D, int KT, int MODE, bool HAS_BIAS, bool DET = false>
 int launch_gen_b(const GenArgs& a, const AttnGeom& g, cudaStream_t stream) {
   using CF = GenCfg<D, KT, MODE, HAS_BIAS>;
   static bool configured = false;
   if (!configured) {
-    SWB_CUDA(cudaFuncSetAttribute(attn_gen_kernel<D, KT, MODE, HAS_BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, CF::kBytes));
+    SWB_CUDA(cudaFuncSetAttribute(attn_gen_kernel<D, KT, MODE, HAS_BIAS, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, CF::kBytes));
     configured = true;
   }
   const long long ctas = (long long)g.B * g.nW * g.heads * ((g.L + 127) / 128);
@@ -584,36 +594,40 @@ int launch_gen_b(const GenArgs& a, const AttnGeom& g, cudaStream_t stream) {
     set_error("window_attn (tcgen05): %lld CTAs exceed the grid limit", ctas);
     return SWINB200_ERR_UNSUPPORTED;
   }
-  attn_gen_kernel<D, KT, MODE, HAS_BIAS><<<(unsigned)ctas, 128, CF::kBytes, stream>>>(a, g);
+  attn_gen_kernel<D, KT, MODE, HAS_BIAS, DET><<<(unsigned)ctas, 128, CF::kBytes, stream>>>(a, g);
   SWB_LAUNCH_CHECK();
   return SWINB200_OK;
 }
+// det: only the backward modes have a deterministic instantiation (the forward sums nothing across CTAs)
 template <int D, int KT, int MODE>
-int launch_gen(const GenArgs& a, const AttnGeom& g, cudaStream_t stream) {
+int launch_gen(const GenArgs& a, const AttnGeom& g, cudaStream_t stream, bool det = false) {
+  if constexpr (MODE != kModeFwd) {
+    if (det) return a.bias != nullptr ? launch_gen_b<D, KT, MODE, true, true>(a, g, stream) : launch_gen_b<D, KT, MODE, false, true>(a, g, stream);
+  }
   return a.bias != nullptr ? launch_gen_b<D, KT, MODE, true>(a, g, stream) : launch_gen_b<D, KT, MODE, false>(a, g, stream);
 }
 
 // head_dim 256: 206 KB of shared memory for the forward at KT = 64 and for backward A at KT = 32; backward B as the V pass
 // (KT = 64) followed by the K pass (KT = 32), 196 KB each; every one of them allocates 512 tensor-memory columns
 template <int MODE>
-int launch_gen_256(const GenArgs& a, const AttnGeom& g, cudaStream_t stream) {
+int launch_gen_256(const GenArgs& a, const AttnGeom& g, cudaStream_t stream, bool det) {
   if constexpr (MODE == kModeFwd) return launch_gen<256, 64, kModeFwd>(a, g, stream);
-  if constexpr (MODE == kModeBwdQ) return launch_gen<256, 32, kModeBwdQ>(a, g, stream);
+  if constexpr (MODE == kModeBwdQ) return launch_gen<256, 32, kModeBwdQ>(a, g, stream, det);
   if constexpr (MODE == kModeBwdKV) {
-    if (int e = launch_gen<256, 64, kModeBwdV>(a, g, stream)) return e;
-    return launch_gen<256, 32, kModeBwdK>(a, g, stream);
+    if (int e = launch_gen<256, 64, kModeBwdV>(a, g, stream, det)) return e;
+    return launch_gen<256, 32, kModeBwdK>(a, g, stream, det);
   }
 }
 
 template <int MODE>
-int dispatch_gen(const GenArgs& a, const AttnGeom& g, cudaStream_t stream) {
+int dispatch_gen(const GenArgs& a, const AttnGeom& g, cudaStream_t stream, bool det = false) {
   switch (g.C / g.heads) {
-    case 48: return launch_gen<48, 64, MODE>(a, g, stream);
-    case 64: return launch_gen<64, 64, MODE>(a, g, stream);
-    case 96: return launch_gen<96, 64, MODE>(a, g, stream);
-    case 128: return launch_gen<128, 64, MODE>(a, g, stream);
-    case 192: return launch_gen<192, 64, MODE>(a, g, stream);
-    case 256: return launch_gen_256<MODE>(a, g, stream);
+    case 48: return launch_gen<48, 64, MODE>(a, g, stream, det);
+    case 64: return launch_gen<64, 64, MODE>(a, g, stream, det);
+    case 96: return launch_gen<96, 64, MODE>(a, g, stream, det);
+    case 128: return launch_gen<128, 64, MODE>(a, g, stream, det);
+    case 192: return launch_gen<192, 64, MODE>(a, g, stream, det);
+    case 256: return launch_gen_256<MODE>(a, g, stream, det);
     default:
       set_error("window_attn (tcgen05): head_dim %d is not instantiated (48, 64, 96, 128, 192, 256)", g.C / g.heads);
       return SWINB200_ERR_UNSUPPORTED;
@@ -653,7 +667,8 @@ __global__ void __launch_bounds__(256) attn_gen_rowdot_kernel(const __nv_bfloat1
 }
 
 int attn_tcgen05_gen_bwd(const void* qkv, const float* inv_norm, const float* scale, const float* bias, const void* o, const void* d_o,
-                         const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, const AttnGeom& g, cudaStream_t stream) {
+                         const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, const AttnGeom& g, cudaStream_t stream,
+                         float* det_part) {
   if (ws == nullptr) {
     set_error("window_attn_bwd (tcgen05): a workspace of B*H*W*heads floats is required for this geometry");
     return SWINB200_ERR_INVALID_ARG;
@@ -665,8 +680,19 @@ int attn_tcgen05_gen_bwd(const void* qkv, const float* inv_norm, const float* sc
   GenArgs a{};
   a.qkv = (const __nv_bfloat16*)qkv; a.d_o = (const __nv_bfloat16*)d_o; a.inv_norm = inv_norm; a.scale = scale; a.bias = bias;
   a.Dpre = ws; a.lse = const_cast<float*>(lse); a.out = (__nv_bfloat16*)dqkv; a.dscale = dscale; a.dbias = dbias;
-  if (int e = dispatch_gen<kModeBwdQ>(a, g, stream)) return e;
-  return dispatch_gen<kModeBwdKV>(a, g, stream);
+  if (det_part == nullptr) {
+    if (int e = dispatch_gen<kModeBwdQ>(a, g, stream)) return e;
+    return dispatch_gen<kModeBwdKV>(a, g, stream);
+  }
+  const int bw = g.B * g.nW, slots = 4 * ((g.L + 127) / 128);
+  const long long dbias_n = (long long)g.heads * g.L * g.L;
+  a.dscale = det_part;
+  a.dbias = (dbias != nullptr) ? det_part + attn_det_dscale_slots(g) : nullptr;
+  if (int e = dispatch_gen<kModeBwdQ>(a, g, stream, true)) return e;
+  if (int e = dispatch_gen<kModeBwdKV>(a, g, stream, true)) return e;
+  if (int e = ordered_reduce(det_part, bw, (long long)g.heads * slots, g.heads, slots, dscale, 1, stream)) return e;
+  if (dbias != nullptr) return ordered_reduce(a.dbias, bw, dbias_n, dbias_n, 1, dbias, 1, stream);
+  return SWINB200_OK;
 }
 
 }  // namespace swinb200

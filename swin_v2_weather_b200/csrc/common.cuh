@@ -45,6 +45,11 @@ inline int sm_count() {
   return n;
 }
 
+// out[i] (+)= sum_{p < n_part} sum_{j < inner} part[p * stride + i * inner + j], summed in exactly that order and added once
+// into out: the second stage of every deterministic-mode reduction (determinism.cu)
+int ordered_reduce(const float* part, int n_part, long long stride, long long n, int inner, float* out, int accumulate,
+                   cudaStream_t stream);
+
 // LayerNorm + DropPath scale + residual operands of the fused proj / fc2 epilogue (SWINB200_EPI_BIAS_LN, gemm_tc.cu)
 struct GemmLnFuse {
   const float* x_in;

@@ -372,7 +372,8 @@ __device__ __forceinline__ void lnb_mbar_wait(uint64_t* bar, uint32_t parity) {
 
 // NJ: 256-channel chunks per row in pass 1 (4: C <= 1024, gamma held in registers; 8: C <= 2048, gamma re-read through L1 --
 // 64 more registers would spill at two CTAs per SM)
-template <typename T, int NJ>
+// DET: dgamma is a [gridDim.x * ngrp, 3, C] scratch; every (CTA, pass-2 group) stores its sums to its own row
+template <typename T, int NJ, bool DET = false>
 __global__ void __launch_bounds__(256, 2) ln_residual_bwd_kernel(const float* __restrict__ dx, const T* __restrict__ z,
                                                                  const float* __restrict__ stats, const float* __restrict__ gamma,
                                                                  const float* __restrict__ sample_scale, T* __restrict__ dz,
@@ -512,11 +513,21 @@ __global__ void __launch_bounds__(256, 2) ln_residual_bwd_kernel(const float* __
   }
   if (tid == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   if (p2_active) {
+    if constexpr (DET) {
+      float* prow = dgamma + ((size_t)blockIdx.x * ngrp + grp) * 3 * C;
 #pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      atomicAdd(dgamma + c2 + e, a_g[e]);
-      atomicAdd(dbeta + c2 + e, a_b[e]);
-      if (dbias_prev) atomicAdd(dbias_prev + c2 + e, a_z[e]);
+      for (int e = 0; e < 8; ++e) {
+        prow[c2 + e] = a_g[e];
+        prow[C + c2 + e] = a_b[e];
+        prow[2 * C + c2 + e] = a_z[e];
+      }
+    } else {
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        atomicAdd(dgamma + c2 + e, a_g[e]);
+        atomicAdd(dbeta + c2 + e, a_b[e]);
+        if (dbias_prev) atomicAdd(dbias_prev + c2 + e, a_z[e]);
+      }
     }
   }
 }
@@ -524,7 +535,8 @@ __global__ void __launch_bounds__(256, 2) ln_residual_bwd_kernel(const float* __
 // ------------------------------------------------------------------------------------------------
 // column sums (bias gradients)
 // ------------------------------------------------------------------------------------------------
-template <typename T>
+// DET: out is a [gridDim.y, cols] scratch, one row per row block
+template <typename T, bool DET = false>
 __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ x, float* __restrict__ out, int rows, int cols,
                                                      int ld) {
   __shared__ float red[8][256 + 8];
@@ -563,7 +575,11 @@ __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ x, fl
 #pragma unroll
   for (int y = 0; y < 8; ++y) s += red[y][col];
   const int gc = blockIdx.x * 256 + col;
-  if (gc < cols) atomicAdd(out + gc, s);
+  if constexpr (DET) {
+    if (gc < cols) out[(size_t)blockIdx.y * cols + gc] = s;
+  } else {
+    if (gc < cols) atomicAdd(out + gc, s);
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -627,6 +643,8 @@ __global__ void shift_mask_kernel(float* __restrict__ mask, int H, int W, int Wh
 // ------------------------------------------------------------------------------------------------
 // latitude-weighted L2 loss
 // ------------------------------------------------------------------------------------------------
+// DET: num / den are [gridDim.y, planes] scratch rows, one per row block
+template <bool DET = false>
 __global__ void __launch_bounds__(256) latw_l2_fwd_kernel(const float* __restrict__ prd, const float* __restrict__ tar,
                                                           const float* __restrict__ qw, float* __restrict__ num,
                                                           float* __restrict__ den, int H, int W, int rows_per_block) {
@@ -673,8 +691,13 @@ __global__ void __launch_bounds__(256) latw_l2_fwd_kernel(const float* __restric
     an = warp_sum(an);
     ad = warp_sum(ad);
     if (lane == 0) {
-      atomicAdd(num + plane, an);
-      atomicAdd(den + plane, ad);
+      if constexpr (DET) {
+        num[(size_t)blockIdx.y * gridDim.x + plane] = an;
+        den[(size_t)blockIdx.y * gridDim.x + plane] = ad;
+      } else {
+        atomicAdd(num + plane, an);
+        atomicAdd(den + plane, ad);
+      }
     }
   }
 }
@@ -925,7 +948,9 @@ struct LnbSmem {
   static constexpr int kBytes = kOffBar + 64;
 };
 
-template <int NK>
+// DET: the consumer warps park their sums in the drained ring, one fold in warp order per channel, and dgamma is a
+// [gridDim.x, 3, C] scratch receiving one row per CTA
+template <int NK, bool DET = false>
 __global__ void __launch_bounds__(kLnbThreads, 1)
 ln_bwd_rowwarp_kernel(const float* __restrict__ dx, const __nv_bfloat16* __restrict__ z, const float* __restrict__ stats,
                       const float* __restrict__ gamma, const float* __restrict__ sample_scale, __nv_bfloat16* __restrict__ dz,
@@ -1062,35 +1087,80 @@ ln_bwd_rowwarp_kernel(const float* __restrict__ dx, const __nv_bfloat16* __restr
       ++nstores;
     }
     if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+    if constexpr (DET) {
+      static_assert(kLnbRows * 3 * C * 4 <= kLnbStages * SM::kStage, "per-warp sums fit the ring");
+      float* wsum = reinterpret_cast<float*>(lsm) + warp * 3 * C;
+      asm volatile("bar.sync 1, %0;" ::"r"(kLnbRows * 32) : "memory");   // every consumer has read its last ring slot
 #pragma unroll
-    for (int k = 0; k < NK; ++k)
+      for (int k = 0; k < NK; ++k)
 #pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        const int c = lane * 4 + 128 * k + e;
-        atomicAdd(red + c, a_g[k][e]);
-        atomicAdd(red + C + c, a_b[k][e]);
-        atomicAdd(red + 2 * C + c, a_z[k][e]);
-      }
+        for (int e = 0; e < 4; ++e) {
+          const int c = lane * 4 + 128 * k + e;
+          wsum[c] = a_g[k][e];
+          wsum[C + c] = a_b[k][e];
+          wsum[2 * C + c] = a_z[k][e];
+        }
+    } else {
+#pragma unroll
+      for (int k = 0; k < NK; ++k)
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          const int c = lane * 4 + 128 * k + e;
+          atomicAdd(red + c, a_g[k][e]);
+          atomicAdd(red + C + c, a_b[k][e]);
+          atomicAdd(red + 2 * C + c, a_z[k][e]);
+        }
+    }
   }
   __syncthreads();
-  for (int c = tid; c < C; c += kLnbThreads) {
-    atomicAdd(dgamma + c, red[c]);
-    atomicAdd(dbeta + c, red[C + c]);
-    if (dbias_prev) atomicAdd(dbias_prev + c, red[2 * C + c]);
+  if constexpr (DET) {
+    const float* wsum = reinterpret_cast<const float*>(lsm);
+    for (int c = tid; c < 3 * C; c += kLnbThreads) {
+      float v = 0.f;
+#pragma unroll
+      for (int w = 0; w < kLnbRows; ++w) v += wsum[w * 3 * C + c];
+      dgamma[(size_t)blockIdx.x * 3 * C + c] = v;
+    }
+  } else {
+    for (int c = tid; c < C; c += kLnbThreads) {
+      atomicAdd(dgamma + c, red[c]);
+      atomicAdd(dbeta + c, red[C + c]);
+      if (dbias_prev) atomicAdd(dbias_prev + c, red[2 * C + c]);
+    }
   }
+}
+
+// deterministic mode: at most this many CTAs, each leaving (per pass-2 group) one row of partial sums
+constexpr int kLnDetCtas = 256;
+
+// part (deterministic mode): the partial-sum rows, reduced in CTA order into dgamma / dbeta / dbias_prev afterwards
+static int ln_bwd_reduce_partials(const float* part, int n_part, int C, float* dgamma, float* dbeta, float* dbias_prev, cudaStream_t s) {
+  const long long row = 3LL * C;
+  if (int e = ordered_reduce(part, n_part, row, C, 1, dgamma, 1, s)) return e;
+  if (int e = ordered_reduce(part + C, n_part, row, C, 1, dbeta, 1, s)) return e;
+  if (dbias_prev) return ordered_reduce(part + 2 * C, n_part, row, C, 1, dbias_prev, 1, s);
+  return SWINB200_OK;
 }
 
 template <int NK>
 static int launch_ln_bwd_rowwarp(const float* dx, const __nv_bfloat16* z, const float* stats, const float* gamma, const float* ss,
                                  __nv_bfloat16* dz, float* dgamma, float* dbeta, float* dbias_prev, int rows, int rps,
-                                 cudaStream_t s) {
+                                 cudaStream_t s, float* part = nullptr) {
   using SM = LnbSmem<NK>;
-  static bool configured = false;
-  if (!configured) {
-    SWB_CUDA(cudaFuncSetAttribute(ln_bwd_rowwarp_kernel<NK>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM::kBytes));
-    configured = true;
+  static bool configured[2] = {false, false};
+  const bool det = part != nullptr;
+  if (!configured[det]) {
+    SWB_CUDA(cudaFuncSetAttribute(det ? ln_bwd_rowwarp_kernel<NK, true> : ln_bwd_rowwarp_kernel<NK>,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, SM::kBytes));
+    configured[det] = true;
   }
   const int ntiles = (rows + kLnbRows - 1) / kLnbRows;
+  if (det) {
+    const int grid = max(1, min(ntiles, min(sm_count(), kLnDetCtas)));
+    ln_bwd_rowwarp_kernel<NK, true><<<grid, kLnbThreads, SM::kBytes, s>>>(dx, z, stats, gamma, ss, dz, part, nullptr, nullptr, rows, rps);
+    SWB_LAUNCH_CHECK();
+    return ln_bwd_reduce_partials(part, grid, SM::C, dgamma, dbeta, dbias_prev, s);
+  }
   ln_bwd_rowwarp_kernel<NK><<<max(1, min(ntiles, sm_count())), kLnbThreads, SM::kBytes, s>>>(dx, z, stats, gamma, ss, dz, dgamma,
                                                                                            dbeta, dbias_prev, rows, rps);
   SWB_LAUNCH_CHECK();
@@ -1099,10 +1169,11 @@ static int launch_ln_bwd_rowwarp(const float* dx, const __nv_bfloat16* z, const 
 
 template <typename T>
 static int launch_ln_bwd(const float* dx, const T* z, const float* stats, const float* gamma, const float* ss, T* dz,
-                         float* dgamma, float* dbeta, float* dbias_prev, int rows, int C, int rps, cudaStream_t s) {
+                         float* dgamma, float* dbeta, float* dbias_prev, int rows, int C, int rps, cudaStream_t s,
+                         float* part = nullptr) {
   if constexpr (sizeof(T) == 2) {
     const bool aligned = ((uintptr_t)dx % 16 == 0) && ((uintptr_t)z % 16 == 0) && ((uintptr_t)dz % 16 == 0) && ((uintptr_t)gamma % 16 == 0);
-    if (C == 768 && aligned) return launch_ln_bwd_rowwarp<6>(dx, z, stats, gamma, ss, dz, dgamma, dbeta, dbias_prev, rows, rps, s);
+    if (C == 768 && aligned) return launch_ln_bwd_rowwarp<6>(dx, z, stats, gamma, ss, dz, dgamma, dbeta, dbias_prev, rows, rps, s, part);
   }
   if (C / 8 > 256) {
     set_error("ln_residual_bwd: C=%d > 2048 unsupported", C);
@@ -1124,6 +1195,22 @@ static int launch_ln_bwd(const float* dx, const T* z, const float* stats, const 
     configured[wide] = true;
   }
   const int ntiles = (rows + TR - 1) / TR;
+  if (part != nullptr) {
+    static bool configured_det[2] = {false, false};
+    if (!configured_det[wide]) {
+      SWB_CUDA(cudaFuncSetAttribute(wide ? ln_residual_bwd_kernel<T, 8, true> : ln_residual_bwd_kernel<T, 4, true>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
+      configured_det[wide] = true;
+    }
+    const int grid = max(1, min(ntiles, kLnDetCtas));
+    const int ngrp = max(1, 256 / (C / 8));
+    if (wide)
+      ln_residual_bwd_kernel<T, 8, true><<<grid, 256, smem, s>>>(dx, z, stats, gamma, ss, dz, part, nullptr, nullptr, rows, C, rps, TR);
+    else
+      ln_residual_bwd_kernel<T, 4, true><<<grid, 256, smem, s>>>(dx, z, stats, gamma, ss, dz, part, nullptr, nullptr, rows, C, rps, TR);
+    SWB_LAUNCH_CHECK();
+    return ln_bwd_reduce_partials(part, grid * ngrp, C, dgamma, dbeta, dbias_prev, s);
+  }
   const int blocks = max(1, min(ntiles, 2 * sm_count()));
   if (wide)
     ln_residual_bwd_kernel<T, 8><<<blocks, 256, smem, s>>>(dx, z, stats, gamma, ss, dz, dgamma, dbeta, dbias_prev, rows, C, rps, TR);
@@ -1219,6 +1306,65 @@ extern "C" int swinb200_latw_l2_bwd(const float* prd, const float* tar, const fl
   int rpb = max(1, (H + split - 1) / split);
   split = (H + rpb - 1) / rpb;
   latw_l2_bwd_kernel<<<dim3(planes, split), 256, 0, (cudaStream_t)stream>>>(prd, tar, qw, chw, num, den, gloss, relative, squared, dprd, C, H, W, rpb);
+  SWB_LAUNCH_CHECK();
+  return SWINB200_OK;
+}
+
+// ---- deterministic mode ---------------------------------------------------------------------------------------------------
+extern "C" int swinb200_ln_residual_bwd_det(const float* dx, const void* z, int act_dtype, const float* stats, const float* gamma,
+                                            const float* sample_scale, void* dz, float* dgamma, float* dbeta, float* dbias_prev,
+                                            int rows, int C, int rows_per_sample, float* part, long long part_floats, void* stream) {
+  SWB_CHECK_ARG(dx && z && stats && gamma && dz && dgamma && dbeta, "ln_residual_bwd_det: null pointer");
+  SWB_CHECK_ARG(rows > 0 && C > 0 && C % 8 == 0 && rows_per_sample > 0, "ln_residual_bwd_det: bad shape rows=%d C=%d", rows, C);
+  const long long need = 3LL * C * kLnDetCtas * max(1, 2048 / C);
+  SWB_CHECK_ARG(part != nullptr && part_floats >= need, "ln_residual_bwd_det: scratch of %lld floats required, got %lld", need, part_floats);
+  if (act_dtype == SWINB200_BF16)
+    return launch_ln_bwd<__nv_bfloat16>(dx, (const __nv_bfloat16*)z, stats, gamma, sample_scale, (__nv_bfloat16*)dz, dgamma, dbeta, dbias_prev,
+                                        rows, C, rows_per_sample, (cudaStream_t)stream, part);
+  if (act_dtype == SWINB200_F32)
+    return launch_ln_bwd<float>(dx, (const float*)z, stats, gamma, sample_scale, (float*)dz, dgamma, dbeta, dbias_prev, rows, C,
+                                rows_per_sample, (cudaStream_t)stream, part);
+  SWB_CHECK_ARG(false, "ln_residual_bwd_det: bad act_dtype %d", act_dtype);
+}
+
+extern "C" int swinb200_colsum_det(const void* x, int act_dtype, float* out, int rows, int cols, int ld, float* part, long long part_floats,
+                                   void* stream) {
+  SWB_CHECK_ARG(x && out && rows > 0 && cols > 0 && cols % 8 == 0 && ld % 8 == 0, "colsum_det: bad arguments rows=%d cols=%d ld=%d", rows,
+                cols, ld);
+  const int gy = min((rows + 63) / 64, 256);
+  SWB_CHECK_ARG(part != nullptr && part_floats >= (long long)gy * cols, "colsum_det: scratch of %lld floats required, got %lld",
+                (long long)gy * cols, part_floats);
+  cudaStream_t s = (cudaStream_t)stream;
+  dim3 grid((cols + 255) / 256, gy);
+  if (act_dtype == SWINB200_BF16)
+    colsum_kernel<__nv_bfloat16, true><<<grid, 256, 0, s>>>((const __nv_bfloat16*)x, part, rows, cols, ld);
+  else if (act_dtype == SWINB200_F32)
+    colsum_kernel<float, true><<<grid, 256, 0, s>>>((const float*)x, part, rows, cols, ld);
+  else
+    SWB_CHECK_ARG(false, "colsum_det: bad act_dtype %d", act_dtype);
+  SWB_LAUNCH_CHECK();
+  return ordered_reduce(part, gy, cols, cols, 1, out, 1, s);
+}
+
+extern "C" int swinb200_latw_l2_fwd_det(const float* prd, const float* tar, const float* qw, const float* chw, int relative, int squared,
+                                        float* num, float* den, float* loss, int B, int C, int H, int W, float* part, long long part_floats,
+                                        void* stream) {
+  SWB_CHECK_ARG(prd && tar && qw && chw && num && den && loss, "latw_l2_fwd_det: null pointer");
+  SWB_CHECK_ARG(B > 0 && C > 0 && H > 0 && W > 0 && W % 4 == 0, "latw_l2_fwd_det: bad shape (W must be a multiple of 4)");
+  SWB_CHECK_ARG(part != nullptr && part_floats >= 2LL * B * C * H, "latw_l2_fwd_det: scratch of 2*B*C*H = %lld floats required, got %lld",
+                2LL * B * C * H, part_floats);
+  cudaStream_t s = (cudaStream_t)stream;
+  const int planes = B * C;
+  int split = max(1, (sm_count() * 8 + planes - 1) / planes);
+  int rpb = max(1, (H + split - 1) / split);
+  split = (H + rpb - 1) / rpb;
+  float* pnum = part;
+  float* pden = part + (size_t)split * planes;
+  latw_l2_fwd_kernel<true><<<dim3(planes, split), 256, 0, s>>>(prd, tar, qw, pnum, pden, H, W, rpb);
+  SWB_LAUNCH_CHECK();
+  if (int e = ordered_reduce(pnum, split, planes, planes, 1, num, 0, s)) return e;
+  if (int e = ordered_reduce(pden, split, planes, planes, 1, den, 0, s)) return e;
+  latw_l2_finish_kernel<<<1, 256, 0, s>>>(num, den, chw, relative, squared, loss, planes, C);
   SWB_LAUNCH_CHECK();
   return SWINB200_OK;
 }

@@ -114,7 +114,7 @@ static int launch_simt(int M, int N, int K, const T* A, int a_major, int lda, co
 
 int gemm_tcgen05(int M, int N, int K, const void* A, int a_major, int lda, const void* B, int b_major, int ldb, int epilogue,
                  const float* bias, void* D, int ldd, void* D2, const void* aux, int ld_aux, int accumulate, int split_k,
-                 cudaStream_t stream, const GemmLnFuse* ln = nullptr, float* colsum_out = nullptr);
+                 cudaStream_t stream, const GemmLnFuse* ln = nullptr, float* colsum_out = nullptr, float* part = nullptr);
 
 }  // namespace swinb200
 
@@ -184,4 +184,44 @@ extern "C" int swinb200_linear_ln_residual(int backend, int M, int N, int K, con
   }
   GemmLnFuse ln{x_in, gamma, beta, sample_scale, x_out, xb_out, stats, counters, n_counters, rows_per_sample, eps};
   return gemm_tcgen05(M, N, K, A, 0, lda, W, 0, ldw, SWINB200_EPI_BIAS_LN, bias, z, ldz, nullptr, nullptr, 0, 0, 1, (cudaStream_t)stream, &ln);
+}
+
+extern "C" int swinb200_gemm_wgrad_det(int backend, int M, int N, int K, const void* A, int lda, const void* B, int ldb, int in_dtype,
+                                       float* D, int split_k, float* part, long long part_floats, void* stream) {
+  SWB_CHECK_ARG(M > 0 && N > 0 && K > 0 && split_k >= 1, "gemm_wgrad_det: bad shape M=%d N=%d K=%d split_k=%d", M, N, K, split_k);
+  SWB_CHECK_ARG(A && B && D, "gemm_wgrad_det: null operand");
+  SWB_CHECK_ARG(lda >= M && ldb >= N, "gemm_wgrad_det: leading dimension too small");
+  cudaStream_t s = (cudaStream_t)stream;
+  if (backend == SWINB200_GEMM_TCGEN05) {
+    SWB_CHECK_ARG(in_dtype == SWINB200_BF16, "gemm_wgrad_det: the tcgen05 back end needs bf16 operands");
+    SWB_CHECK_ARG(part != nullptr && part_floats >= (long long)split_k * M * N,
+                  "gemm_wgrad_det: scratch of split_k*M*N = %lld floats required, got %lld", (long long)split_k * M * N, part_floats);
+    return gemm_tcgen05(M, N, K, A, 1, lda, B, 1, ldb, SWINB200_EPI_F32, nullptr, D, N, nullptr, nullptr, 0, 1, split_k, s, nullptr,
+                        nullptr, part);
+  }
+  // the CUDA-core GEMM does not split K: one thread adds each element once, in a fixed k order
+  SWB_CHECK_ARG(backend == SWINB200_GEMM_SIMT, "gemm_wgrad_det: unknown backend %d", backend);
+  if (in_dtype == SWINB200_BF16)
+    return launch_simt<__nv_bfloat16>(M, N, K, (const __nv_bfloat16*)A, 1, lda, (const __nv_bfloat16*)B, 1, ldb, SWINB200_EPI_F32, nullptr, D, N,
+                                      nullptr, nullptr, 0, 1, s);
+  if (in_dtype == SWINB200_F32)
+    return launch_simt<float>(M, N, K, (const float*)A, 1, lda, (const float*)B, 1, ldb, SWINB200_EPI_F32, nullptr, D, N, nullptr, nullptr, 0, 1, s);
+  SWB_CHECK_ARG(false, "gemm_wgrad_det: bad in_dtype %d", in_dtype);
+}
+
+extern "C" int swinb200_linear_wgrad_det(int backend, int n_out, int n_in, int T, const void* dY, int ldy, const void* X, int ldx,
+                                         float* dW, float* dbias, int split_k, float* part, long long part_floats, void* stream) {
+  SWB_CHECK_ARG(n_out > 0 && n_in > 0 && T > 0, "linear_wgrad_det: bad shape n_out=%d n_in=%d T=%d", n_out, n_in, T);
+  SWB_CHECK_ARG(dY && X && dW, "linear_wgrad_det: null pointer");
+  SWB_CHECK_ARG(ldy >= n_out && ldx >= n_in && split_k >= 1, "linear_wgrad_det: leading dimension too small");
+  const long long need = (long long)split_k * ((long long)n_out * n_in + n_out);
+  SWB_CHECK_ARG(part != nullptr && part_floats >= need, "linear_wgrad_det: scratch of split_k*(n_out*n_in + n_out) = %lld floats required, got %lld",
+                need, part_floats);
+  if (backend != SWINB200_GEMM_TCGEN05 || n_out % 256 != 0 || n_in < 256) {
+    set_error("linear_wgrad_det: tcgen05 / bf16 only, n_out a multiple of 256 and n_in >= 256 (backend %d, n_out = %d, n_in = %d)",
+              backend, n_out, n_in);
+    return SWINB200_ERR_UNSUPPORTED;
+  }
+  return gemm_tcgen05(n_out, n_in, T, dY, 1, ldy, X, 1, ldx, SWINB200_EPI_F32, nullptr, dW, n_in, nullptr, nullptr, 0, 1, split_k,
+                      (cudaStream_t)stream, nullptr, dbias, part);
 }

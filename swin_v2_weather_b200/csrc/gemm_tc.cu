@@ -163,6 +163,13 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, const void* s
                "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
                : "memory");
 }
+// 3-D map [S, M, N]: box depth 1, so the copy engine clips a ragged tile's rows at M inside its own slice
+__device__ __forceinline__ void tma_store_3d(const CUtensorMap* m, const void* smem_src, int c0, int c1, int c2) {
+  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.tile.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(
+                   reinterpret_cast<uint64_t>(m)),
+               "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2)
+               : "memory");
+}
 __device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* m, const void* smem_src, int c0, int c1) {
   asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
                    reinterpret_cast<uint64_t>(m)),
@@ -255,7 +262,9 @@ __device__ __forceinline__ unsigned char* staging_chunk(unsigned char* buf, int 
   return buf + r * 64 + ((c ^ ((r >> 1) & 3)) << 4);
 }
 
-template <int BN, bool A_MN, bool B_MN, int EPI, bool PAIR>
+// DET (split-K weight gradients in deterministic mode): split ks stores its fp32 tile into slice ks of a [S, M, N] scratch
+// (tmD is then a 3-D map) and its column sums into row ks of an [S, M] scratch; swinb200_ordered_reduce adds them up.
+template <int BN, bool A_MN, bool B_MN, int EPI, bool PAIR, bool DET = false>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmD, const __grid_constant__ CUtensorMap tmD2, const GemmTcParams p) {
@@ -648,7 +657,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
             for (int g8 = 0; g8 < 8; ++g8) tot += xch[(bx * 8 + g8) * kWarpStg + wd * 2 + hf];
             const int col = m0 + t_;
-            if (col < p.M) atomicAdd(p.colsum_out + col, tot);
+            if constexpr (DET) {
+              if (col < p.M) p.colsum_out[(size_t)ks_ * p.M + col] = tot;
+            } else {
+              if (col < p.M) atomicAdd(p.colsum_out + col, tot);
+            }
           }
           asm volatile("bar.sync 7, %0;" ::"r"(kEpiGroups * 128) : "memory");   // before the staging buffers take output pieces
         }
@@ -863,7 +876,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0 && !(p.debug & 2)) {
-            if (EPI == SWINB200_EPI_F32 && p.atomic_out) tma_reduce_add_2d(&tmD, stg0, nb, m0 + mrow0);
+            if constexpr (DET) tma_store_3d(&tmD, stg0, nb, m0 + mrow0, tile % p.split_k);
+            else if (EPI == SWINB200_EPI_F32 && p.atomic_out) tma_reduce_add_2d(&tmD, stg0, nb, m0 + mrow0);
             else if (EPI == SWINB200_EPI_BIAS_GELU && pass == 0) tma_store_2d(&tmD2, stg0, nb, m0 + mrow0);
             else tma_store_2d(&tmD, stg0, nb, m0 + mrow0);
             bulk_commit();
@@ -952,11 +966,33 @@ int make_tmap_2d(CUtensorMap* m, bool f32, const void* base, uint64_t inner, uin
   return SWINB200_OK;
 }
 
-template <int BN, bool A_MN, bool B_MN, int EPI, bool PAIR>
+// 3-D fp32 map over `depth` slices of `outer` x `inner` (row pitch `inner`): the partial-sum scratch of DET launches
+static int make_tmap_3d_f32(CUtensorMap* m, const void* base, uint64_t inner, uint64_t outer, uint64_t depth, uint32_t box_inner,
+                            uint32_t box_outer) {
+  EncodeTiledFn enc = get_encode_tiled();
+  if (!enc) {
+    set_error("cuTensorMapEncodeTiled is not available from the driver");
+    return SWINB200_ERR_CUDA;
+  }
+  cuuint64_t dims[3] = {inner, outer, depth};
+  cuuint64_t strides[2] = {inner * 4, inner * outer * 4};
+  cuuint32_t box[3] = {box_inner, box_outer, 1};
+  cuuint32_t estr[3] = {1, 1, 1};
+  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_error("cuTensorMapEncodeTiled (3-D) failed (%d): base=%p dims=%llux%llux%llu", (int)r, base, (unsigned long long)inner,
+              (unsigned long long)outer, (unsigned long long)depth);
+    return SWINB200_ERR_CUDA;
+  }
+  return SWINB200_OK;
+}
+
+template <int BN, bool A_MN, bool B_MN, int EPI, bool PAIR, bool DET = false>
 static int launch_tc_impl(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmD, const CUtensorMap& tmD2,
                           const GemmTcParams& p, cudaStream_t s) {
   using Cfg = GemmCfg<BN, PAIR, EPI == SWINB200_EPI_BIAS_LN>;
-  auto kern = gemm_tc_kernel<BN, A_MN, B_MN, EPI, PAIR>;
+  auto kern = gemm_tc_kernel<BN, A_MN, B_MN, EPI, PAIR, DET>;
   static bool configured = false;
   if (!configured) {
     SWB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmem));
@@ -986,13 +1022,13 @@ static int launch_tc_impl(const CUtensorMap& tmA, const CUtensorMap& tmB, const 
 }
 
 // p.num_m_tiles counts 128-row tiles for single-CTA launches and 256-row pair tiles for PAIR launches
-template <int BN, bool A_MN, bool B_MN, int EPI>
+template <int BN, bool A_MN, bool B_MN, int EPI, bool DET = false>
 static int launch_tc(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmD, const CUtensorMap& tmD2,
                      const GemmTcParams& p, cudaStream_t s) {
   if (p.pair) {
-    if constexpr (BN == 256) return launch_tc_impl<BN, A_MN, B_MN, EPI, true>(tmA, tmB, tmD, tmD2, p, s);
+    if constexpr (BN == 256) return launch_tc_impl<BN, A_MN, B_MN, EPI, true, DET>(tmA, tmB, tmD, tmD2, p, s);
   }
-  return launch_tc_impl<BN, A_MN, B_MN, EPI, false>(tmA, tmB, tmD, tmD2, p, s);
+  return launch_tc_impl<BN, A_MN, B_MN, EPI, false, DET>(tmA, tmB, tmD, tmD2, p, s);
 }
 
 // Only the operand-major / epilogue pairs the model uses are instantiated:
@@ -1020,7 +1056,7 @@ static int dispatch(int epi, int a_major, int b_major, const CUtensorMap& tmA, c
 
 int gemm_tcgen05(int M, int N, int K, const void* A, int a_major, int lda, const void* B, int b_major, int ldb, int epilogue,
                  const float* bias, void* D, int ldd, void* D2, const void* aux, int ld_aux, int accumulate, int split_k,
-                 cudaStream_t stream, const GemmLnFuse* ln, float* colsum_out) {
+                 cudaStream_t stream, const GemmLnFuse* ln, float* colsum_out, float* part) {
   const bool qknorm = (epilogue == SWINB200_EPI_BIAS_QKNORM);
   if (epilogue == SWINB200_EPI_BIAS_LN) {
     SWB_CHECK_ARG(ln != nullptr && ln->x_in && ln->gamma && ln->beta && ln->x_out && ln->xb_out && ln->stats && ln->counters,
@@ -1037,6 +1073,8 @@ int gemm_tcgen05(int M, int N, int K, const void* A, int a_major, int lda, const
   SWB_CHECK_ARG(aux == nullptr || (((uintptr_t)aux % 16 == 0) && ld_aux % 8 == 0), "gemm(tcgen05): aux must be 16-byte aligned with ld_aux %% 8 == 0");
   SWB_CHECK_ARG(D2 == nullptr || ((uintptr_t)D2 % 16 == 0), "gemm(tcgen05): D2 must be 16-byte aligned");
   SWB_CHECK_ARG(bias == nullptr || ((uintptr_t)bias % 16 == 0), "gemm(tcgen05): bias must be 16-byte aligned");
+  SWB_CHECK_ARG(part == nullptr || (epilogue == SWINB200_EPI_F32 && a_major == 1 && b_major == 1 && ((uintptr_t)part % 16 == 0)),
+                "gemm(tcgen05): split partials are a weight-gradient (a1, b1, EPI_F32) option and need 16-byte alignment");
 
   const int BN = qknorm ? 192 : ((N > 128) ? 256 : 128);   // QKNORM: two 96-wide heads per tile
   const bool f32_out = (epilogue == SWINB200_EPI_ADD_F32 || epilogue == SWINB200_EPI_F32);
@@ -1052,6 +1090,7 @@ int gemm_tcgen05(int M, int N, int K, const void* A, int a_major, int lda, const
   p.ln_x_in = nullptr; p.ln_gamma = nullptr; p.ln_beta = nullptr; p.ln_sample_scale = nullptr; p.ln_x_out = nullptr;
   p.ln_xb_out = nullptr; p.ln_stats = nullptr; p.ln_z = nullptr; p.ln_ldz = 0; p.ln_counters = nullptr;
   p.ln_rows_per_sample = 1; p.ln_eps = 0.f; p.ln_slices = 0; p.colsum_out = colsum_out;
+  if (part != nullptr) SWB_CHECK_ARG(ldd == N, "gemm(tcgen05): split partials need a dense D (ldd == N)");
   if (epilogue == SWINB200_EPI_BIAS_LN) {
     p.ln_x_in = ln->x_in; p.ln_gamma = ln->gamma; p.ln_beta = ln->beta; p.ln_sample_scale = ln->sample_scale;
     p.ln_x_out = ln->x_out; p.ln_xb_out = reinterpret_cast<__nv_bfloat16*>(ln->xb_out); p.ln_stats = ln->stats;
@@ -1075,6 +1114,7 @@ int gemm_tcgen05(int M, int N, int K, const void* A, int a_major, int lda, const
   split_k = max(1, min(split_k, p.kb_total));
   p.kb_per_split = (p.kb_total + split_k - 1) / split_k;
   p.split_k = (p.kb_total + p.kb_per_split - 1) / p.kb_per_split;  // no empty splits
+  if (part != nullptr && colsum_out != nullptr) p.colsum_out = part + (size_t)p.split_k * M * N;   // [S, M] after the [S, M, N] slices
 
   CUtensorMap tmA, tmB, tmD, tmD2;
   int e;
@@ -1085,7 +1125,8 @@ int gemm_tcgen05(int M, int N, int K, const void* A, int a_major, int lda, const
   else e = make_tmap_2d(&tmB, false, B, (uint64_t)N, (uint64_t)K, (uint64_t)ldb, 64, GBK);
   if (e) return e;
   // output maps: one [32 rows x 64 bytes] box per staged piece; the copy engine clips rows >= M and columns >= N
-  e = make_tmap_2d(&tmD, f32_out, D, (uint64_t)N, (uint64_t)M, (uint64_t)ldd, f32_out ? 16 : 32, 32, true);
+  if (part != nullptr) e = make_tmap_3d_f32(&tmD, part, (uint64_t)N, (uint64_t)M, (uint64_t)p.split_k, 16, 32);
+  else e = make_tmap_2d(&tmD, f32_out, D, (uint64_t)N, (uint64_t)M, (uint64_t)ldd, f32_out ? 16 : 32, 32, true);
   if (e) return e;
   tmD2 = tmD;
   if (epilogue == SWINB200_EPI_BIAS_GELU) {
@@ -1098,6 +1139,16 @@ int gemm_tcgen05(int M, int N, int K, const void* A, int a_major, int lda, const
     return launch_tc_impl<192, false, false, SWINB200_EPI_BIAS_QKNORM, false>(tmA, tmB, tmD, tmD2, p, stream);
   }
   if (epilogue == SWINB200_EPI_BIAS_LN) return launch_tc_impl<256, false, false, SWINB200_EPI_BIAS_LN, true>(tmA, tmB, tmD, tmD2, p, stream);
+  if (part != nullptr) {
+    // every split writes its own slice with plain stores; the slices (and the column-sum rows) are then added in split order
+    e = (BN == 256) ? launch_tc<256, true, true, SWINB200_EPI_F32, true>(tmA, tmB, tmD, tmD2, p, stream)
+                    : launch_tc<128, true, true, SWINB200_EPI_F32, true>(tmA, tmB, tmD, tmD2, p, stream);
+    if (e) return e;
+    const long long mn = (long long)M * N;
+    if ((e = ordered_reduce(part, p.split_k, mn, mn, 1, reinterpret_cast<float*>(D), accumulate, stream))) return e;
+    if (colsum_out != nullptr) return ordered_reduce(p.colsum_out, p.split_k, M, M, 1, colsum_out, 1, stream);
+    return SWINB200_OK;
+  }
   if (BN == 256) return dispatch<256>(epilogue, a_major, b_major, tmA, tmB, tmD, tmD2, p, stream);
   return dispatch<128>(epilogue, a_major, b_major, tmA, tmB, tmD, tmD2, p, stream);
 }

@@ -7,7 +7,8 @@
 namespace swinb200 {
 
 // NACC accumulators per plane:  MODE 0 (L1): {sum q|p-t|, sum q|t|};  MODE 1 (ACC): {sum q p t, sum q p p, sum q t t}
-template <int MODE>
+// DET: acc_out is a [gridDim.y, planes, NACC] scratch, one row per row block
+template <int MODE, bool DET = false>
 __global__ void __launch_bounds__(256) latw_reduce_kernel(const float* __restrict__ prd, const float* __restrict__ tar,
                                                           const float* __restrict__ qw, float* __restrict__ acc_out, int H, int W,
                                                           int rows_per_block) {
@@ -63,7 +64,11 @@ __global__ void __launch_bounds__(256) latw_reduce_kernel(const float* __restric
     for (int k = 0; k < NACC; ++k) {
       float v = lane < (int)(blockDim.x >> 5) ? red[k][lane] : 0.f;
       v = warp_sum(v);
-      if (lane == 0) atomicAdd(acc_out + (size_t)plane * NACC + k, v);
+      if constexpr (DET) {
+        if (lane == 0) acc_out[((size_t)blockIdx.y * gridDim.x + plane) * NACC + k] = v;
+      } else {
+        if (lane == 0) atomicAdd(acc_out + (size_t)plane * NACC + k, v);
+      }
     }
   }
 }
@@ -164,6 +169,43 @@ extern "C" int swinb200_latw_acc(const float* prd, const float* tar, const float
   latw_reduce_kernel<1><<<dim3(planes, split), 256, 0, s>>>(prd, tar, qw, sums, H, W, rpb);
   SWB_LAUNCH_CHECK();
   latw_acc_finish_kernel<<<(planes + 255) / 256, 256, 0, s>>>(sums, acc, planes);
+  SWB_LAUNCH_CHECK();
+  return SWINB200_OK;
+}
+
+// ---- deterministic mode: row-block partials, summed in row-block order by swinb200_ordered_reduce ------------------------
+template <int MODE>
+static int latw_sums_det(const float* prd, const float* tar, const float* qw, float* sums, int B, int C, int H, int W, float* part,
+                         long long part_floats, cudaStream_t s) {
+  constexpr int NACC = MODE == 0 ? 2 : 3;
+  SWB_CHECK_ARG(part != nullptr && part_floats >= (long long)NACC * B * C * H, "latw (deterministic): scratch of %d*B*C*H = %lld floats "
+                "required, got %lld", NACC, (long long)NACC * B * C * H, part_floats);
+  const int planes = B * C;
+  int split, rpb;
+  plane_split(planes, H, split, rpb);
+  latw_reduce_kernel<MODE, true><<<dim3(planes, split), 256, 0, s>>>(prd, tar, qw, part, H, W, rpb);
+  SWB_LAUNCH_CHECK();
+  return ordered_reduce(part, split, (long long)planes * NACC, (long long)planes * NACC, 1, sums, 0, s);
+}
+
+extern "C" int swinb200_latw_l1_fwd_det(const float* prd, const float* tar, const float* qw, const float* chw, int relative, float* sums,
+                                        float* loss, int B, int C, int H, int W, float* part, long long part_floats, void* stream) {
+  SWB_CHECK_ARG(prd && tar && qw && chw && sums && loss, "latw_l1_fwd_det: null pointer");
+  SWB_CHECK_ARG(B > 0 && C > 0 && H > 0 && W > 0 && W % 4 == 0, "latw_l1_fwd_det: bad shape (W must be a multiple of 4)");
+  cudaStream_t s = (cudaStream_t)stream;
+  if (int e = latw_sums_det<0>(prd, tar, qw, sums, B, C, H, W, part, part_floats, s)) return e;
+  latw_l1_finish_kernel<<<1, 256, 0, s>>>(sums, chw, relative, loss, B * C, C);
+  SWB_LAUNCH_CHECK();
+  return SWINB200_OK;
+}
+
+extern "C" int swinb200_latw_acc_det(const float* prd, const float* tar, const float* qw, float* sums, float* acc, int B, int C, int H,
+                                     int W, float* part, long long part_floats, void* stream) {
+  SWB_CHECK_ARG(prd && tar && qw && sums && acc, "latw_acc_det: null pointer");
+  SWB_CHECK_ARG(B > 0 && C > 0 && H > 0 && W > 0 && W % 4 == 0, "latw_acc_det: bad shape (W must be a multiple of 4)");
+  cudaStream_t s = (cudaStream_t)stream;
+  if (int e = latw_sums_det<1>(prd, tar, qw, sums, B, C, H, W, part, part_floats, s)) return e;
+  latw_acc_finish_kernel<<<(B * C + 255) / 256, 256, 0, s>>>(sums, acc, B * C);
   SWB_LAUNCH_CHECK();
   return SWINB200_OK;
 }

@@ -3,10 +3,16 @@
 PyTorch is used here for device memory, streams and shape bookkeeping only: every arithmetic
 operation below is one of our CUDA kernels, launched on torch's current stream.  Arguments are
 validated (device, dtype, contiguity) before their raw pointers cross the ABI.
+
+Deterministic mode: while torch.use_deterministic_algorithms(True) is in force, every reduction whose float sums would depend on
+the order in which CTAs finish (split-K weight gradients, bias / LayerNorm parameter gradients, loss and metric sums, attention
+d(scale) / d(bias)) runs through the fixed-order `swinb200_*_det` entry points, with scratch from the torch allocator
+(DESIGN.md section 10).  With the flag off nothing changes.
 """
 from __future__ import annotations
 
 import os
+import warnings
 
 from dataclasses import dataclass
 from typing import Optional
@@ -46,6 +52,16 @@ MODES = {m.name: m for m in (MODE_BF16, MODE_BF16_SIMT, MODE_FP32)}
 
 def _stream() -> int:
     return torch.cuda.current_stream().cuda_stream
+
+
+def deterministic() -> bool:
+    """Read at every call: torch.use_deterministic_algorithms(True) selects the fixed-order reductions."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def _scratch(n_floats: int, device) -> torch.Tensor:
+    """Partial-sum scratch of a deterministic entry point (every slot is written before it is read)."""
+    return torch.empty((max(1, int(n_floats)),), dtype=torch.float32, device=device)
 
 
 def _chk(t: Optional[torch.Tensor], name: str, dtype=None, allow_none=False) -> int:
@@ -154,6 +170,14 @@ def gemm(mode: ComputeMode, A: torch.Tensor, a_major: int, B: torch.Tensor, b_ma
     if epilogue == EPI_BIAS_GELU and out2 is None:
         out2 = torch.empty((M, N), dtype=out_dtype, device=A.device)
     be = mode.gemm_backend if backend is None else backend
+    if split_k > 1 and be == BACKEND_TCGEN05 and deterministic():
+        # split-K reduce-adds arrive in scheduling order: every split stores its own slice, the slices are summed in order
+        if not (epilogue == EPI_F32 and accumulate and a_major == 1 and b_major == 1):
+            raise SwinB200Error("gemm: split_k > 1 is a weight-gradient option (a_major 1, b_major 1, EPI_F32, accumulate)")
+        part = _scratch(split_k * M * N, A.device)
+        _lib.call("swinb200_gemm_wgrad_det", be, M, N, K, _chk(A, "A"), A.shape[1], _chk(B, "B"), B.shape[1], _code(A.dtype),
+                  _chk(out, "out", torch.float32), int(split_k), part.data_ptr(), part.numel(), _stream())
+        return out
     _lib.call("swinb200_gemm", be, M, N, K, _chk(A, "A"), a_major, A.shape[1], _chk(B, "B"), b_major, B.shape[1], _code(A.dtype),
               epilogue, _chk(bias, "bias", torch.float32, True), _chk(out, "out", out_dtype), out.shape[1],
               _chk(out2, "out2", out_dtype, True), _chk(aux, "aux", None, True), 0 if aux is None else aux.shape[1],
@@ -219,6 +243,12 @@ def linear_wgrad(mode: ComputeMode, dy: torch.Tensor, x: torch.Tensor, dw: torch
     if fuse is None:
         fuse = os.environ.get("SWINB200_FUSE_COLSUM", "1") != "0"
     if fuse and dbias is not None and mode.gemm_backend == BACKEND_TCGEN05 and n_out % 256 == 0 and n_in >= 256:
+        if deterministic():
+            part = _scratch(split_k * (n_out * n_in + n_out), dy.device)
+            _lib.call("swinb200_linear_wgrad_det", BACKEND_TCGEN05, n_out, n_in, T, _chk(dy, "dy", torch.bfloat16), n_out,
+                      _chk(x, "x", torch.bfloat16), n_in, _chk(dw, "dw", torch.float32), _chk(dbias, "dbias", torch.float32),
+                      int(split_k), part.data_ptr(), part.numel(), _stream())
+            return dw, dbias
         _lib.call("swinb200_linear_wgrad", BACKEND_TCGEN05, n_out, n_in, T, _chk(dy, "dy", torch.bfloat16), n_out,
                   _chk(x, "x", torch.bfloat16), n_in, _chk(dw, "dw", torch.float32), n_in, _chk(dbias, "dbias", torch.float32),
                   int(split_k), _stream())
@@ -274,6 +304,13 @@ def ln_residual_bwd(dx, z, stats, gamma, sample_scale, rows_per_sample: int, mod
     dz = torch.empty((rows, C), dtype=mode.act_dtype, device=z.device)
     if acc is None:
         acc = torch.zeros((3, C), dtype=torch.float32, device=z.device)
+    if deterministic():
+        part = _scratch(3 * C * 256 * max(1, 2048 // C), z.device)
+        _lib.call("swinb200_ln_residual_bwd_det", _chk(dx, "dx", torch.float32), _chk(z, "z", mode.act_dtype), mode.act_code,
+                  _chk(stats, "stats", torch.float32), _chk(gamma, "gamma", torch.float32),
+                  _chk(sample_scale, "sample_scale", torch.float32, True), dz.data_ptr(), acc[0].data_ptr(), acc[1].data_ptr(),
+                  acc[2].data_ptr() if want_dbias_prev else 0, rows, C, rows_per_sample, part.data_ptr(), part.numel(), _stream())
+        return dz, acc[0], acc[1], acc[2]
     _lib.call("swinb200_ln_residual_bwd", _chk(dx, "dx", torch.float32), _chk(z, "z", mode.act_dtype), mode.act_code,
               _chk(stats, "stats", torch.float32), _chk(gamma, "gamma", torch.float32),
               _chk(sample_scale, "sample_scale", torch.float32, True), dz.data_ptr(), acc[0].data_ptr(), acc[1].data_ptr(),
@@ -299,6 +336,11 @@ def colsum(x: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     rows, cols = x.shape
     if out is None:
         out = torch.zeros((cols,), dtype=torch.float32, device=x.device)
+    if deterministic():
+        part = _scratch(cols * min((rows + 63) // 64, 256), x.device)
+        _lib.call("swinb200_colsum_det", _chk(x, "x"), _code(x.dtype), out.data_ptr(), rows, cols, cols, part.data_ptr(), part.numel(),
+                  _stream())
+        return out
     _lib.call("swinb200_colsum", _chk(x, "x"), _code(x.dtype), out.data_ptr(), rows, cols, cols, _stream())
     return out
 
@@ -356,6 +398,22 @@ def window_attn_bwd(qkv, inv_norm, scale, bias, o, d_o, lse, B, H, W, C, heads, 
     dbias = torch.zeros((heads, L, L), dtype=torch.float32, device=qkv.device) if bias is not None else None
     # scratch for the row term D = <dO, O> (tcgen05 back end: enables the persistent kernel)
     ws = torch.empty((qkv.shape[0] * heads,), dtype=torch.float32, device=qkv.device) if backend == BACKEND_TCGEN05 else None
+    if deterministic():
+        items = B * (H // Wh) * (W // Ww) * heads
+        part = _scratch(items * (4 * ((L + 127) // 128) + (L * L if dbias is not None else 0)), qkv.device)
+        try:
+            _lib.call("swinb200_window_attn_bwd_det", backend, _chk(qkv, "qkv"), _code(qkv.dtype),
+                      _chk(inv_norm, "inv_norm", torch.float32), _chk(scale, "scale", torch.float32),
+                      _chk(bias, "bias", torch.float32, True), _chk(o, "o", qkv.dtype), _chk(d_o, "d_o", qkv.dtype),
+                      _chk(lse, "lse", torch.float32), dqkv.data_ptr(), dscale.data_ptr(), 0 if dbias is None else dbias.data_ptr(),
+                      0 if ws is None else ws.data_ptr(), B, H, W, C, heads, Wh, Ww, s0, s1, part.data_ptr(), part.numel(), _stream())
+            return dqkv, dscale, dbias
+        except SwinB200Error as e:
+            # the legacy kernels (SWINB200_ATTN_BWD=1/2) have no deterministic version: as torch does for such an op, an error,
+            # or a warning and the ordinary kernel under warn_only=True
+            if e.code != _lib.ERR_UNSUPPORTED or not torch.is_deterministic_algorithms_warn_only_enabled():
+                raise
+            warnings.warn(f"window_attn_bwd has no deterministic version for this configuration: {e}")
     _lib.call("swinb200_window_attn_bwd", backend, _chk(qkv, "qkv"), _code(qkv.dtype),
               _chk(inv_norm, "inv_norm", torch.float32), _chk(scale, "scale", torch.float32),
               _chk(bias, "bias", torch.float32, True), _chk(o, "o", qkv.dtype), _chk(d_o, "d_o", qkv.dtype),
@@ -371,6 +429,12 @@ def latw_l2_fwd(prd, tar, qw, chw, relative: bool, squared: bool = True):
     num = torch.empty((B * C,), dtype=torch.float32, device=prd.device)
     den = torch.empty((B * C,), dtype=torch.float32, device=prd.device)
     loss = torch.empty((1,), dtype=torch.float32, device=prd.device)
+    if deterministic():
+        part = _scratch(2 * B * C * H, prd.device)
+        _lib.call("swinb200_latw_l2_fwd_det", _chk(prd, "prd", torch.float32), _chk(tar, "tar", torch.float32),
+                  _chk(qw, "qw", torch.float32), _chk(chw, "chw", torch.float32), int(relative), int(squared), num.data_ptr(),
+                  den.data_ptr(), loss.data_ptr(), B, C, H, W, part.data_ptr(), part.numel(), _stream())
+        return loss, num, den
     _lib.call("swinb200_latw_l2_fwd", _chk(prd, "prd", torch.float32), _chk(tar, "tar", torch.float32), _chk(qw, "qw", torch.float32),
               _chk(chw, "chw", torch.float32), int(relative), int(squared), num.data_ptr(), den.data_ptr(), loss.data_ptr(), B, C, H, W, _stream())
     return loss, num, den
@@ -400,6 +464,12 @@ def latw_l1_fwd(prd, tar, qw, chw, relative: bool):
     B, C, H, W = prd.shape
     sums = torch.empty((B * C, 2), dtype=torch.float32, device=prd.device)
     loss = torch.empty((1,), dtype=torch.float32, device=prd.device)
+    if deterministic():
+        part = _scratch(2 * B * C * H, prd.device)
+        _lib.call("swinb200_latw_l1_fwd_det", _chk(prd, "prd", torch.float32), _chk(tar, "tar", torch.float32),
+                  _chk(qw, "qw", torch.float32), _chk(chw, "chw", torch.float32), int(relative), sums.data_ptr(), loss.data_ptr(),
+                  B, C, H, W, part.data_ptr(), part.numel(), _stream())
+        return loss, sums
     _lib.call("swinb200_latw_l1_fwd", _chk(prd, "prd", torch.float32), _chk(tar, "tar", torch.float32), _chk(qw, "qw", torch.float32),
               _chk(chw, "chw", torch.float32), int(relative), sums.data_ptr(), loss.data_ptr(), B, C, H, W, _stream())
     return loss, sums
@@ -421,6 +491,11 @@ def latw_acc(prd, tar, qw):
     B, C, H, W = prd.shape
     sums = torch.empty((B * C, 3), dtype=torch.float32, device=prd.device)
     acc = torch.empty((B, C), dtype=torch.float32, device=prd.device)
+    if deterministic():
+        part = _scratch(3 * B * C * H, prd.device)
+        _lib.call("swinb200_latw_acc_det", _chk(prd, "prd", torch.float32), _chk(tar, "tar", torch.float32),
+                  _chk(qw, "qw", torch.float32), sums.data_ptr(), acc.data_ptr(), B, C, H, W, part.data_ptr(), part.numel(), _stream())
+        return acc
     _lib.call("swinb200_latw_acc", _chk(prd, "prd", torch.float32), _chk(tar, "tar", torch.float32), _chk(qw, "qw", torch.float32),
               sums.data_ptr(), acc.data_ptr(), B, C, H, W, _stream())
     return acc
