@@ -163,10 +163,10 @@ int swinb200_colsum(const void* x, int act_dtype, float* out, int rows, int cols
  *   the tcgen05 backward accumulates d(scale) against it so that the sum is insensitive to the rounding of O).
  * window_attn_bwd: dqkv (T, 3C) act = gradients w.r.t. the *un-normalised* q, k and v;
  *   dscale (heads) += sum dS * cos ; dbias (heads, L, L) += sum_windows dS (nullable).
- *   ws: optional scratch of T*heads floats (the library allocates nothing).  With it the tcgen05 back end runs its
- *   persistent kernel (window operands arrive as TMA boxes while the previous window is processed; the row term
- *   D = <dO, O> comes from a streaming pre-pass into ws); with NULL every window is one self-contained CTA.
- * backend: SWINB200_GEMM_SIMT (CUDA cores, any act dtype) or SWINB200_GEMM_TCGEN05 (bf16). */
+ *   ws: required by the tcgen05 back end; T*heads floats (the library allocates nothing), which receive the row term
+ *   D = <dO, O> from a streaming pre-pass.  Unused by the CUDA-core back end (nullable there).
+ * backend: SWINB200_GEMM_SIMT (CUDA cores, any act dtype) or SWINB200_GEMM_TCGEN05 (bf16).  The tcgen05 back end needs
+ *   qkv and o (forward), and qkv, o, d_o and dqkv (backward), 16-byte aligned: SWINB200_ERR_INVALID_ARG otherwise. */
 int swinb200_qk_normalize(void* qkv, int act_dtype, float* inv_norm, int T, int C, int heads, void* stream);
 int swinb200_shift_mask(float* mask, int H, int W, int Wh, int Ww, int s0, int s1, void* stream);
 int swinb200_window_attn_fwd(int backend, const void* qkv, int act_dtype, const float* scale,
@@ -240,9 +240,7 @@ int swinb200_adam_step(int n_tensors, void* const* params, const void* const* gr
  *   3*B*C*H (ACC) floats (at most one row block per image row).
  * swinb200_window_attn_bwd_det: swinb200_window_attn_bwd; with nW = (H/Wh)*(W/Ww), L = Wh*Ww and items = B*nW*heads,
  *   scratch >= items*(4*ceil(L/128) + (dbias ? L*L : 0)) floats: d(scale) slots per item, then one (L, L) d(bias) slice
- *   per item (336 MB at 9x18 windows / 8 heads / B = 1 on the 180x360 token grid with a bias table).  The tcgen05 kernels
- *   selected by SWINB200_ATTN_BWD=1/2, a NULL ws or operands that are not 16-byte aligned have no deterministic version:
- *   SWINB200_ERR_UNSUPPORTED, nothing launched. */
+ *   per item (336 MB at 9x18 windows / 8 heads / B = 1 on the 180x360 token grid with a bias table). */
 int swinb200_ordered_reduce(const float* part, int n_part, long long stride, long long n, int inner, float* out, int accumulate,
                             void* stream);
 int swinb200_gemm_wgrad_det(int backend, int M, int N, int K, const void* A, int lda, const void* B, int ldb, int in_dtype,

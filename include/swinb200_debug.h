@@ -14,8 +14,8 @@ extern "C" {
 int swinb200_debug_umma_probe(const void* A, const void* B, float* D, int N, int K, int a_mode, int b_mode,
                               int pad16, void* stream);
 
-/* bring-up aid: when buf != NULL the tcgen05 attention kernels write clock64() stamps per phase for CTAs < 4096
- * into buf[cta*16 + phase] (int64).  Pass NULL to switch it off. */
+/* bring-up aid: when buf != NULL the tcgen05 attention backward at 9x18 windows / head_dim 96 writes the clock64() cycles
+ * each CTA < 4096 spent per phase into buf[cta*16 + phase] (int64).  Pass NULL to switch it off. */
 int swinb200_debug_attn_phase_buffer(void* buf);
 
 #ifdef __cplusplus

@@ -1,5 +1,5 @@
-// Shared pieces of the tcgen05 window-attention kernels (attn_tc.cu: forward + first backward generations,
-// attn_tc_bwd3.cu: the warp-specialised single-pass backward).
+// Shared pieces of the tcgen05 window-attention kernels: attn_tc_fwd4.cu and attn_tc_bwd3.cu (9x18 windows, head_dim 96),
+// attn_tc_gen.cu (every other geometry) and the dispatch in attn_tc.cu.
 #pragma once
 #include "common.cuh"
 #include "ptx.cuh"
@@ -96,39 +96,6 @@ __device__ __forceinline__ void tma_load_5d(void* smem_dst, const CUtensorMap* m
 }
 
 
-__device__ __forceinline__ void tma_store_5d(const CUtensorMap* m, const void* smem_src, int c0, int c1, int c2, int c3, int c4) {
-  asm volatile("cp.async.bulk.tensor.5d.global.shared::cta.tile.bulk_group [%0, {%2, %3, %4, %5, %6}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-               : "memory");
-}
-
-// Row tiles leave the kernel through shared memory: each thread parks its [1 x D] bf16 row (pitch kRowPitch keeps the
-// 16-byte stores conflict-free), then the CTA writes token rows with consecutive threads on consecutive 16-byte pieces,
-// so every global store instruction covers whole 192-byte rows instead of 32 scattered 16-byte fragments.
-constexpr int kRowPitch = 208;
-template <int D>
-__device__ __forceinline__ void park_row(unsigned char* stage, int row, const float (&v)[D]) {
-#pragma unroll
-  for (int c = 0; c < D / 8; ++c) {
-    uint4 pk;
-    pk.x = pack_bf16x2(v[c * 8 + 0], v[c * 8 + 1]); pk.y = pack_bf16x2(v[c * 8 + 2], v[c * 8 + 3]);
-    pk.z = pack_bf16x2(v[c * 8 + 4], v[c * 8 + 5]); pk.w = pack_bf16x2(v[c * 8 + 6], v[c * 8 + 7]);
-    *reinterpret_cast<uint4*>(stage + row * kRowPitch + c * 16) = pk;
-  }
-}
-// rows [0, nrows) of `stage` -> dst[tok[slot0 + row] * ld + col0 ...]; executed by `nthr` threads with index `t`
-template <int D>
-__device__ __forceinline__ void scatter_rows(const unsigned char* stage, int nrows, const int* tok, int slot0,
-                                             __nv_bfloat16* dst, int ld, int col0, int t, int nthr) {
-  constexpr int kPieces = D / 8;
-  for (int i = t; i < nrows * kPieces; i += nthr) {
-    const int row = i / kPieces, c = i - row * kPieces;
-    const uint4 v = *reinterpret_cast<const uint4*>(stage + row * kRowPitch + c * 16);
-    *reinterpret_cast<uint4*>(dst + (size_t)tok[slot0 + row] * ld + col0 + c * 8) = v;
-  }
-}
-
-
 bool attn_gen_supports(int head_dim);
 int attn_tcgen05_gen_fwd(const void* qkv, const float* scale, const float* bias, void* o, float* lse, const AttnGeom& g, cudaStream_t stream);
 // det_part (deterministic mode, see swinb200_window_attn_bwd_det): attn_det_dscale_slots(g) d(scale) slots, followed (with a
@@ -139,10 +106,12 @@ int attn_tcgen05_gen_bwd(const void* qkv, const float* inv_norm, const float* sc
 int attn_make_geom(AttnGeom& g, int B, int H, int W, int C, int heads, int Wh, int Ww, int s0, int s1);
 int attn_make_window_tmap(CUtensorMap* m, const void* base, int B, int H, int W, int channels, int Wh, int Ww);
 int attn_tcgen05_fwd4(const void* qkv, const float* scale, const float* bias, void* o, float* lse, const AttnGeom& g, cudaStream_t stream);
-int attn_tcgen05_fwd3(const void* qkv, const float* scale, const float* bias, void* o, float* lse, const AttnGeom& g, cudaStream_t stream);
 int attn_tcgen05_bwd3(const void* qkv, const float* inv_norm, const float* scale, const float* bias, const void* o, const void* d_o,
                       const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, const AttnGeom& g, cudaStream_t stream,
                       float* det_part = nullptr);
+// D[t, h] = <dO[t, h, :], O[t, h, :]> over n_pairs (token, head) rows of d elements: the backward's pre-pass into ws
+__global__ void attn_rowdot_kernel(const __nv_bfloat16* __restrict__ o, const __nv_bfloat16* __restrict__ d_o, float* __restrict__ out,
+                                   long long n_pairs, int d);
 // one slot per (item, 128-row tile, warp of attn_tc_gen.cu) -- enough for every back end
 inline long long attn_det_dscale_slots(const AttnGeom& g) { return (long long)g.B * g.nW * g.heads * 4 * ((g.L + 127) / 128); }
 

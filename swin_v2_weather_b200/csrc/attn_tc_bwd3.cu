@@ -691,29 +691,6 @@ attn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_con
   }
 }
 
-__global__ void __launch_bounds__(256) attn_rowdot3_kernel(const __nv_bfloat16* __restrict__ o, const __nv_bfloat16* __restrict__ d_o,
-                                                           float* __restrict__ out, long long n_pairs, int d) {
-  // D[t, h] = <dO[t, h, :], O[t, h, :]>, four lanes per (token, head)
-  const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const long long pair = gid >> 2;
-  const int q = (int)(gid & 3);
-  float acc = 0.f;
-  if (pair < n_pairs) {
-    const __nv_bfloat16* a = o + pair * d;
-    const __nv_bfloat16* b = d_o + pair * d;
-    for (int c = q * 8; c < d; c += 32) {
-      float a8[8], b8[8];
-      ld8(a + c, a8);
-      ld8(b + c, b8);
-#pragma unroll
-      for (int e = 0; e < 8; ++e) acc = fmaf(a8[e], b8[e], acc);
-    }
-  }
-  acc += __shfl_xor_sync(0xffffffffu, acc, 1);
-  acc += __shfl_xor_sync(0xffffffffu, acc, 2);
-  if (q == 0 && pair < n_pairs) out[pair] = acc;
-}
-
 static bool g_prof3 = false;
 int attn_set_phase_buffer3(long long* buf) {
   SWB_CUDA(cudaMemcpyToSymbol(g_phase_buf3, &buf, sizeof(buf)));
@@ -736,8 +713,8 @@ int attn_tcgen05_bwd3(const void* qkv, const float* inv_norm, const float* scale
   if (int e = attn_make_window_tmap(&tm_qkv, qkv, g.B, g.H, g.W, 3 * g.C, g.Wh, g.Ww)) return e;
   if (int e = attn_make_window_tmap(&tm_do, d_o, g.B, g.H, g.W, g.C, g.Wh, g.Ww)) return e;
   const long long n_pairs = (long long)g.B * g.H * g.W * g.heads;
-  attn_rowdot3_kernel<<<(unsigned)((n_pairs * 4 + 255) / 256), 256, 0, stream>>>((const __nv_bfloat16*)o, (const __nv_bfloat16*)d_o, ws,
-                                                                                 n_pairs, g.C / g.heads);
+  attn_rowdot_kernel<<<(unsigned)((n_pairs * 4 + 255) / 256), 256, 0, stream>>>((const __nv_bfloat16*)o, (const __nv_bfloat16*)d_o, ws,
+                                                                                n_pairs, g.C / g.heads);
   SWB_LAUNCH_CHECK();
   const int grid = min(g.B * g.nW * g.heads, sm_count());
   static int dbg_env = -1;   // bring-up timing experiments (wrong results): SWINB200_BWD3_DEBUG bit mask, see the kernel

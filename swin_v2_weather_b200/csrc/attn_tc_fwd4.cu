@@ -1,10 +1,15 @@
-// tcgen05 windowed cosine attention, forward, fourth generation: TWO (window, head) items in flight per SM.
+// tcgen05 windowed cosine attention, forward, 9x18 windows at head_dim 96: TWO (window, head) items in flight per SM.
 //
-// Reference math: swinv2_global.py:300-318 (as attn_tc_fwd3.cu).  The third generation processes one item per SM at a time and
-// every phase of that item waits for the previous one (DESIGN.md 5.0: no unit is busy more than 25 %).  Here a CTA is two
-// independent halves, each with four compute warps (thread = query row = TMEM lane), its own control warp (one elected lane
-// issues the TMA boxes and every tcgen05.mma), its own (Q^, K^, V) stage in shared memory, its own 256 tensor-memory columns and
-// its own barriers; half g takes the CTA's items g, g+2, g+4, ...  While one half waits for an MMA, a TMA box or its row
+// Reference math: swinv2_global.py:300-318 -- S = scale * q^ k^T (+ CPB bias) (+ shift mask), P = softmax(S), O = P v; the
+// roll / window_partition / window_reverse copies (:89-119, 446-478) are folded into the TMA box coordinates and the scatter.
+// Operands arrive as TMA window boxes: per 32-channel chunk, one [32 channels x Ww x Wh] box of a 5-D tensor map over the
+// (B, H, W, 3C) activation (attn_make_window_tmap), 64B-swizzled; windows that wrap around the cyclic shift are gathered with
+// cp.async instead.  K^ / V pad rows [L, 176) are zeroed once and never written again, so padded keys contribute exact zeros.
+//
+// With one item per SM at a time every phase of that item waits for the previous one (DESIGN.md 5.0: no unit is busy more
+// than 25 %).  Here a CTA is two independent halves, each with four compute warps (thread = query row = TMEM lane), its own
+// control warp (one elected lane issues the TMA boxes and every tcgen05.mma), its own (Q^, K^, V) stage in shared memory, its
+// own 256 tensor-memory columns and its own barriers; half g takes the CTA's items g, g+2, g+4, ...  While one half waits for an MMA, a TMA box or its row
 // stores, the other half's softmax owns the issue slots.
 //   per item and half:  for each 128-query tile t:  S_t = Q^_t K^T (SS) -> softmax in tensor memory, P packed in place ->
 //                       O_t = P_t V (TS) -> O_t / rowsum into registers (tensor memory is free for S_{t+1}) -> rows parked
@@ -304,7 +309,10 @@ attn_tc_fwd4_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __nv_bfloa
           if (row_ok) {
             const size_t ri = (((size_t)b * g.nW + w) * g.heads + head) * L + n;
             lse[ri] = (row_max + log2f(row_sum)) * 0.6931471805599453f;
-            lse[(size_t)g.B * g.nW * g.heads * L + ri] = cos_sum / row_sum;       // E_P[cos] (see attn_tc_fwd3.cu)
+            // second plane: E_P[cos] of the row.  The backward accumulates d(scale) = sum dS (cos - E_P[cos]); the row sum of dS
+            // is zero in exact arithmetic, so this changes nothing but removes the first-order sensitivity to D = <dO, O>
+            // being formed from the bf16-rounded O.
+            lse[(size_t)g.B * g.nW * g.heads * L + ri] = cos_sum / row_sum;
           }
           tmem_st_wait();
         }

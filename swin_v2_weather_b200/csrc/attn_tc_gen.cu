@@ -1,4 +1,4 @@
-// tcgen05 window attention for every geometry the specialised 9x18 / head_dim-96 kernels (attn_tc_fwd3.cu,
+// tcgen05 window attention for every geometry the specialised 9x18 / head_dim-96 kernels (attn_tc_fwd4.cu,
 // attn_tc_bwd3.cu) are not instantiated for: head_dim 48 / 64 / 96 / 128 / 192 / 256 and windows of any size (BASELINE
 // config 5: 6x12, 12x24, 18x36 ...).  Restates WindowMultiHeadAttention.forward (reference networks/swinv2_global.py:300-319)
 // and its backward as three flash-style kernels of one shape:
@@ -646,36 +646,12 @@ int attn_tcgen05_gen_fwd(const void* qkv, const float* scale, const float* bias,
   return dispatch_gen<kModeFwd>(a, g, stream);
 }
 
-__global__ void __launch_bounds__(256) attn_gen_rowdot_kernel(const __nv_bfloat16* __restrict__ o, const __nv_bfloat16* __restrict__ d_o,
-                                                              float* __restrict__ out, long long n_pairs, int d) {
-  const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const long long pair = gid >> 2;
-  const int q = (int)(gid & 3);
-  float acc = 0.f;
-  if (pair < n_pairs) {
-    for (int c = q * 8; c < d; c += 32) {
-      float a8[8], b8[8];
-      ld8(o + pair * d + c, a8);
-      ld8(d_o + pair * d + c, b8);
-#pragma unroll
-      for (int e = 0; e < 8; ++e) acc = fmaf(a8[e], b8[e], acc);
-    }
-  }
-  acc += __shfl_xor_sync(0xffffffffu, acc, 1);
-  acc += __shfl_xor_sync(0xffffffffu, acc, 2);
-  if (q == 0 && pair < n_pairs) out[pair] = acc;
-}
-
 int attn_tcgen05_gen_bwd(const void* qkv, const float* inv_norm, const float* scale, const float* bias, const void* o, const void* d_o,
                          const float* lse, void* dqkv, float* dscale, float* dbias, float* ws, const AttnGeom& g, cudaStream_t stream,
                          float* det_part) {
-  if (ws == nullptr) {
-    set_error("window_attn_bwd (tcgen05): a workspace of B*H*W*heads floats is required for this geometry");
-    return SWINB200_ERR_INVALID_ARG;
-  }
   const long long n_pairs = (long long)g.B * g.H * g.W * g.heads;
-  attn_gen_rowdot_kernel<<<(unsigned)((n_pairs * 4 + 255) / 256), 256, 0, stream>>>((const __nv_bfloat16*)o, (const __nv_bfloat16*)d_o, ws,
-                                                                                      n_pairs, g.C / g.heads);
+  attn_rowdot_kernel<<<(unsigned)((n_pairs * 4 + 255) / 256), 256, 0, stream>>>((const __nv_bfloat16*)o, (const __nv_bfloat16*)d_o, ws,
+                                                                                n_pairs, g.C / g.heads);
   SWB_LAUNCH_CHECK();
   GenArgs a{};
   a.qkv = (const __nv_bfloat16*)qkv; a.d_o = (const __nv_bfloat16*)d_o; a.inv_norm = inv_norm; a.scale = scale; a.bias = bias;

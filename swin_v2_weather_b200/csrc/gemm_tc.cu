@@ -1021,14 +1021,11 @@ static int launch_tc_impl(const CUtensorMap& tmA, const CUtensorMap& tmB, const 
   return SWINB200_OK;
 }
 
-// p.num_m_tiles counts 128-row tiles for single-CTA launches and 256-row pair tiles for PAIR launches
+// BN 256 runs as CTA pairs, BN 128 (N <= 128) as single CTAs; p.num_m_tiles counts 256-row pair tiles or 128-row tiles to match
 template <int BN, bool A_MN, bool B_MN, int EPI, bool DET = false>
 static int launch_tc(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmD, const CUtensorMap& tmD2,
                      const GemmTcParams& p, cudaStream_t s) {
-  if (p.pair) {
-    if constexpr (BN == 256) return launch_tc_impl<BN, A_MN, B_MN, EPI, true, DET>(tmA, tmB, tmD, tmD2, p, s);
-  }
-  return launch_tc_impl<BN, A_MN, B_MN, EPI, false, DET>(tmA, tmB, tmD, tmD2, p, s);
+  return launch_tc_impl<BN, A_MN, B_MN, EPI, BN == 256, DET>(tmA, tmB, tmD, tmD2, p, s);
 }
 
 // Only the operand-major / epilogue pairs the model uses are instantiated:
@@ -1103,11 +1100,7 @@ int gemm_tcgen05(int M, int N, int K, const void* A, int a_major, int lda, const
     }
   }
   p.atomic_out = (epilogue == SWINB200_EPI_F32 && (accumulate || split_k > 1)) ? 1 : 0;
-  {
-    static int pair_env = -1;
-    if (pair_env < 0) { const char* e = getenv("SWINB200_GEMM_PAIR"); pair_env = e ? atoi(e) : 1; }
-    p.pair = ((pair_env || epilogue == SWINB200_EPI_BIAS_LN) && (BN == 256 || BN == 192)) ? 1 : 0;   // BIAS_LN exists as a pair kernel only
-  }
+  p.pair = (BN == 256 || BN == 192) ? 1 : 0;
   p.num_m_tiles = p.pair ? (M + 2 * GBM - 1) / (2 * GBM) : (M + GBM - 1) / GBM;
   p.num_n_tiles = (N + BN - 1) / BN;
   p.kb_total = (K + GBK - 1) / GBK;
@@ -1134,10 +1127,7 @@ int gemm_tcgen05(int M, int N, int K, const void* A, int a_major, int lda, const
     if (e) return e;
   }
 
-  if (qknorm) {
-    if (p.pair) return launch_tc_impl<192, false, false, SWINB200_EPI_BIAS_QKNORM, true>(tmA, tmB, tmD, tmD2, p, stream);
-    return launch_tc_impl<192, false, false, SWINB200_EPI_BIAS_QKNORM, false>(tmA, tmB, tmD, tmD2, p, stream);
-  }
+  if (qknorm) return launch_tc_impl<192, false, false, SWINB200_EPI_BIAS_QKNORM, true>(tmA, tmB, tmD, tmD2, p, stream);
   if (epilogue == SWINB200_EPI_BIAS_LN) return launch_tc_impl<256, false, false, SWINB200_EPI_BIAS_LN, true>(tmA, tmB, tmD, tmD2, p, stream);
   if (part != nullptr) {
     // every split writes its own slice with plain stores; the slices (and the column-sum rows) are then added in split order

@@ -6,8 +6,6 @@ activation storage + fp32 row statistics -- ~24.6 KB/token, 1.6 GB per block per
 """
 from __future__ import annotations
 
-import os
-
 import weakref
 from typing import Dict, Optional, Tuple
 
@@ -198,27 +196,20 @@ class SwinBlockFn(torch.autograd.Function):
         # Order: every tensor is consumed right after it was produced, and consecutive kernels alternate their direction over
         # the token rows (GEMMs ascend, the row-wise kernels descend), so each one starts on the ~100 MB its predecessor left
         # in L2.  The two weight gradients that do not touch the fresh tensor (fc2: dz2, g; proj: dz1, o) run last.
-        reorder = os.environ.get("SWINB200_BWD_ORDER", "1") != "0"
         dh = ops.gemm(mode, dz2, 0, w2, 1, EPI_DGELU, aux=h)                                     # (T, hidden)
-        if not reorder:
-            dw_fc2 = wgrad(dz2, g, C, hid, "w_fc2")
         dx_mid = ops.gemm(mode, dh, 0, w1, 1, EPI_ADD_F32, aux=dx_out)                           # fp32 (T, C)
         # weight + bias gradient of fc1 in one kernel (the bias gradient is the column sum of the dh tiles the GEMM stages)
         dw_fc1, dbias_fc1 = ops.linear_wgrad(mode, dh, xb_mid, acc["w_fc1"].view(hid, C), acc["b_fc1"], ops.wgrad_split_k(hid, C, T))
         del dh
-        if reorder:
-            dw_fc2 = wgrad(dz2, g, C, hid, "w_fc2")
+        dw_fc2 = wgrad(dz2, g, C, hid, "w_fc2")
         # ---- attention branch: x_mid = x + dp1 * LN1(proj(attn(qkv(xb))))
         dz1, dg1, db1, dbias_proj = ops.ln_residual_bwd(dx_mid, z1, st1, n1_w.detach(), dp1, H * W, mode, acc=acc["ln1"].view(3, C))
         d_o = ops.gemm(mode, dz1, 0, wp, 1, EPI_BIAS)                                            # (T, C)
-        if not reorder:
-            dw_proj = wgrad(dz1, o, C, C, "w_proj")
         dqkv, dscale, dbias_tab = ops.window_attn_bwd(qkv, inv_norm, scale_c, bias_c, o, d_o, lse, B, H, W, C, heads, Wh, Ww,
                                                        s0, s1, mode, dscale=acc["dscale"])
         dx_in = ops.gemm(mode, dqkv, 0, wq, 1, EPI_ADD_F32, aux=dx_mid)                          # fp32 (T, C)
         dw_qkv, dbias_qkv = ops.linear_wgrad(mode, dqkv, xb, acc["w_qkv"].view(3 * C, C), acc["b_qkv"], ops.wgrad_split_k(3 * C, C, T))
-        if reorder:
-            dw_proj = wgrad(dz1, o, C, C, "w_proj")
+        dw_proj = wgrad(dz1, o, C, C, "w_proj")
         return (dx_in.view(B, H, W, C), None, dscale, dbias_tab, dw_qkv, dbias_qkv, dw_proj, dbias_proj, dg1, db1, dw_fc1,
                 dbias_fc1, dw_fc2, dbias_fc2, dg2, db2, None, None, None, None)
 

@@ -12,7 +12,6 @@ d(scale) / d(bias)) runs through the fixed-order `swinb200_*_det` entry points, 
 from __future__ import annotations
 
 import os
-import warnings
 
 from dataclasses import dataclass
 from typing import Optional
@@ -233,15 +232,13 @@ def ln_residual_fwd(z, x_in, gamma, beta, sample_scale, pos, rows_per_sample: in
 
 
 def linear_wgrad(mode: ComputeMode, dy: torch.Tensor, x: torch.Tensor, dw: torch.Tensor, dbias: Optional[torch.Tensor],
-                 split_k: int, fuse: Optional[bool] = None):
+                 split_k: int, fuse: bool = True):
     """dw (n_out, n_in) fp32 += dy^T x ;  dbias (n_out) fp32 += column sums of dy  (both pre-zeroed accumulators).
     tcgen05, n_out a multiple of 256: ONE kernel -- the epilogue warps of the weight-gradient GEMM sum the dy tiles the main
     loop stages in shared memory (swinb200_linear_wgrad), so dy is not read again by a column-sum pass.  Otherwise (and with
-    SWINB200_FUSE_COLSUM=0): the split-K GEMM followed by swinb200_colsum."""
+    fuse=False): the split-K GEMM followed by swinb200_colsum."""
     T, n_out = dy.shape
     n_in = x.shape[1]
-    if fuse is None:
-        fuse = os.environ.get("SWINB200_FUSE_COLSUM", "1") != "0"
     if fuse and dbias is not None and mode.gemm_backend == BACKEND_TCGEN05 and n_out % 256 == 0 and n_in >= 256:
         if deterministic():
             part = _scratch(split_k * (n_out * n_in + n_out), dy.device)
@@ -396,24 +393,17 @@ def window_attn_bwd(qkv, inv_norm, scale, bias, o, d_o, lse, B, H, W, C, heads, 
     if dscale is None:
         dscale = torch.zeros((heads,), dtype=torch.float32, device=qkv.device)
     dbias = torch.zeros((heads, L, L), dtype=torch.float32, device=qkv.device) if bias is not None else None
-    # scratch for the row term D = <dO, O> (tcgen05 back end: enables the persistent kernel)
+    # scratch for the row term D = <dO, O> (required by the tcgen05 back end)
     ws = torch.empty((qkv.shape[0] * heads,), dtype=torch.float32, device=qkv.device) if backend == BACKEND_TCGEN05 else None
     if deterministic():
         items = B * (H // Wh) * (W // Ww) * heads
         part = _scratch(items * (4 * ((L + 127) // 128) + (L * L if dbias is not None else 0)), qkv.device)
-        try:
-            _lib.call("swinb200_window_attn_bwd_det", backend, _chk(qkv, "qkv"), _code(qkv.dtype),
-                      _chk(inv_norm, "inv_norm", torch.float32), _chk(scale, "scale", torch.float32),
-                      _chk(bias, "bias", torch.float32, True), _chk(o, "o", qkv.dtype), _chk(d_o, "d_o", qkv.dtype),
-                      _chk(lse, "lse", torch.float32), dqkv.data_ptr(), dscale.data_ptr(), 0 if dbias is None else dbias.data_ptr(),
-                      0 if ws is None else ws.data_ptr(), B, H, W, C, heads, Wh, Ww, s0, s1, part.data_ptr(), part.numel(), _stream())
-            return dqkv, dscale, dbias
-        except SwinB200Error as e:
-            # the legacy kernels (SWINB200_ATTN_BWD=1/2) have no deterministic version: as torch does for such an op, an error,
-            # or a warning and the ordinary kernel under warn_only=True
-            if e.code != _lib.ERR_UNSUPPORTED or not torch.is_deterministic_algorithms_warn_only_enabled():
-                raise
-            warnings.warn(f"window_attn_bwd has no deterministic version for this configuration: {e}")
+        _lib.call("swinb200_window_attn_bwd_det", backend, _chk(qkv, "qkv"), _code(qkv.dtype),
+                  _chk(inv_norm, "inv_norm", torch.float32), _chk(scale, "scale", torch.float32),
+                  _chk(bias, "bias", torch.float32, True), _chk(o, "o", qkv.dtype), _chk(d_o, "d_o", qkv.dtype),
+                  _chk(lse, "lse", torch.float32), dqkv.data_ptr(), dscale.data_ptr(), 0 if dbias is None else dbias.data_ptr(),
+                  0 if ws is None else ws.data_ptr(), B, H, W, C, heads, Wh, Ww, s0, s1, part.data_ptr(), part.numel(), _stream())
+        return dqkv, dscale, dbias
     _lib.call("swinb200_window_attn_bwd", backend, _chk(qkv, "qkv"), _code(qkv.dtype),
               _chk(inv_norm, "inv_norm", torch.float32), _chk(scale, "scale", torch.float32),
               _chk(bias, "bias", torch.float32, True), _chk(o, "o", qkv.dtype), _chk(d_o, "d_o", qkv.dtype),

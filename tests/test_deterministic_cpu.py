@@ -49,6 +49,27 @@ def test_wgrad_det_rejects_what_it_is_not_built_for():
     assert b"bias table" in lib.swinb200_last_error()
 
 
+def test_tcgen05_attention_rejects_missing_workspace_or_unaligned_operands():
+    """The tcgen05 attention needs the D = <dO, O> workspace and 16-byte aligned operands at every geometry, in the plain and
+    the deterministic entry points alike; here at the shipped 9x18 windows / head_dim 96."""
+    lib = _lib.load()
+    tc, bf16, geom = _lib.BACKEND_TCGEN05, _lib.BF16, (1, 36, 72, 768, 8, 9, 18, 0, 0)
+    U = ctypes.c_void_p(18)
+
+    def bwd(qkv, ws):
+        return lib.swinb200_window_attn_bwd(tc, qkv, bf16, P, P, None, P, P, P, P, P, None, ws, *geom, None)
+
+    def bwd_det(ws):
+        return lib.swinb200_window_attn_bwd_det(tc, P, bf16, P, P, None, P, P, P, P, P, None, ws, *geom, P, 1 << 30, None)
+
+    for call in (lambda: bwd(P, None), lambda: bwd_det(None)):
+        assert call() == _lib.ERR_INVALID_ARG
+        assert b"workspace" in lib.swinb200_last_error()
+    for call in (lambda: lib.swinb200_window_attn_fwd(tc, U, bf16, P, None, P, P, *geom, None), lambda: bwd(U, P)):
+        assert call() == _lib.ERR_INVALID_ARG
+        assert b"16-byte aligned" in lib.swinb200_last_error()
+
+
 @pytest.fixture
 def recorder(monkeypatch):
     calls = []

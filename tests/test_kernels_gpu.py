@@ -474,6 +474,15 @@ GEMM_CASES = [
     (768, 3072, 1000, 1, 1, EPI_F32),       # wgrad, K tail
     (2304, 768, 1300, 1, 1, EPI_F32),
     (1168, 768, 648, 1, 1, EPI_F32),        # head wgrad: M tail
+    # N <= 128: single-CTA 128 x 128 tiles instead of CTA pairs, one row per instantiation, N tails included
+    (300, 128, 768, 0, 0, EPI_BIAS),
+    (333, 72, 520, 0, 0, EPI_BIAS_GELU),
+    (300, 120, 768, 0, 0, EPI_F32),
+    (515, 72, 768, 0, 1, EPI_BIAS),
+    (515, 128, 3072, 0, 1, EPI_DGELU),
+    (515, 96, 2304, 0, 1, EPI_ADD_F32),
+    (515, 72, 1168, 0, 1, EPI_F32),
+    (768, 72, 1000, 1, 1, EPI_F32),         # wgrad, N tail
 ]
 
 
@@ -579,6 +588,7 @@ def test_gemm_tcgen05_persistent_many_tiles():
     # more tiles than SMs: exercises the TMEM double buffering and the smem ring wrap-around
     run_gemm_case((128 * 40, 2304, 768, 0, 0, EPI_BIAS), torch.bfloat16, BACKEND_TCGEN05)
     run_gemm_case((128 * 40 + 17, 3072, 768, 0, 0, EPI_BIAS_GELU), torch.bfloat16, BACKEND_TCGEN05)
+    run_gemm_case((128 * 160 + 17, 96, 768, 0, 0, EPI_BIAS_GELU), torch.bfloat16, BACKEND_TCGEN05)   # single-CTA: 161 row tiles
 
 
 # ---- optimizer (SURVEY 8(f) rank 1) --------------------------------------------------------------------------
@@ -678,15 +688,3 @@ def test_patchify_cat_equals_patchify_of_concatenation(dtype):
     assert torch.equal(ops.patchify_cat(parts, 4, mode), ops.patchify(cat, 4, 0, mode))
     assert torch.equal(ops.patchify_cat([cat], 4, mode), ops.patchify(cat, 4, 0, mode))
 
-
-def test_alternate_kernel_variants_in_a_fresh_process():
-    """The env-selected variants (first-generation attention kernels, single-CTA statically scheduled GEMM) are read once
-    per process, so they are exercised in a child process: same parity tests, different kernels."""
-    import os
-    import subprocess
-    import sys
-    env = dict(os.environ, SWINB200_ATTN_FWD="1", SWINB200_ATTN_BWD="1", SWINB200_GEMM_PAIR="0")
-    sel = "test_window_attention_tcgen05 or test_gemm_tcgen05 or test_gemm_tcgen05_split_k or persistent_many_tiles"
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-q", "-x", "-k", sel, "-p", "no:cacheprovider"],
-                       env=env, capture_output=True, text=True, timeout=900, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]

@@ -1,4 +1,5 @@
-"""Per-phase cycle breakdown of the tcgen05 attention kernels at the full 180x360 geometry (bring-up aid)."""
+"""Per-phase cycle breakdown of the tcgen05 attention backward at the full 180x360 geometry, and the launch times of the
+forward and the backward (bring-up aid).  Only the backward kernel writes phase counters."""
 import sys
 import torch
 sys.path.insert(0, ".")
@@ -13,32 +14,29 @@ inv = ops.qk_normalize_(qkv, C, heads)
 scale = torch.full((heads,), 10.0, device="cuda")
 buf = torch.zeros(4096 * 16, dtype=torch.int64, device="cuda")
 for shift in ((0, 0), (4, 9)):
-    for name in ("fwd", "bwd"):
-        _lib.call("swinb200_debug_attn_phase_buffer", buf.data_ptr())
-        buf.zero_()
-        o, lse = ops.window_attn_fwd(qkv, scale, None, B, H, W, C, heads, 9, 18, shift[0], shift[1], ops.MODE_BF16, backend=BACKEND_TCGEN05)
-        if name == "bwd":
-            buf.zero_()
-            d_o = torch.randn_like(o)
-            ops.window_attn_bwd(qkv, inv, scale, None, o, d_o, lse, B, H, W, C, heads, 9, 18, shift[0], shift[1], ops.MODE_BF16, backend=BACKEND_TCGEN05)
-        torch.cuda.synchronize()
-        _lib.call("swinb200_debug_attn_phase_buffer", 0)
-        if name == "fwd":   # persistent kernel: [wait S, softmax, wait PV, O read, park+barrier, scatter+barrier, token table / release]
-            st = buf.view(4096, 16)[:148, :8].double()
-            items = 3200 / 148
-            print(name, shift, "mean cycles per phase per item:", [int(v / items) for v in st.mean(0).tolist()], "total/item", int(st.sum(1).mean() / items))
-        else:   # persistent kernel: per-CTA accumulated cycles per phase over all its items
-            st = buf.view(4096, 16)[:148, :16].double()
-            items = 3200 / 148
-            print(name, shift, "mean cycles per phase per item:", [int(v / items) for v in st.mean(0).tolist()], "total/item", int(st.sum(1).mean() / items))
-        # timing
+    def fwd():
+        return ops.window_attn_fwd(qkv, scale, None, B, H, W, C, heads, 9, 18, shift[0], shift[1], ops.MODE_BF16, backend=BACKEND_TCGEN05)
+
+    o, lse = fwd()
+    d_o = torch.randn_like(o)
+
+    def bwd():
+        ops.window_attn_bwd(qkv, inv, scale, None, o, d_o, lse, B, H, W, C, heads, 9, 18, shift[0], shift[1], ops.MODE_BF16, backend=BACKEND_TCGEN05)
+
+    _lib.call("swinb200_debug_attn_phase_buffer", buf.data_ptr())
+    buf.zero_()
+    bwd()
+    torch.cuda.synchronize()
+    _lib.call("swinb200_debug_attn_phase_buffer", 0)
+    # persistent kernel: per-CTA accumulated cycles per phase over all its items
+    st = buf.view(4096, 16)[:148, :16].double()
+    items = 3200 / 148
+    print("bwd", shift, "mean cycles per phase per item:", [int(v / items) for v in st.mean(0).tolist()], "total/item", int(st.sum(1).mean() / items))
+    for name, run in (("fwd", fwd), ("bwd", bwd)):
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
         ev[0].record()
         for _ in range(5):
-            if name == "fwd":
-                ops.window_attn_fwd(qkv, scale, None, B, H, W, C, heads, 9, 18, shift[0], shift[1], ops.MODE_BF16, backend=BACKEND_TCGEN05)
-            else:
-                ops.window_attn_bwd(qkv, inv, scale, None, o, d_o, lse, B, H, W, C, heads, 9, 18, shift[0], shift[1], ops.MODE_BF16, backend=BACKEND_TCGEN05)
+            run()
         ev[1].record()
         torch.cuda.synchronize()
         print("   ", name, "time per launch: %.1f us" % (ev[0].elapsed_time(ev[1]) * 1000 / 5))
