@@ -38,6 +38,8 @@ enum {
                                    reciprocal norms.  tcgen05 back end, head_dim 96 only.               (D: act)  */
   SWINB200_EPI_BIAS_LN = 6,   /* internal to swinb200_linear_ln_residual: D = acc + bias, then LayerNorm + residual of
                                    every finished 128-row block inside the epilogue                      (D: act)  */
+  SWINB200_EPI_BIAS_GELU_FWD = 7, /* D = gelu_erf(act(acc + bias)): the D output of BIAS_GELU, bit for bit, without the
+                                     pre-activation D2 (forward-only runs, where no backward reads it; D2 unused) (D: act) */
 };
 /* GEMM back ends */
 enum { SWINB200_GEMM_SIMT = 0, SWINB200_GEMM_TCGEN05 = 1 };
@@ -92,7 +94,8 @@ int swinb200_unpatchify_norm(const void* y, int act_dtype, const float* skip, in
  * Replaces nn.Linear forward (a0,b0), its input gradient (a0,b1 with B = weight) and its weight
  * gradient (a1,b1) -- swinv2_global.py:181,199,300,319,381-386,544,787 and their autograd
  * backward.  in_dtype is the storage type of A and B.  split_k > 1 is allowed only with
- * SWINB200_EPI_F32 and accumulate (atomic fp32 adds into a pre-initialised D).
+ * SWINB200_EPI_F32 and accumulate (atomic fp32 adds into a pre-initialised D).  BIAS_GELU_FWD, like BIAS_GELU, is a
+ * forward epilogue (a_major 0, b_major 0 on the tcgen05 back end).
  * backend SWINB200_GEMM_TCGEN05 requires in_dtype == SWINB200_BF16. */
 int swinb200_gemm(int backend, int M, int N, int K, const void* A, int a_major, int lda, const void* B,
                   int b_major, int ldb, int in_dtype, int epilogue, const float* bias, void* D, int ldd,
@@ -128,7 +131,8 @@ int swinb200_linear_ln_residual(int backend, int M, int N, int K, const void* A,
  *       x_out = (x_in ? x_in : 0) + u ;  xb_out = act(x_out) ;  stats[row] = (mean, rstd)
  *   == `x + drop_path(norm(branch))` (swinv2_global.py:490,494), and PatchEmbed.norm + pos_embed add
  *   (swinv2_global.py:545,780) with x_in = NULL, pos = pos_embed transposed to token-major
- *   (rows_per_sample, C) fp32 by swinb200_transpose_f32.
+ *   (rows_per_sample, C) fp32 by swinb200_transpose_f32.  stats may be NULL (forward-only runs): the statistics are
+ *   then not stored and everything else is unchanged.
  * bwd:  given dx = dL/dx_out (fp32): dz (act) ; dgamma, dbeta, dbias_prev += column sums (fp32 atomics,
  *       caller zero-initialises).  dL/dx_in is dx itself (identity path), handled by the caller. */
 int swinb200_ln_residual_fwd(const void* z, int act_dtype, const float* x_in, const float* gamma,
@@ -150,7 +154,7 @@ int swinb200_colsum(const void* x, int act_dtype, float* out, int rows, int cols
 /* ---- windowed cosine attention ----------------------------------------------------------------------
  * qk_normalize: in place on qkv (T, 3C): q and k of every (token, head) are divided by
  *   max(||.||_2, 1e-12) (F.normalize, swinv2_global.py:185,304); inv_norm (T, 2, heads) fp32 receives
- *   the reciprocal factors for backward.
+ *   the reciprocal factors for backward (nullable: not stored).  The same holds for D2 of SWINB200_EPI_BIAS_QKNORM.
  * window_attn_fwd: per (sample, window, head), with roll(-s)/window_partition/window_reverse/roll(+s)
  *   (swinv2_global.py:89-119,446-478) folded into addressing:
  *     S = scale[h] * qhat khat^T (+ bias[h]) (+ shift mask) ; P = softmax(S) ; O = P v
@@ -160,7 +164,8 @@ int swinb200_colsum(const void* x, int act_dtype, float* out, int rows, int cols
  *   same predicate as the reference's (nW, L, L) buffer for bit-exact checks.
  *   o: (T, C) act in un-rolled token order; lse: (2, B, nW, heads, L) fp32 -- plane 0 = log-sum-exp of every softmax row,
  *   plane 1 = the row's softmax-weighted mean cosine sum_j P_ij cos_ij (zero from back ends whose backward does not use it;
- *   the tcgen05 backward accumulates d(scale) against it so that the sum is insensitive to the rounding of O).
+ *   the tcgen05 backward accumulates d(scale) against it so that the sum is insensitive to the rounding of O).  lse may
+ *   be NULL when no backward follows: neither plane is written, o is unchanged.
  * window_attn_bwd: dqkv (T, 3C) act = gradients w.r.t. the *un-normalised* q, k and v;
  *   dscale (heads) += sum dS * cos ; dbias (heads, L, L) += sum_windows dS (nullable).
  *   ws: required by the tcgen05 back end; T*heads floats (the library allocates nothing), which receive the row term

@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(_HERE, "libswinb200.so")
 # enums of include/swinb200.h
 F32, BF16 = 0, 1
 EPI_BIAS, EPI_BIAS_GELU, EPI_DGELU, EPI_ADD_F32, EPI_F32, EPI_BIAS_QKNORM = 0, 1, 2, 3, 4, 5
+EPI_BIAS_GELU_FWD = 7     # BIAS_GELU's activation output alone (forward-only runs); 6 is internal to swinb200_linear_ln_residual
 BACKEND_SIMT, BACKEND_TCGEN05 = 0, 1
 
 _P = c_void_p

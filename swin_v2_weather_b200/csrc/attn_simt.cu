@@ -37,7 +37,9 @@ __device__ __forceinline__ int pad_d(int d) { return sizeof(T) == 4 ? d + 1 : d 
 // ------------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------------
-template <typename T, bool GLOBAL_KV>
+// LSE = false: forward-only launches (lse == NULL).  A compile-time flag rather than a runtime test: the test pushed the
+// fp32 global-K/V kernel into a spill.
+template <typename T, bool GLOBAL_KV, bool LSE = true>
 __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_fwd_kernel(const T* __restrict__ qkv, const float* __restrict__ scale_p,
                                                                         const float* __restrict__ bias, T* __restrict__ o,
                                                                         float* __restrict__ lse, WinGeom g) {
@@ -110,7 +112,7 @@ __global__ void __launch_bounds__(kAttnWarps * 32) attn_simt_fwd_kernel(const T*
       for (int j = 0; j < L; ++j) acc = fmaf(myp[j], Act<T>::ld(v_row(j) + c), acc);
       Act<T>::st(orow + c, acc * inv);
     }
-    if (lane == 0) lse[(((size_t)b * g.nW() + w) * g.heads + head) * L + i] = mx + logf(sum);
+    if (LSE && lane == 0) lse[(((size_t)b * g.nW() + w) * g.heads + head) * L + i] = mx + logf(sum);
     __syncwarp();
   }
 }
@@ -324,7 +326,8 @@ static int launch_fwd(const T* qkv, const float* scale, const float* bias, T* o,
     set_error("window_attn_fwd (CUDA-core back end): window %dx%d, head_dim %d needs %zu B of shared memory", g.Wh, g.Ww, g.d(), smem);
     return SWINB200_ERR_UNSUPPORTED;
   }
-  auto kernel = global_kv ? attn_simt_fwd_kernel<T, true> : attn_simt_fwd_kernel<T, false>;
+  auto kernel = global_kv ? (lse ? attn_simt_fwd_kernel<T, true> : attn_simt_fwd_kernel<T, true, false>)
+                          : (lse ? attn_simt_fwd_kernel<T, false> : attn_simt_fwd_kernel<T, false, false>);
   SWB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kernel<<<g.B * g.nW() * g.heads, kAttnWarps * 32, smem, s>>>(qkv, scale, bias, o, lse, g);
   SWB_LAUNCH_CHECK();
@@ -382,7 +385,7 @@ using namespace swinb200;
 extern "C" int swinb200_window_attn_fwd(int backend, const void* qkv, int act_dtype, const float* scale, const float* bias,
                                         void* o, float* lse, int B, int H, int W, int C, int heads, int Wh, int Ww, int s0,
                                         int s1, void* stream) {
-  SWB_CHECK_ARG(qkv && scale && o && lse, "window_attn_fwd: null pointer");
+  SWB_CHECK_ARG(qkv && scale && o, "window_attn_fwd: null pointer");     // lse may be null (forward-only)
   if (int e = check_geom("window_attn_fwd", B, H, W, C, heads, Wh, Ww, s0, s1)) return e;
   const WinGeom g{B, H, W, C, heads, Wh, Ww, s0, s1};
   cudaStream_t s = (cudaStream_t)stream;
@@ -392,7 +395,8 @@ extern "C" int swinb200_window_attn_fwd(int backend, const void* qkv, int act_dt
   }
   SWB_CHECK_ARG(backend == SWINB200_GEMM_SIMT, "window_attn_fwd: unknown backend %d", backend);
   // second plane of `lse` (softmax-weighted mean cosine): not used by this back end's backward, defined as zero
-  SWB_CUDA(cudaMemsetAsync(lse + (size_t)B * g.nW() * heads * Wh * Ww, 0, sizeof(float) * (size_t)B * g.nW() * heads * Wh * Ww, s));
+  if (lse != nullptr)
+    SWB_CUDA(cudaMemsetAsync(lse + (size_t)B * g.nW() * heads * Wh * Ww, 0, sizeof(float) * (size_t)B * g.nW() * heads * Wh * Ww, s));
   if (act_dtype == SWINB200_BF16) return launch_fwd<__nv_bfloat16>((const __nv_bfloat16*)qkv, scale, bias, (__nv_bfloat16*)o, lse, g, s);
   if (act_dtype == SWINB200_F32) return launch_fwd<float>((const float*)qkv, scale, bias, (float*)o, lse, g, s);
   SWB_CHECK_ARG(false, "window_attn_fwd: bad act_dtype %d", act_dtype);

@@ -306,7 +306,7 @@ attn_tc_fwd4_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __nv_bfloa
               tmem_st_32x8(t_s + c0 / 2, pack8(p, 0), pack8(p, 8));
             }
           }
-          if (row_ok) {
+          if (row_ok && lse != nullptr) {       // null: forward-only run
             const size_t ri = (((size_t)b * g.nW + w) * g.heads + head) * L + n;
             lse[ri] = (row_max + log2f(row_sum)) * 0.6931471805599453f;
             // second plane: E_P[cos] of the row.  The backward accumulates d(scale) = sum dS (cos - E_P[cos]); the row sum of dS

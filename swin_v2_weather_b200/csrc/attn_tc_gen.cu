@@ -72,7 +72,7 @@ struct GenArgs {
   const float* scale;            // (heads) exp(min(logit_scale, ln 100))
   const float* bias;             // (heads, L, L) or null
   const float* Dpre;             // (T, heads) <dO, O>                         (backward)
-  float* lse;                    // (2, B, nW, heads, L): LSE | E_P[cos];  written by forward, read by backward
+  float* lse;                    // (2, B, nW, heads, L): LSE | E_P[cos];  written by forward (unless null), read by backward
   __nv_bfloat16* out;            // forward: o (T, C);  backward: dqkv (T, 3C)
   float* dscale;                 // (heads)
   float* dbias;                  // (heads, L, L) or null
@@ -536,7 +536,7 @@ __global__ void __launch_bounds__(128) attn_gen_kernel(const GenArgs a, const At
   };
 
   if (MODE == kModeFwd) {
-    if (row_ok) {
+    if (row_ok && a.lse != nullptr) {       // null: forward-only run
       const float off = bounded ? scale_l2 : row_max;
       a.lse[row_base + nx] = (off + log2f(row_sum)) * kLn2;
       a.lse[(size_t)g.B * g.nW * g.heads * L + row_base + nx] = cos_sum / row_sum;

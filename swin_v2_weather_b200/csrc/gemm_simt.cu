@@ -77,6 +77,9 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(int M, int N, int K, con
         Act<T>::st(reinterpret_cast<T*>(D2v) + o, v);
         // GELU is evaluated on the stored (rounded) pre-activation so forward and backward agree
         Act<T>::st(reinterpret_cast<T*>(Dv) + o, gelu_erf(Act<T>::round(v)));
+      } else if (EPI == SWINB200_EPI_BIAS_GELU_FWD) {
+        if (bias) v += bias[n];
+        Act<T>::st(reinterpret_cast<T*>(Dv) + o, gelu_erf(Act<T>::round(v)));   // BIAS_GELU's D without D2
       } else if (EPI == SWINB200_EPI_DGELU) {
         const float h = Act<T>::ld(reinterpret_cast<const T*>(auxv) + (size_t)m * ld_aux + n);
         Act<T>::st(reinterpret_cast<T*>(Dv) + o, v * gelu_erf_grad(h));
@@ -102,6 +105,7 @@ static int launch_simt(int M, int N, int K, const T* A, int a_major, int lda, co
   switch (epi) {
     case SWINB200_EPI_BIAS: SWB_SIMT(SWINB200_EPI_BIAS); break;
     case SWINB200_EPI_BIAS_GELU: SWB_SIMT(SWINB200_EPI_BIAS_GELU); break;
+    case SWINB200_EPI_BIAS_GELU_FWD: SWB_SIMT(SWINB200_EPI_BIAS_GELU_FWD); break;
     case SWINB200_EPI_DGELU: SWB_SIMT(SWINB200_EPI_DGELU); break;
     case SWINB200_EPI_ADD_F32: SWB_SIMT(SWINB200_EPI_ADD_F32); break;
     case SWINB200_EPI_F32: SWB_SIMT(SWINB200_EPI_F32); break;
@@ -128,12 +132,13 @@ extern "C" int swinb200_gemm(int backend, int M, int N, int K, const void* A, in
   SWB_CHECK_ARG(a_major == 0 || a_major == 1, "gemm: a_major must be 0/1");
   SWB_CHECK_ARG(b_major == 0 || b_major == 1, "gemm: b_major must be 0/1");
   SWB_CHECK_ARG(lda >= (a_major ? M : K) && ldb >= (b_major ? N : K) && ldd >= N, "gemm: leading dimension too small");
-  SWB_CHECK_ARG(epilogue >= SWINB200_EPI_BIAS && epilogue <= SWINB200_EPI_BIAS_QKNORM, "gemm: unknown epilogue %d", epilogue);
+  SWB_CHECK_ARG((epilogue >= SWINB200_EPI_BIAS && epilogue <= SWINB200_EPI_BIAS_QKNORM) || epilogue == SWINB200_EPI_BIAS_GELU_FWD,
+                "gemm: unknown epilogue %d", epilogue);
   if (epilogue == SWINB200_EPI_BIAS_QKNORM) {
     SWB_CHECK_ARG(backend == SWINB200_GEMM_TCGEN05 && in_dtype == SWINB200_BF16 && out_dtype == SWINB200_BF16,
                   "gemm: BIAS_QKNORM is a tcgen05 / bf16 epilogue (use BIAS + swinb200_qk_normalize elsewhere)");
-    SWB_CHECK_ARG(D2 != nullptr && ld_aux == 96 && N % 288 == 0 && a_major == 0 && b_major == 0,
-                  "gemm: BIAS_QKNORM needs D2 (inverse norms), head_dim 96 and N = 3*C with C a multiple of 96");
+    SWB_CHECK_ARG(ld_aux == 96 && N % 288 == 0 && a_major == 0 && b_major == 0,
+                  "gemm: BIAS_QKNORM needs head_dim 96 and N = 3*C with C a multiple of 96");
     return gemm_tcgen05(M, N, K, A, a_major, lda, B, b_major, ldb, epilogue, bias, D, ldd, D2, aux, ld_aux, accumulate, 1, (cudaStream_t)stream);
   }
   const bool f32_out = (epilogue == SWINB200_EPI_ADD_F32 || epilogue == SWINB200_EPI_F32);

@@ -43,7 +43,7 @@ struct GemmTcParams {
   int M, N, K;
   const float* bias;
   const void* aux;
-  float* inv_norm;   // BIAS_QKNORM: (M, 2*N/(3*96)) reciprocal L2 norms of the q / k head vectors
+  float* inv_norm;   // BIAS_QKNORM: (M, 2*N/(3*96)) reciprocal L2 norms of the q / k head vectors, or null (not stored)
   int ld_aux;
   int pair;        // 1 = CTA-pair (cta_group::2) launch: 256 x 256 tiles over two SMs
   int debug;       // bring-up timing experiments (SWINB200_GEMM_DEBUG): 1 = no staging wait, 2 = no store, 4 = no tmem ld wait
@@ -471,7 +471,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     unsigned char* stg_base = smem + Cfg::kOffStaging + ew * kSB * kStagingBytes;
     uint32_t stg_sel = 0;                  // staging buffer of the next piece
     // Each warp stages and stores its own 32 rows: no cross-warp barrier sits between tcgen05.ld and the TMA store.
-    constexpr bool kBiasEpi = (EPI == SWINB200_EPI_BIAS || EPI == SWINB200_EPI_BIAS_GELU || EPI == SWINB200_EPI_BIAS_QKNORM || kLn);
+    constexpr bool kBiasEpi = (EPI == SWINB200_EPI_BIAS || EPI == SWINB200_EPI_BIAS_GELU || EPI == SWINB200_EPI_BIAS_GELU_FWD ||
+                               EPI == SWINB200_EPI_BIAS_QKNORM || kLn);
     constexpr int kChunksPerGroup = (kNumChunks + kEpiGroups - 1) / kEpiGroups;
     constexpr int kBiasSlots = kChunksPerGroup * kChunkCols;
     static_assert(!kBiasEpi || kBiasSlots <= 64, "bias slices must fit");
@@ -737,7 +738,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               const int hp = (pc / 3) * 3;                              // first piece of this piece's head
               const float tot = ssq[hp * GBM + r] + ssq[(hp + 1) * GBM + r] + ssq[(hp + 2) * GBM + r];
               inv = 1.0f / fmaxf(sqrtf(tot), 1e-12f);
-              if (pc == hp && row_ok) p.inv_norm[(size_t)m * ((p.N / 3) * 2 / 96) + nb / 96] = inv;
+              if (pc == hp && row_ok && p.inv_norm != nullptr) p.inv_norm[(size_t)m * ((p.N / 3) * 2 / 96) + nb / 96] = inv;
             }
             unsigned char* stg0 = stg_base + (stg_sel & (kSB - 1)) * kStagingBytes;
             stg_sel ^= 1;
@@ -848,6 +849,20 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           for (int g = 0; g < 4; ++g) {           // 4 x (4 fp32)
             v[g * 4 + 0] += __uint_as_float(aux_cur[g].x); v[g * 4 + 1] += __uint_as_float(aux_cur[g].y);
             v[g * 4 + 2] += __uint_as_float(aux_cur[g].z); v[g * 4 + 3] += __uint_as_float(aux_cur[g].w);
+          }
+        }
+        if constexpr (EPI == SWINB200_EPI_BIAS_GELU_FWD) {
+          // forward-only fc1: the activation of BIAS_GELU's second pass -- GELU of the bf16-rounded pre-activation, same
+          // rounding, same polynomial, so the bits equal BIAS_GELU's D -- in one pass, the pre-activation is never stored
+#pragma unroll
+          for (int c = 0; c < 4; ++c) {
+            float h8[8];
+            unpack_bf16x2(pack_bf16x2(v[c * 8 + 0], v[c * 8 + 1]), h8[0], h8[1]);
+            unpack_bf16x2(pack_bf16x2(v[c * 8 + 2], v[c * 8 + 3]), h8[2], h8[3]);
+            unpack_bf16x2(pack_bf16x2(v[c * 8 + 4], v[c * 8 + 5]), h8[4], h8[5]);
+            unpack_bf16x2(pack_bf16x2(v[c * 8 + 6], v[c * 8 + 7]), h8[6], h8[7]);
+#pragma unroll
+            for (int e = 0; e < 8; e += 2) gelu_fast2(h8[e], h8[e + 1], v[c * 8 + e], v[c * 8 + e + 1]);
           }
         }
         // ---- stage this warp's 32 rows of the chunk and hand them to the copy engine; the warp's previous store must
@@ -1029,7 +1044,7 @@ static int launch_tc(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUten
 }
 
 // Only the operand-major / epilogue pairs the model uses are instantiated:
-//   forward  (A k-major, B k-major) : BIAS, BIAS_GELU, F32
+//   forward  (A k-major, B k-major) : BIAS, BIAS_GELU, BIAS_GELU_FWD (forward-only fc1), F32
 //   dgrad    (A k-major, B n-major) : BIAS (no bias pointer), DGELU, ADD_F32, F32
 //   wgrad    (A m-major, B n-major) : F32 (plain or split-K reduce-add)
 template <int BN>
@@ -1038,6 +1053,7 @@ static int dispatch(int epi, int a_major, int b_major, const CUtensorMap& tmA, c
   if (!a_major && !b_major) {
     if (epi == SWINB200_EPI_BIAS) return launch_tc<BN, false, false, SWINB200_EPI_BIAS>(tmA, tmB, tmD, tmD2, p, s);
     if (epi == SWINB200_EPI_BIAS_GELU) return launch_tc<BN, false, false, SWINB200_EPI_BIAS_GELU>(tmA, tmB, tmD, tmD2, p, s);
+    if (epi == SWINB200_EPI_BIAS_GELU_FWD) return launch_tc<BN, false, false, SWINB200_EPI_BIAS_GELU_FWD>(tmA, tmB, tmD, tmD2, p, s);
     if (epi == SWINB200_EPI_F32) return launch_tc<BN, false, false, SWINB200_EPI_F32>(tmA, tmB, tmD, tmD2, p, s);
   } else if (!a_major && b_major) {
     if (epi == SWINB200_EPI_BIAS) return launch_tc<BN, false, true, SWINB200_EPI_BIAS>(tmA, tmB, tmD, tmD2, p, s);

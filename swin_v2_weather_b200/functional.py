@@ -3,6 +3,10 @@ kernels (swin_v2_weather_b200/ops.py).  Nothing here computes with PyTorch ops e
 
 Saved-for-backward per block (bf16 mode, per token): xb, qkv (q^,k^,v), o, z1, xb_mid, h, g, z2 in
 activation storage + fp32 row statistics -- ~24.6 KB/token, 1.6 GB per block per 64,800-token sample.
+
+Forward-only runs (no gradient will be taken): `patch_embed_forward_only`, `block_forward_only` and `head_forward_only` issue
+the C-ABI sequence of the three Functions' forwards with fc1 on the single-output BIAS_GELU_FWD epilogue (the pre-activation
+h is never written) and NULL row statistics, and save nothing.  Every output is bit-identical to the training forward's.
 """
 from __future__ import annotations
 
@@ -12,7 +16,7 @@ from typing import Dict, Optional, Tuple
 import torch
 
 from . import ops
-from .ops import ComputeMode, EPI_ADD_F32, EPI_BIAS, EPI_BIAS_GELU, EPI_DGELU, EPI_F32
+from .ops import ComputeMode, EPI_ADD_F32, EPI_BIAS, EPI_BIAS_GELU, EPI_BIAS_GELU_FWD, EPI_DGELU, EPI_F32
 
 
 # ---- bf16 weight shadows ------------------------------------------------------------------------------
@@ -20,25 +24,37 @@ class _ShadowCache:
     """bf16 copies of fp32 master weights, refreshed when the parameter's version counter moves
     (optimizer.step() bumps it).  Parameters themselves are never replaced (optimizer / DDP hold them).
     Entries are validated by object identity (weak reference), version and storage pointer: `id()` values and
-    allocator blocks are both recycled once a model is freed, so neither alone identifies a parameter."""
+    allocator blocks are both recycled once a model is freed, so neither alone identifies a parameter.
+    The same entries hold the token-major fp32 copy of pos_embed that forward-only runs read (`pos_tokens`)."""
 
     def __init__(self):
-        self._store: Dict[int, Tuple[weakref.ref, int, int, torch.Tensor]] = {}
+        self._store: Dict[object, Tuple[weakref.ref, int, int, torch.Tensor]] = {}
 
-    def get(self, w: torch.Tensor, mode: ComputeMode) -> torch.Tensor:
-        if mode.act_dtype == torch.float32:
-            return w.detach()
-        key = id(w)
+    def _cached(self, key, w: torch.Tensor, shape, make) -> torch.Tensor:
+        """The entry `key` derived from `w` (expected `shape`), rebuilt by make(old buffer or None) when `w` has changed."""
         ent = self._store.get(key)
         ver, ptr = w._version, w.data_ptr()
-        if ent is not None and ent[0]() is w and ent[1] == ver and ent[2] == ptr and ent[3].shape == w.shape:
+        if ent is not None and ent[0]() is w and ent[1] == ver and ent[2] == ptr and ent[3].shape == shape:
             return ent[3]
-        reuse = ent is not None and ent[0]() is w and ent[3].shape == w.shape and ent[3].device == w.device
-        sh = ops.cast_bf16(w.detach().contiguous(), ent[3] if reuse else None)
+        reuse = ent is not None and ent[0]() is w and ent[3].shape == shape and ent[3].device == w.device
+        sh = make(ent[3] if reuse else None)
         if ent is None:     # a new parameter: drop the shadows of parameters that have been freed since (discarded models)
             self._store = {k: v for k, v in self._store.items() if v[0]() is not None}
         self._store[key] = (weakref.ref(w), ver, ptr, sh)
         return sh
+
+    def get(self, w: torch.Tensor, mode: ComputeMode) -> torch.Tensor:
+        if mode.act_dtype == torch.float32:
+            return w.detach()
+        return self._cached(id(w), w, w.shape, lambda old: ops.cast_bf16(w.detach().contiguous(), old))
+
+    def pos_tokens(self, pos_embed: torch.Tensor) -> torch.Tensor:
+        """(H*W, E) fp32 token-major copy of the (1, E, H, W) pos_embed parameter, rewritten only when the parameter has changed
+        (forward-only runs; the training forward transposes it every call, as it always has)."""
+        E = pos_embed.shape[1]
+        rows = pos_embed.numel() // E
+        return self._cached(("pos_tokens", id(pos_embed)), pos_embed, (rows, E),
+                            lambda old: ops.transpose_f32(pos_embed.detach().reshape(E, rows), old))
 
     def peek(self, w: torch.Tensor):
         """The live shadow of `w` (possibly stale), or None -- lets the fused optimizer rewrite it in its own pass."""
@@ -123,6 +139,30 @@ class PatchEmbedFn(torch.autograd.Function):
             if ctx.in_std is not None:      # d/dx (x - m)/s = 1/s
                 dimg = dimg / ctx.in_std[:C0].view(1, C0, 1, 1)
         return (dimg, dw.view(wshape), dbias, dgamma, dbeta, dpos, None, None, None, None) + (None,) * n_more
+
+
+def patch_embed_forward_only(img, proj_w, proj_b, norm_w, norm_b, pos_embed, patch: int, mode: ComputeMode, in_mean, in_std,
+                             *more_channels):
+    """PatchEmbedFn.forward without saving anything: the LayerNorm statistics are not stored and the token-major pos_embed
+    comes from the shadow cache instead of a fresh transpose.  Returns (x (B, H, W, E), shadow) as the Function does."""
+    B, C0, Hi, Wi = img.shape
+    E = proj_w.shape[0]
+    H, W = Hi // patch, Wi // patch
+    if more_channels or in_mean is not None:
+        patches = ops.patchify_cat([img.contiguous()] + [t.detach().float().contiguous() for t in more_channels], patch, mode,
+                                   in_mean, in_std)
+    else:
+        patches = ops.patchify(img.contiguous(), patch, 0, mode)
+    w2 = SHADOWS.get(proj_w, mode).reshape(E, -1)
+    if w2.shape[1] != patches.shape[1]:
+        Cin = C0 + sum(t.shape[1] for t in more_channels)
+        raise ValueError(f"PatchEmbed: input has {Cin} channels, the projection expects {w2.shape[1] // (patch * patch)}")
+    z0 = ops.gemm(mode, patches, 0, w2, 0, EPI_BIAS, bias=proj_b.detach())
+    del patches
+    pos_tok = SHADOWS.pos_tokens(pos_embed) if pos_embed is not None else None
+    x, xb, _ = ops.ln_residual_fwd(z0, None, norm_w.detach(), norm_b.detach(), None, pos_tok, H * W, mode, need_stats=False)
+    shadow = xb if mode.act_dtype != torch.float32 else x.new_empty(0)
+    return x.view(B, H, W, E), shadow
 
 
 # ---- one SwinV2 block ------------------------------------------------------------------------------------
@@ -214,6 +254,35 @@ class SwinBlockFn(torch.autograd.Function):
                 dbias_fc1, dw_fc2, dbias_fc2, dg2, db2, None, None, None, None)
 
 
+def block_forward_only(x, xb, scale, bias, qkv_w, qkv_b, proj_w, proj_b, n1_w, n1_b, fc1_w, fc1_b, fc2_w, fc2_b, n2_w, n2_b,
+                       dp1, dp2, geom, mode: ComputeMode):
+    """SwinBlockFn.forward without saving anything (same arguments, same (x_out, shadow) result, same bits): fc1 runs the
+    single-output BIAS_GELU_FWD epilogue and the LayerNorm / q-k norm / softmax statistics are not stored.  Intermediates are
+    released as soon as they are consumed, so the peak is the fc1 output plus the residual stream."""
+    B, H, W, C = x.shape
+    heads, Wh, Ww, s0, s1 = geom
+    T = B * H * W
+    x2 = x.contiguous().view(T, C)
+    if mode.act_dtype == torch.float32:
+        xb = x2
+    wq, wp = SHADOWS.get(qkv_w, mode), SHADOWS.get(proj_w, mode)
+    w1, w2 = SHADOWS.get(fc1_w, mode), SHADOWS.get(fc2_w, mode)
+    scale_c = scale.detach().contiguous()
+    bias_c = None if bias is None else bias.detach().contiguous()
+    qkv, _ = ops.qkv_projection(mode, xb, wq, qkv_b.detach(), C, heads, need_stats=False)
+    o, _ = ops.window_attn_fwd(qkv, scale_c, bias_c, B, H, W, C, heads, Wh, Ww, s0, s1, mode, need_stats=False)
+    del qkv
+    _, x_mid, xb_mid, _ = ops.linear_ln_residual(mode, o, wp, proj_b.detach(), x2, n1_w.detach(), n1_b.detach(), dp1, H * W,
+                                                 need_stats=False)
+    del o
+    g = ops.gemm(mode, xb_mid, 0, w1, 0, EPI_BIAS_GELU_FWD, bias=fc1_b.detach())
+    del xb_mid
+    _, x_out, xb_out, _ = ops.linear_ln_residual(mode, g, w2, fc2_b.detach(), x_mid, n2_w.detach(), n2_b.detach(), dp2, H * W,
+                                                 need_stats=False)
+    shadow = xb_out if mode.act_dtype != torch.float32 else x_out.new_empty(0)
+    return x_out.view(B, H, W, C), shadow
+
+
 # ---- head + unpatchify (+ skip) ------------------------------------------------------------------------------
 class HeadFn(torch.autograd.Function):
     """reference: forward_head + `x + skip[:, :out_chans]` (swinv2_global.py:784-803)."""
@@ -248,6 +317,16 @@ class HeadFn(torch.autograd.Function):
             dskip = torch.zeros((B, skip_ch, H * patch, W * patch), dtype=torch.float32, device=dout.device)
             dskip[:, :Co] = dout if ctx.skip_std is None else dout / ctx.skip_std[:Co].view(1, Co, 1, 1)
         return dx.view(B, H, W, C), None, dw, dskip, None, None, None, None, None
+
+
+def head_forward_only(x, xb, head_w, skip, out_chans: int, patch: int, mode: ComputeMode, skip_mean=None, skip_std=None):
+    """HeadFn.forward without saving anything (the head saves no statistics: the launches are the same)."""
+    B, H, W, C = x.shape
+    if mode.act_dtype == torch.float32:
+        xb = x.contiguous().view(B * H * W, C)
+    y = ops.gemm(mode, xb, 0, SHADOWS.get(head_w, mode), 0, EPI_BIAS)
+    return ops.unpatchify(y, None if skip is None else skip.contiguous(), B, out_chans, H * patch, W * patch, patch,
+                          skip_mean=skip_mean, skip_std=skip_std)
 
 
 # ---- loss ---------------------------------------------------------------------------------------------------------

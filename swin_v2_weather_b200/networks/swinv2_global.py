@@ -13,7 +13,11 @@ Differences from the reference, all deliberate:
     on demand (bit-identical to the reference's non-persistent buffer) instead of being stored;
   * torch.roll / window_partition / window_reverse never run: they are folded into kernel addressing;
   * `compute_mode`: "bf16" (default; bf16 storage + tcgen05 GEMMs, fp32 residual stream/statistics) or
-    "fp32" (validation mode).  Ambient torch autocast is ignored by the kernels.
+    "fp32" (validation mode).  Ambient torch autocast is ignored by the kernels;
+  * when no gradient will be taken -- grad mode off (torch.no_grad / torch.inference_mode), or nothing a call reads
+    requires grad -- PatchEmbed, the blocks and the head run forward-only: same kernels and bits, but nothing is kept
+    for a backward (no fc1 pre-activation, no row statistics).  Like deterministic mode this follows torch's state;
+    there is no option.
 """
 from __future__ import annotations
 
@@ -51,6 +55,15 @@ def _carry_shadow(dst: torch.Tensor, shadow: Optional[torch.Tensor]) -> torch.Te
     if shadow is not None and shadow.numel() > 0:
         setattr(dst, _SHADOW_ATTR, shadow)
     return dst
+
+
+def _forward_only(*tensors: Optional[torch.Tensor]) -> bool:
+    """True when no gradient can be taken through a call reading `tensors` (inputs and parameters): grad mode is off, or
+    none of them requires grad.  checkpoint(use_reentrant=False) runs (and re-runs) its forward with grad enabled, so
+    checkpointed training keeps the training path."""
+    if not torch.is_grad_enabled():
+        return True
+    return not any(t is not None and t.requires_grad for t in tensors)
 
 
 def _shadow_of(x_bhwc: torch.Tensor, mode: ops.ComputeMode) -> torch.Tensor:
@@ -298,10 +311,13 @@ class SwinTransformerV2CrBlock(nn.Module):
         dp1 = self._drop_scale(self.drop_path1, x, 4)
         dp2 = self._drop_scale(self.drop_path2, x, 3)
         geom = (a.num_heads, self.window_size[0], self.window_size[1], self.shift_size[0], self.shift_size[1])
-        out, shadow = Fn.SwinBlockFn.apply(
-            x, xb, (a.logit_scale_factor() if scale is None else scale).float(), bias, a.qkv.weight, a.qkv.bias, a.proj.weight, a.proj.bias,
-            self.norm1.weight, self.norm1.bias, self.mlp.fc1.weight, self.mlp.fc1.bias, self.mlp.fc2.weight,
-            self.mlp.fc2.bias, self.norm2.weight, self.norm2.bias, dp1, dp2, geom, mode)
+        scale = (a.logit_scale_factor() if scale is None else scale).float()
+        weights = (a.qkv.weight, a.qkv.bias, a.proj.weight, a.proj.bias, self.norm1.weight, self.norm1.bias, self.mlp.fc1.weight,
+                   self.mlp.fc1.bias, self.mlp.fc2.weight, self.mlp.fc2.bias, self.norm2.weight, self.norm2.bias)
+        if _forward_only(x, scale, bias, *weights):
+            out, shadow = Fn.block_forward_only(x, xb, scale, bias, *weights, dp1, dp2, geom, mode)
+        else:
+            out, shadow = Fn.SwinBlockFn.apply(x, xb, scale, bias, *weights, dp1, dp2, geom, mode)
         return _carry_shadow(out, shadow)
 
 
@@ -467,9 +483,13 @@ class SwinTransformerV2Cr(nn.Module):
         assert W == self.img_size[1], f"Input image width ({W}) doesn't match model ({self.img_size[1]})."
         pe = self.patch_embed
         mean, std = self._input_stats(input_stats, sum(t.shape[1] for t in parts), parts[0].device)
-        tok, shadow = Fn.PatchEmbedFn.apply(parts[0], pe.proj.weight, pe.proj.bias, pe.norm.weight, pe.norm.bias,
-                                            self.pos_embed if self.full_pos_embed else None, self.patch_size, mode, mean, std,
-                                            *parts[1:])
+        pos = self.pos_embed if self.full_pos_embed else None
+        if _forward_only(*parts, pe.proj.weight, pe.proj.bias, pe.norm.weight, pe.norm.bias, pos, mean, std):
+            tok, shadow = Fn.patch_embed_forward_only(parts[0], pe.proj.weight, pe.proj.bias, pe.norm.weight, pe.norm.bias, pos,
+                                                      self.patch_size, mode, mean, std, *parts[1:])
+        else:
+            tok, shadow = Fn.PatchEmbedFn.apply(parts[0], pe.proj.weight, pe.proj.bias, pe.norm.weight, pe.norm.bias, pos,
+                                                self.patch_size, mode, mean, std, *parts[1:])
         x = _carry_shadow(bhwc_to_bchw(tok), shadow)
         return self.stages(x)
 
@@ -480,6 +500,9 @@ class SwinTransformerV2Cr(nn.Module):
         if not t.is_contiguous():
             t = t.contiguous()
         t = _carry_shadow(t.float(), shadow)
+        if _forward_only(t, self.head.weight, skip):
+            return Fn.head_forward_only(t, _shadow_of(t, mode), self.head.weight, skip, self.out_chans, self.patch_size, mode,
+                                        *skip_stats)
         return Fn.HeadFn.apply(t, _shadow_of(t, mode), self.head.weight, skip, self.out_chans, self.patch_size, mode, *skip_stats)
 
     def forward(self, x, input_stats=None) -> torch.Tensor:

@@ -8,6 +8,9 @@ Deterministic mode: while torch.use_deterministic_algorithms(True) is in force, 
 the order in which CTAs finish (split-K weight gradients, bias / LayerNorm parameter gradients, loss and metric sums, attention
 d(scale) / d(bias)) runs through the fixed-order `swinb200_*_det` entry points, with scratch from the torch allocator
 (DESIGN.md section 10).  With the flag off nothing changes.
+
+Forward-only runs: `need_stats=False` (ln_residual_fwd, linear_ln_residual, qkv_projection, window_attn_fwd) allocates none of
+the row statistics that only a backward reads and passes NULL for them; every other output is bit-identical.
 """
 from __future__ import annotations
 
@@ -19,8 +22,8 @@ from typing import Optional
 import torch
 
 from . import _lib
-from ._lib import (BACKEND_SIMT, BACKEND_TCGEN05, BF16, EPI_ADD_F32, EPI_BIAS, EPI_BIAS_GELU, EPI_BIAS_QKNORM, EPI_DGELU,
-                   EPI_F32, F32, SwinB200Error)
+from ._lib import (BACKEND_SIMT, BACKEND_TCGEN05, BF16, EPI_ADD_F32, EPI_BIAS, EPI_BIAS_GELU, EPI_BIAS_GELU_FWD, EPI_BIAS_QKNORM,
+                   EPI_DGELU, EPI_F32, F32, SwinB200Error)
 
 LN_EPS = 1e-5
 
@@ -149,7 +152,8 @@ def unpatchify(y: torch.Tensor, skip: Optional[torch.Tensor], B: int, Co: int, H
 def gemm(mode: ComputeMode, A: torch.Tensor, a_major: int, B: torch.Tensor, b_major: int, epilogue: int, *,
          bias: Optional[torch.Tensor] = None, aux: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None,
          out2: Optional[torch.Tensor] = None, accumulate: bool = False, split_k: int = 1, backend: Optional[int] = None):
-    """D[M,N] = epi(sum_k A(m,k) B(n,k)); see swinb200_gemm.  A/B are 2-D contiguous tensors."""
+    """D[M,N] = epi(sum_k A(m,k) B(n,k)); see swinb200_gemm.  A/B are 2-D contiguous tensors.
+    Returns D, or (D, D2) for EPI_BIAS_GELU (activation, pre-activation); EPI_BIAS_GELU_FWD returns the activation alone."""
     if a_major == 0:
         M, K = A.shape
     else:
@@ -184,20 +188,22 @@ def gemm(mode: ComputeMode, A: torch.Tensor, a_major: int, B: torch.Tensor, b_ma
     return (out, out2) if epilogue == EPI_BIAS_GELU else out
 
 
-def qkv_projection(mode: ComputeMode, xb: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, C: int, heads: int):
-    """qkv = xb @ W^T + b with q and k L2-normalised per head; returns (qkv, inv_norm (T, 2, heads)).
+def qkv_projection(mode: ComputeMode, xb: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, C: int, heads: int,
+                   need_stats: bool = True):
+    """qkv = xb @ W^T + b with q and k L2-normalised per head; returns (qkv, inv_norm (T, 2, heads)), inv_norm None when
+    not `need_stats`.
     tcgen05 / head_dim 96: the normalisation runs in the GEMM epilogue (accumulators never leave fp32 before it);
     otherwise the GEMM is followed by the stand-alone normalisation kernel."""
     T = xb.shape[0]
     if mode.gemm_backend == BACKEND_TCGEN05 and C // heads == 96:
         qkv = torch.empty((T, 3 * C), dtype=xb.dtype, device=xb.device)
-        inv_norm = torch.empty((T, 2, heads), dtype=torch.float32, device=xb.device)
+        inv_norm = torch.empty((T, 2, heads), dtype=torch.float32, device=xb.device) if need_stats else None
         _lib.call("swinb200_gemm", BACKEND_TCGEN05, T, 3 * C, C, _chk(xb, "xb", torch.bfloat16), 0, C, _chk(w, "w", torch.bfloat16), 0, C,
-                  BF16, EPI_BIAS_QKNORM, _chk(bias, "bias", torch.float32), qkv.data_ptr(), 3 * C, inv_norm.data_ptr(), 0, 96, BF16,
-                  0, 1, _stream())
+                  BF16, EPI_BIAS_QKNORM, _chk(bias, "bias", torch.float32), qkv.data_ptr(), 3 * C,
+                  0 if inv_norm is None else inv_norm.data_ptr(), 0, 96, BF16, 0, 1, _stream())
         return qkv, inv_norm
     qkv = gemm(mode, xb, 0, w, 0, EPI_BIAS, bias=bias)
-    return qkv, qk_normalize_(qkv, C, heads)
+    return qkv, qk_normalize_(qkv, C, heads, need_stats)
 
 
 def wgrad_split_k(M: int, N: int, K: int) -> int:
@@ -219,15 +225,16 @@ def wgrad_split_k(M: int, N: int, K: int) -> int:
 
 
 # ---- LayerNorm + residual ------------------------------------------------------------------------------
-def ln_residual_fwd(z, x_in, gamma, beta, sample_scale, pos, rows_per_sample: int, mode: ComputeMode):
+def ln_residual_fwd(z, x_in, gamma, beta, sample_scale, pos, rows_per_sample: int, mode: ComputeMode, need_stats: bool = True):
+    """-> (x_out, xb_out, stats (rows, 2) or None when not `need_stats`)"""
     rows, C = z.shape
     x_out = torch.empty((rows, C), dtype=torch.float32, device=z.device)
     xb = x_out if mode.act_dtype == torch.float32 else torch.empty((rows, C), dtype=mode.act_dtype, device=z.device)
-    stats = torch.empty((rows, 2), dtype=torch.float32, device=z.device)
+    stats = torch.empty((rows, 2), dtype=torch.float32, device=z.device) if need_stats else None
     _lib.call("swinb200_ln_residual_fwd", _chk(z, "z", mode.act_dtype), mode.act_code, _chk(x_in, "x_in", torch.float32, True),
               _chk(gamma, "gamma", torch.float32), _chk(beta, "beta", torch.float32),
               _chk(sample_scale, "sample_scale", torch.float32, True), _chk(pos, "pos", torch.float32, True),
-              x_out.data_ptr(), xb.data_ptr(), stats.data_ptr(), rows, C, rows_per_sample, LN_EPS, _stream())
+              x_out.data_ptr(), xb.data_ptr(), 0 if stats is None else stats.data_ptr(), rows, C, rows_per_sample, LN_EPS, _stream())
     return x_out, xb, stats
 
 
@@ -260,7 +267,7 @@ _LN_COUNTERS = {}
 
 
 def linear_ln_residual(mode: ComputeMode, a, w, bias, x_in, gamma, beta, sample_scale, rows_per_sample: int,
-                       fuse: Optional[bool] = None):
+                       fuse: Optional[bool] = None, need_stats: bool = True):
     """z = a @ w^T + bias ; x_out = x_in + sample_scale * (LN(z) gamma + beta)  ->  (z, x_out, xb_out, stats).
 
     Two implementations with identical results (tests/test_kernels_gpu.py::test_linear_ln_residual_fused_epilogue):
@@ -268,7 +275,8 @@ def linear_ln_residual(mode: ComputeMode, a, w, bias, x_in, gamma, beta, sample_
     * `fuse=True` / SWINB200_FUSE_LN=1, tcgen05 / 768 channels: ONE kernel, the LayerNorm + DropPath scale + residual run
       inside the GEMM epilogue (swinb200_linear_ln_residual).  Measured on the B200 it is not faster -- fc2: 323 us against
       216 + 105 us, proj: 225 us against 65 + 105 us -- because the LayerNorm's 600 MB of HBM traffic raises the latency of
-      the operand loads beyond what the 4-stage ring covers (DESIGN.md section 5.2), so the model keeps the two kernels."""
+      the operand loads beyond what the 4-stage ring covers (DESIGN.md section 5.2), so the model keeps the two kernels.
+    `need_stats=False` drops the statistics of the two-kernel path (None is returned); the fused kernel always stores them."""
     M, K = a.shape
     N = w.shape[0]
     if fuse is None:
@@ -276,7 +284,7 @@ def linear_ln_residual(mode: ComputeMode, a, w, bias, x_in, gamma, beta, sample_
         fuse = env == "1" or (env == "2" and K >= 2048)
     if not (fuse and mode.gemm_backend == BACKEND_TCGEN05 and N == 768):
         z = gemm(mode, a, 0, w, 0, EPI_BIAS, bias=bias)
-        return (z,) + ln_residual_fwd(z, x_in, gamma, beta, sample_scale, None, rows_per_sample, mode)
+        return (z,) + ln_residual_fwd(z, x_in, gamma, beta, sample_scale, None, rows_per_sample, mode, need_stats)
     dev = a.device
     counters = _LN_COUNTERS.get(dev)
     n_blocks = (M + 127) // 128
@@ -315,9 +323,12 @@ def ln_residual_bwd(dx, z, stats, gamma, sample_scale, rows_per_sample: int, mod
     return dz, acc[0], acc[1], acc[2]
 
 
-def transpose_f32(src: torch.Tensor) -> torch.Tensor:
+def transpose_f32(src: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     R, Cc = src.shape
-    dst = torch.empty((Cc, R), dtype=torch.float32, device=src.device)
+    dst = torch.empty((Cc, R), dtype=torch.float32, device=src.device) if out is None else out
+    if tuple(dst.shape) != (Cc, R):
+        raise SwinB200Error(f"transpose_f32: out has shape {tuple(dst.shape)}, expected {(Cc, R)}")
+    _chk(dst, "out", torch.float32)
     _lib.call("swinb200_transpose_f32", _chk(src, "src", torch.float32), dst.data_ptr(), R, Cc, _stream())
     return dst
 
@@ -343,10 +354,11 @@ def colsum(x: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
 
 
 # ---- attention --------------------------------------------------------------------------------------------
-def qk_normalize_(qkv: torch.Tensor, C: int, heads: int) -> torch.Tensor:
+def qk_normalize_(qkv: torch.Tensor, C: int, heads: int, need_stats: bool = True) -> Optional[torch.Tensor]:
     T = qkv.shape[0]
-    inv_norm = torch.empty((T, 2, heads), dtype=torch.float32, device=qkv.device)
-    _lib.call("swinb200_qk_normalize", _chk(qkv, "qkv"), _code(qkv.dtype), inv_norm.data_ptr(), T, C, heads, _stream())
+    inv_norm = torch.empty((T, 2, heads), dtype=torch.float32, device=qkv.device) if need_stats else None
+    _lib.call("swinb200_qk_normalize", _chk(qkv, "qkv"), _code(qkv.dtype), 0 if inv_norm is None else inv_norm.data_ptr(), T, C,
+              heads, _stream())
     return inv_norm
 
 
@@ -371,15 +383,19 @@ def attn_backend_for(mode: ComputeMode, C: int, heads: int, Wh: int, Ww: int) ->
     return BACKEND_SIMT
 
 
-def window_attn_fwd(qkv, scale, bias, B, H, W, C, heads, Wh, Ww, s0, s1, mode: ComputeMode, backend=None):
+def window_attn_fwd(qkv, scale, bias, B, H, W, C, heads, Wh, Ww, s0, s1, mode: ComputeMode, backend=None, need_stats: bool = True):
+    """-> (o, lse (2, B, nW, heads, L) or None when not `need_stats`)"""
     T = B * H * W
     if backend is None:
         backend = attn_backend_for(mode, C, heads, Wh, Ww)
     nW, L = (H // Wh) * (W // Ww), Wh * Ww
     o = torch.empty((T, C), dtype=qkv.dtype, device=qkv.device)
-    lse = torch.empty((2, B, nW, heads, L), dtype=torch.float32, device=qkv.device)   # plane 0: LSE, plane 1: mean cosine
+    lse = None
+    if need_stats:
+        lse = torch.empty((2, B, nW, heads, L), dtype=torch.float32, device=qkv.device)   # plane 0: LSE, plane 1: mean cosine
     _lib.call("swinb200_window_attn_fwd", backend, _chk(qkv, "qkv"), _code(qkv.dtype),
-              _chk(scale, "scale", torch.float32), _chk(bias, "bias", torch.float32, True), o.data_ptr(), lse.data_ptr(),
+              _chk(scale, "scale", torch.float32), _chk(bias, "bias", torch.float32, True), o.data_ptr(),
+              0 if lse is None else lse.data_ptr(),
               B, H, W, C, heads, Wh, Ww, s0, s1, _stream())
     return o, lse
 
